@@ -2,6 +2,7 @@
 semantics to the reference's OWN code: onnx_controller/src/controller.cpp and onnx_inference/src/cpp/onnx_actor.cpp,
 compiled from /root/reference against stub ROS / Eigen / ONNX-Runtime headers (oracle/Makefile -> oracle/_ref).
 Inside that build Session::Run is the C fp32 restatement, so A7 itself stays "parity unpinned" (DESIGN.md)."""
+import hashlib
 import os
 
 import numpy as np
@@ -10,7 +11,21 @@ import pytest
 from oracle import coracle, oracle
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-HAVE_REF = os.path.exists(coracle.REF_LIB_PATH) and os.path.exists("/root/reference/onnx_inference/data/model.onnx")
+HAVE_REF = os.path.exists(coracle.REF_LIB_PATH)
+NEEDS_REF = "needs oracle/_ref, which oracle/Makefile builds only where the reference sources are present"
+MODEL_SHA256 = "9bdcb0f47be89417dbf3f7fb46522ecb3ec42ca65458a905f191aff933a18eae"   # the reference's model.onnx
+
+
+@pytest.fixture
+def ref_share_dir(model_path, tmp_path, monkeypatch):
+    """The compiled controller reads <GO2_REF_ROOT>/onnx_inference/data/model.onnx (ament share directory stub): point
+    it at a copy of the bundled model, which is the reference's file byte for byte, so no reference tree is needed."""
+    data = open(model_path, "rb").read()
+    assert hashlib.sha256(data).hexdigest() == MODEL_SHA256
+    d = tmp_path / "onnx_inference" / "data"
+    d.mkdir(parents=True)
+    (d / "model.onnx").write_bytes(data)
+    monkeypatch.setenv("GO2_REF_ROOT", str(tmp_path))
 
 
 def bits(a):
@@ -58,8 +73,8 @@ def test_numpy_oracle_obs_and_post_match_reference_trace(policy, golden_loop):
         assert np.abs(so.action - pub).max() < 1e-4
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="needs oracle/_ref and the reference tree (build container only)")
-def test_reference_controller_live_vs_oracle_and_fixture(cmodel, golden_loop):
+@pytest.mark.skipif(not HAVE_REF, reason=NEEDS_REF)
+def test_reference_controller_live_vs_oracle_and_fixture(cmodel, golden_loop, ref_share_dir):
     tr = np.load(os.path.join(GOLD, "ref_controller_trace.npz"))
     g = golden_loop
     rc = coracle.RefController()
@@ -75,8 +90,8 @@ def test_reference_controller_live_vs_oracle_and_fixture(cmodel, golden_loop):
         rc.close()
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="needs oracle/_ref and the reference tree (build container only)")
-def test_reference_controller_gates_and_params(golden_loop):
+@pytest.mark.skipif(not HAVE_REF, reason=NEEDS_REF)
+def test_reference_controller_gates_and_params(golden_loop, ref_share_dir):
     """publish() is skipped while the robot is not ready / not safe (controller.cpp:158-171) and kp/kd follow the ROS
     parameters (controller.cpp:254-277); the dead-man button forces kp = 5 (controller.cpp:246)."""
     g = golden_loop
