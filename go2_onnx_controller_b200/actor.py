@@ -59,6 +59,19 @@ class _Handle:
             pass
 
 
+def host_reset_mask(reset, B: int) -> np.ndarray:
+    """Validates a per-robot reset mask for the host-buffer steps: a numpy bool / uint8 array of shape (B,), C-contiguous
+    (one byte per robot, as go2p_step_batch_host_ex reads it).  Returns it unchanged; raises TypeError / ValueError."""
+    if not isinstance(reset, np.ndarray) or reset.dtype not in (np.bool_, np.uint8):
+        raise TypeError(f"reset must be a numpy bool or uint8 array, got {type(reset).__name__}"
+                        + (f" of {reset.dtype}" if isinstance(reset, np.ndarray) else ""))
+    if reset.shape != (B,):
+        raise ValueError(f"reset must have shape ({B},), got {reset.shape}")
+    if not reset.flags.c_contiguous:
+        raise ValueError("reset must be C-contiguous")
+    return reset
+
+
 class ONNXActor:
     """Python face of the reference's ONNXActor: observation/action numpy buffers are bound at construction
     (they must be C-contiguous float32 and outlive the actor) and act() overwrites ``action`` in place."""
@@ -220,25 +233,41 @@ class PolicyBatch:
         capi.check(self._hd.lib.go2p_assemble_batch(self._hd.h, d_raw, d_prev_action, d_vel_cmd, d_obs, B, stream or None))
 
     def step_device(self, d_raw: int, d_vel_cmd: int, d_obs: int, d_action: int, d_qdes: int, B: int,
-                    precision: int = capi.PREC_FP32, stream: int = 0) -> None:
+                    precision: int = capi.PREC_FP32, stream: int = 0, d_reset: int | None = None) -> None:
         """Batched publish() (reference: controller.cpp:173-251 per robot): raw states -> observation history ->
-        policy -> clamp/mask -> q_des, all on device buffers; d_action is the previous published action on entry."""
-        capi.check(self._hd.lib.go2p_step_batch(self._hd.h, d_raw, d_vel_cmd, d_obs, d_action, d_qdes, B, precision,
-                                                stream or None))
+        policy -> clamp/mask -> q_des, all on device buffers; d_action is the previous published action on entry.
+        d_reset: device pointer to [B] bytes (e.g. a torch.bool tensor); robots with a non-zero byte start from the
+        controller's initial state this step (go2p_step_batch_ex)."""
+        if d_reset is None:
+            capi.check(self._hd.lib.go2p_step_batch(self._hd.h, d_raw, d_vel_cmd, d_obs, d_action, d_qdes, B, precision,
+                                                    stream or None))
+        else:
+            capi.check(self._hd.lib.go2p_step_batch_ex(self._hd.h, d_raw, d_reset, d_vel_cmd, d_obs, d_action, d_qdes, None,
+                                                       B, precision, stream or None))
 
     def step_device_cmd(self, d_raw: int, d_vel_cmd: int, d_obs: int, d_action: int, d_qdes: int | None, d_cmd: int | None,
-                        B: int, precision: int = capi.PREC_FP32, stream: int = 0) -> None:
+                        B: int, precision: int = capi.PREC_FP32, stream: int = 0, d_reset: int | None = None) -> None:
         """step_device ending in motor commands: d_cmd [B] go2p_motor_cmd (Unitree motor order), d_qdes may be None."""
-        capi.check(self._hd.lib.go2p_step_batch_cmd(self._hd.h, d_raw, d_vel_cmd, d_obs, d_action, d_qdes, d_cmd, B, precision,
-                                                    stream or None))
+        if d_reset is None:
+            capi.check(self._hd.lib.go2p_step_batch_cmd(self._hd.h, d_raw, d_vel_cmd, d_obs, d_action, d_qdes, d_cmd, B,
+                                                        precision, stream or None))
+        else:
+            capi.check(self._hd.lib.go2p_step_batch_ex(self._hd.h, d_raw, d_reset, d_vel_cmd, d_obs, d_action, d_qdes, d_cmd,
+                                                       B, precision, stream or None))
 
     def step_host(self, raw: np.ndarray, action: np.ndarray, cmd: np.ndarray | None = None,
-                  precision: int = capi.PREC_FP32) -> None:
+                  precision: int = capi.PREC_FP32, reset: np.ndarray | None = None) -> None:
         """Closed-loop step for len(raw) robots from host buffers; per-robot history stays on the device.
-        raw: uint8 [B, 156] (go2p_raw_state records), action: float32 [B, 12] out, cmd: uint8 [B, 112] out or None."""
+        raw: uint8 [B, 156] (go2p_raw_state records), action: float32 [B, 12] out, cmd: uint8 [B, 112] out or None,
+        reset: bool / uint8 [B] or None -- robots to start from the controller's initial state this step."""
         B = raw.shape[0]
-        capi.check(self._hd.lib.go2p_step_batch_host(self._hd.h, raw.ctypes.data, action.ctypes.data,
-                                                     cmd.ctypes.data if cmd is not None else None, B, precision))
+        cmd_p = cmd.ctypes.data if cmd is not None else None
+        if reset is None:
+            capi.check(self._hd.lib.go2p_step_batch_host(self._hd.h, raw.ctypes.data, action.ctypes.data, cmd_p, B, precision))
+        else:
+            reset = host_reset_mask(reset, B)
+            capi.check(self._hd.lib.go2p_step_batch_host_ex(self._hd.h, raw.ctypes.data, reset.ctypes.data, action.ctypes.data,
+                                                            cmd_p, B, precision))
 
     def step_host_reset(self) -> None:
         capi.check(self._hd.lib.go2p_step_batch_host_reset(self._hd.h))
@@ -262,9 +291,16 @@ class Fleet:
     def infer_host(self, obs: np.ndarray, act: np.ndarray, precision: int = capi.PREC_FP32) -> None:
         capi.check(self.lib.go2p_fleet_infer_host(self.f, obs.ctypes.data, act.ctypes.data, obs.shape[0], precision))
 
-    def step_host(self, raw: np.ndarray, action: np.ndarray, cmd: np.ndarray | None = None, precision: int = capi.PREC_FP32) -> None:
-        capi.check(self.lib.go2p_fleet_step_host(self.f, raw.ctypes.data, action.ctypes.data,
-                                                 cmd.ctypes.data if cmd is not None else None, raw.shape[0], precision))
+    def step_host(self, raw: np.ndarray, action: np.ndarray, cmd: np.ndarray | None = None, precision: int = capi.PREC_FP32,
+                  reset: np.ndarray | None = None) -> None:
+        """PolicyBatch.step_host over the devices' shards; reset: bool / uint8 [B] or None."""
+        cmd_p = cmd.ctypes.data if cmd is not None else None
+        if reset is None:
+            capi.check(self.lib.go2p_fleet_step_host(self.f, raw.ctypes.data, action.ctypes.data, cmd_p, raw.shape[0], precision))
+        else:
+            reset = host_reset_mask(reset, raw.shape[0])
+            capi.check(self.lib.go2p_fleet_step_host_ex(self.f, raw.ctypes.data, reset.ctypes.data, action.ctypes.data, cmd_p,
+                                                        raw.shape[0], precision))
 
     def close(self) -> None:
         if self.f:

@@ -98,10 +98,13 @@ SIGNATURES = {
                                         C.c_uint32, C.c_void_p]),
     "go2p_step_batch_cmd": (C.c_int, [_H, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                                        C.c_int, C.c_void_p]),
+    "go2p_step_batch_ex": (C.c_int, [_H, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                      C.c_int64, C.c_int, C.c_void_p]),
     "go2p_step_fused_cmd": (C.c_int, [_H, C.POINTER(RawState), C.POINTER(StepOut), C.POINTER(MotorCmd)]),
     "go2p_motor_order": (C.c_int, [C.POINTER(C.c_int32)]),
     "go2p_step_batch_host": (C.c_int, [_H, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int]),
     "go2p_step_batch_host_reset": (C.c_int, [_H]),
+    "go2p_step_batch_host_ex": (C.c_int, [_H, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int]),
     "go2p_log_enable": (C.c_int, [_H, C.c_int]),
     "go2p_log_drain": (C.c_int, [_H, C.c_void_p, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_uint64)]),
     "go2p_fleet_create": (C.c_int, [C.c_char_p, C.POINTER(Config), C.POINTER(C.c_int32), C.c_int, C.POINTER(C.c_void_p)]),
@@ -110,6 +113,7 @@ SIGNATURES = {
     "go2p_shard_rows": (C.c_int, [C.c_int64, C.c_int, C.c_int, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "go2p_fleet_infer_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int]),
     "go2p_fleet_step_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int]),
+    "go2p_fleet_step_host_ex": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int]),
     "go2p_dev_alloc": (C.c_int, [_H, C.c_size_t, C.POINTER(C.c_void_p)]),
     "go2p_dev_free": (C.c_int, [_H, C.c_void_p]),
     "go2p_host_alloc": (C.c_int, [_H, C.c_size_t, C.POINTER(C.c_void_p)]),

@@ -72,7 +72,7 @@ struct go2p_handle {
   bool wide_ok = false;
   uint16_t* d_wpack[2] = {nullptr, nullptr};   // [0] bf16, [1] fp16
   int k0p = 0;
-  size_t tc_attr_smem[4] = {0, 0, 0, 0};       // dynamic shared memory opted in for tc_mlp_kernel<bf16|fp16, plain|fused> on this device
+  size_t tc_attr_smem[6] = {};                 // dynamic shared memory opted in for tc_mlp_kernel<bf16|fp16, plain|fused|fused+reset> on this device
   bool b1_attr_set = false;                    // same for the one-shot batch-1 kernel
   size_t so_attr_smem = 0;                     // same for small_out_kernel
   WideModel wide{};
@@ -117,6 +117,7 @@ struct go2p_handle {
     go2p_raw_state* raw[kPipeDepth] = {};
     MotorCmdDev* cmd[kPipeDepth] = {};
     int32_t* button[kPipeDepth] = {};
+    uint8_t* reset[kPipeDepth] = {};    // go2p_step_batch_host_ex: the chunk's reset flags
   } fleet;
 };
 
@@ -456,12 +457,12 @@ int launch_fp32(go2p_handle* h, const float* d_obs, const int32_t* d_button0, fl
   return GO2P_OK;
 }
 
-template <bool kFp16, bool kFused>
+template <bool kFp16, bool kFused, bool kReset = false>
 int launch_tc_t(go2p_handle* h, const TcArgs& a, cudaStream_t st) {
   const size_t smem = tc_smem_bytes(a);
-  auto kernel = tc_mlp_kernel<kFp16, kFused>;
+  auto kernel = tc_mlp_kernel<kFp16, kFused, kReset>;
   // the opt-in is a per-device function attribute: remembered per handle (one handle = one device)
-  size_t& configured = h->tc_attr_smem[(kFp16 ? 1 : 0) + (kFused ? 2 : 0)];
+  size_t& configured = h->tc_attr_smem[(kFp16 ? 1 : 0) + (kFused ? 2 : 0) + (kReset ? 2 : 0)];
   if (configured != smem) {
     CU_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     configured = smem;
@@ -482,10 +483,11 @@ int launch_tc_t(go2p_handle* h, const TcArgs& a, cudaStream_t st) {
   return GO2P_OK;
 }
 
-// raw != null: the fused controller step (A1-A6 in the conversion job): d_obs is the robots' history, updated in place
+// raw != null: the fused controller step (A1-A6 in the conversion job): d_obs is the robots' history, updated in place;
+// d_reset (may be null) the robots' reset flags
 int launch_tc(go2p_handle* h, const float* d_obs, const int32_t* d_button0, float* d_act, double* d_qdes,
               MotorCmdDev* d_cmd, int64_t B, bool fp16, uint32_t flags, cudaStream_t st,
-              const RawStateDev* raw = nullptr, float* d_vel_cmd = nullptr) {
+              const RawStateDev* raw = nullptr, float* d_vel_cmd = nullptr, const uint8_t* d_reset = nullptr) {
   if ((reinterpret_cast<uintptr_t>(d_obs) & 15) || (reinterpret_cast<uintptr_t>(d_act) & 15) ||
       (d_qdes && (reinterpret_cast<uintptr_t>(d_qdes) & 15)))
     return fail(GO2P_ERR_INVALID, "tensor-core path needs 16-byte aligned obs/act/qdes device pointers");
@@ -516,6 +518,8 @@ int launch_tc(go2p_handle* h, const float* d_obs, const int32_t* d_button0, floa
   if (const char* e = std::getenv("GO2P_TC_TRACE_PTR")) a.trace = reinterpret_cast<unsigned long long*>(std::strtoull(e, nullptr, 0));
 #endif
   a.raw = raw; a.obs_rw = const_cast<float*>(d_obs); a.vel_cmd = d_vel_cmd; a.H = h->cc.H; a.foot_threshold = h->cc.foot_threshold;
+  a.reset = raw ? d_reset : nullptr;
+  if (raw && d_reset) return fp16 ? launch_tc_t<true, true, true>(h, a, st) : launch_tc_t<false, true, true>(h, a, st);
   if (raw) return fp16 ? launch_tc_t<true, true>(h, a, st) : launch_tc_t<false, true>(h, a, st);
   return fp16 ? launch_tc_t<true, false>(h, a, st) : launch_tc_t<false, false>(h, a, st);
 }
@@ -675,6 +679,7 @@ int go2p_destroy(go2p_handle* h) {
     if (h->fleet.raw[i]) cudaFree(h->fleet.raw[i]);
     if (h->fleet.cmd[i]) cudaFree(h->fleet.cmd[i]);
     if (h->fleet.button[i]) cudaFree(h->fleet.button[i]);
+    if (h->fleet.reset[i]) cudaFree(h->fleet.reset[i]);
   }
   if (h->inbox) cudaFreeHost(h->inbox);
   if (h->outbox) cudaFreeHost(h->outbox);
@@ -1058,9 +1063,12 @@ int go2p_assemble_batch(go2p_handle* h, const go2p_raw_state* d_raw, const float
 }
 
 namespace {
-// publish() for B robots on device buffers; button_scratch [B] receives the dead-man buttons for the epilogue
-int step_batch_on(go2p_handle* h, const go2p_raw_state* d_raw, float* d_vel_cmd, float* d_obs, float* d_action, double* d_qdes,
-                  go2p_motor_cmd* d_cmd, int32_t* button_scratch, int64_t B, int precision, cudaStream_t st) {
+// publish() for B robots on device buffers; button_scratch [B] receives the dead-man buttons for the epilogue.
+// d_reset [B] (may be null): robots to start from the initial state, applied by whichever kernel assembles the
+// observations (the fused kernel's conversion job or assemble_batch_kernel); the path choice does not depend on it.
+int step_batch_on(go2p_handle* h, const go2p_raw_state* d_raw, const uint8_t* d_reset, float* d_vel_cmd, float* d_obs,
+                  float* d_action, double* d_qdes, go2p_motor_cmd* d_cmd, int32_t* button_scratch, int64_t B, int precision,
+                  cudaStream_t st) {
   const uint32_t all_flags = GO2P_F_CLAMP_MASK | (d_qdes ? GO2P_F_QDES : 0u) | (d_cmd ? GO2P_F_MOTOR_CMD : 0u);
   TcArgs probe{};
   probe.n_layers = h->dm.n_layers; probe.in_dim = h->dm.in_dim; probe.k0p = h->k0p;
@@ -1072,11 +1080,11 @@ int step_batch_on(go2p_handle* h, const go2p_raw_state* d_raw, float* d_vel_cmd,
     // ONE launch: A1-A6 run inside the policy kernel's conversion job, the newest frame never round-trips HBM
     h->last_launches = 0;
     return launch_tc(h, d_obs, nullptr, d_action, d_qdes, reinterpret_cast<MotorCmdDev*>(d_cmd), B, precision == GO2P_PREC_FP16,
-                     all_flags, st, reinterpret_cast<const RawStateDev*>(d_raw), d_vel_cmd);
+                     all_flags, st, reinterpret_cast<const RawStateDev*>(d_raw), d_vel_cmd, d_reset);
   }
   // A1-A6: d_action still holds the previous published action here
   launch_assemble_batch(reinterpret_cast<const RawStateDev*>(d_raw), d_action, d_vel_cmd, d_obs, B, h->cc, button_scratch,
-                        h->sm_count, st);
+                        h->sm_count, st, d_reset);
   CU_TRY(cudaGetLastError());
   // A7 + A9 + A11
   const uint32_t flags = GO2P_F_CLAMP_MASK | (d_qdes ? GO2P_F_QDES : 0u) | (d_cmd ? GO2P_F_MOTOR_CMD : 0u);
@@ -1086,8 +1094,8 @@ int step_batch_on(go2p_handle* h, const go2p_raw_state* d_raw, float* d_vel_cmd,
 }
 }  // namespace
 
-int go2p_step_batch_cmd(go2p_handle* h, const go2p_raw_state* d_raw, float* d_vel_cmd, float* d_obs, float* d_action,
-                        double* d_qdes, go2p_motor_cmd* d_cmd, int64_t B, int precision, void* stream) {
+int go2p_step_batch_ex(go2p_handle* h, const go2p_raw_state* d_raw, const uint8_t* d_reset, float* d_vel_cmd, float* d_obs,
+                       float* d_action, double* d_qdes, go2p_motor_cmd* d_cmd, int64_t B, int precision, void* stream) {
   if (!h || !d_raw || !d_vel_cmd || !d_obs || !d_action || (!d_qdes && !d_cmd))
     return fail(GO2P_ERR_INVALID, "go2p_step_batch: null argument");
   if (B <= 0) return B == 0 ? GO2P_OK : fail(GO2P_ERR_INVALID, "negative batch");
@@ -1099,8 +1107,13 @@ int go2p_step_batch_cmd(go2p_handle* h, const go2p_raw_state* d_raw, float* d_ve
     CU_TRY(cudaMalloc((void**)&h->d_step_button, (size_t)B * sizeof(int32_t)));
     h->step_button_rows = B;
   }
-  return step_batch_on(h, d_raw, d_vel_cmd, d_obs, d_action, d_qdes, d_cmd, h->d_step_button, B, precision,
+  return step_batch_on(h, d_raw, d_reset, d_vel_cmd, d_obs, d_action, d_qdes, d_cmd, h->d_step_button, B, precision,
                        static_cast<cudaStream_t>(stream));
+}
+
+int go2p_step_batch_cmd(go2p_handle* h, const go2p_raw_state* d_raw, float* d_vel_cmd, float* d_obs, float* d_action,
+                        double* d_qdes, go2p_motor_cmd* d_cmd, int64_t B, int precision, void* stream) {
+  return go2p_step_batch_ex(h, d_raw, nullptr, d_vel_cmd, d_obs, d_action, d_qdes, d_cmd, B, precision, stream);
 }
 
 int go2p_step_batch(go2p_handle* h, const go2p_raw_state* d_raw, float* d_vel_cmd, float* d_obs, float* d_action,
@@ -1111,9 +1124,10 @@ int go2p_step_batch(go2p_handle* h, const go2p_raw_state* d_raw, float* d_vel_cm
 
 // Closed-loop control step for a fleet from HOST buffers: per-robot history / joystick command / previous action stay
 // on the device inside the handle, so a step moves 156 B of raw state in and 48 B of action (+ 112 B of motor command
-// if asked for) out per robot instead of the 392 + 48 B of go2p_infer_batch_host.
-int go2p_step_batch_host(go2p_handle* h, const go2p_raw_state* h_raw, float* h_action, go2p_motor_cmd* h_cmd, int64_t B,
-                         int precision) {
+// if asked for) out per robot instead of the 392 + 48 B of go2p_infer_batch_host.  h_reset (may be null): 1 B more per
+// robot, staged per chunk next to the raw states.
+int go2p_step_batch_host_ex(go2p_handle* h, const go2p_raw_state* h_raw, const uint8_t* h_reset, float* h_action,
+                            go2p_motor_cmd* h_cmd, int64_t B, int precision) {
   if (!h || !h_raw || !h_action) return fail(GO2P_ERR_INVALID, "go2p_step_batch_host: null argument");
   if (B <= 0) return B == 0 ? GO2P_OK : fail(GO2P_ERR_INVALID, "negative batch");
   if (h->dm.in_dim != kFrame * h->cc.H || h->dm.out_dim != kDof)
@@ -1140,6 +1154,7 @@ int go2p_step_batch_host(go2p_handle* h, const go2p_raw_state* h_raw, float* h_a
       CU_TRY(cudaMalloc((void**)&f.cmd[i], (size_t)kHostChunkRows * sizeof(MotorCmdDev)));
       CU_TRY(cudaMalloc((void**)&f.button[i], (size_t)kHostChunkRows * sizeof(int32_t)));
     }
+    if (h_reset && !f.reset[i]) CU_TRY(cudaMalloc((void**)&f.reset[i], (size_t)kHostChunkRows));
   }
   const int64_t chunk = std::min<int64_t>(B, kHostChunkRows);
   int launches = 0, slot = 0;
@@ -1147,9 +1162,11 @@ int go2p_step_batch_host(go2p_handle* h, const go2p_raw_state* h_raw, float* h_a
     const int64_t rows = std::min(chunk, B - r0);
     cudaStream_t st = h->pipe_stream[slot];
     CU_TRY(cudaMemcpyAsync(f.raw[slot], h_raw + r0, (size_t)rows * sizeof(go2p_raw_state), cudaMemcpyHostToDevice, st));
+    if (h_reset) CU_TRY(cudaMemcpyAsync(f.reset[slot], h_reset + r0, (size_t)rows, cudaMemcpyHostToDevice, st));
     h->scratch_sel = 1 + slot;
-    int rc = step_batch_on(h, f.raw[slot], f.vel + r0 * 3, f.obs + r0 * n_obs, f.act + r0 * kDof, nullptr,
-                           h_cmd ? reinterpret_cast<go2p_motor_cmd*>(f.cmd[slot]) : nullptr, f.button[slot], rows, precision, st);
+    int rc = step_batch_on(h, f.raw[slot], h_reset ? f.reset[slot] : nullptr, f.vel + r0 * 3, f.obs + r0 * n_obs,
+                           f.act + r0 * kDof, nullptr, h_cmd ? reinterpret_cast<go2p_motor_cmd*>(f.cmd[slot]) : nullptr,
+                           f.button[slot], rows, precision, st);
     h->scratch_sel = 0;
     if (rc) return rc;
     launches += h->last_launches;
@@ -1159,6 +1176,11 @@ int go2p_step_batch_host(go2p_handle* h, const go2p_raw_state* h_raw, float* h_a
   for (int i = 0; i < kPipeDepth; ++i) CU_TRY(cudaStreamSynchronize(h->pipe_stream[i]));
   h->last_launches = launches;
   return GO2P_OK;
+}
+
+int go2p_step_batch_host(go2p_handle* h, const go2p_raw_state* h_raw, float* h_action, go2p_motor_cmd* h_cmd, int64_t B,
+                         int precision) {
+  return go2p_step_batch_host_ex(h, h_raw, nullptr, h_action, h_cmd, B, precision);
 }
 
 int go2p_step_batch_host_reset(go2p_handle* h) {
@@ -1265,12 +1287,18 @@ int go2p_fleet_infer_host(go2p_fleet* f, const float* h_obs, float* h_act, int64
   });
 }
 
-int go2p_fleet_step_host(go2p_fleet* f, const go2p_raw_state* h_raw, float* h_action, go2p_motor_cmd* h_cmd, int64_t B,
-                         int precision) {
+int go2p_fleet_step_host_ex(go2p_fleet* f, const go2p_raw_state* h_raw, const uint8_t* h_reset, float* h_action,
+                            go2p_motor_cmd* h_cmd, int64_t B, int precision) {
   if (!f || f->handles.empty() || !h_raw || !h_action || B < 0) return fail(GO2P_ERR_INVALID, "go2p_fleet_step_host: bad argument");
   return fleet_run(f, B, [&](go2p_handle* h, int64_t r0, int64_t rows) {
-    return go2p_step_batch_host(h, h_raw + r0, h_action + r0 * kDof, h_cmd ? h_cmd + r0 : nullptr, rows, precision);
+    return go2p_step_batch_host_ex(h, h_raw + r0, h_reset ? h_reset + r0 : nullptr, h_action + r0 * kDof,
+                                   h_cmd ? h_cmd + r0 : nullptr, rows, precision);
   });
+}
+
+int go2p_fleet_step_host(go2p_fleet* f, const go2p_raw_state* h_raw, float* h_action, go2p_motor_cmd* h_cmd, int64_t B,
+                         int precision) {
+  return go2p_fleet_step_host_ex(f, h_raw, nullptr, h_action, h_cmd, B, precision);
 }
 
 // ------------------------------------------------------------------------------------- helpers

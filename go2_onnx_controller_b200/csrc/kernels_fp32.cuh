@@ -187,6 +187,9 @@ __global__ void post_kernel(float* __restrict__ act, long long total, int out_di
 //   3. the warp walks the 32 observation rows: every lane reads its elements of a row (old frames from the row itself,
 //      the newest frame from shared memory), then writes them back shifted -- coalesced 392-byte rows, no block
 //      barrier, several rows of loads in flight.
+// reset (optional, [B] bytes): a robot whose byte is non-zero starts from the controller's initial state
+// (controller.hpp:132-162): its newest frame takes previous action 0 and, without joystick input, joystick command 0
+// (written back), and its old-frame elements come out as 0 (selected: nothing the row held reaches the output).
 constexpr int kAsmWarps = 4;
 constexpr int kAsmRawWords = 39;                        // sizeof(RawStateDev) / 4
 constexpr int kAsmRowsInFlight = 4;
@@ -195,7 +198,7 @@ template <int kPerLane>
 __global__ void __launch_bounds__(kAsmWarps * 32)
 assemble_batch_kernel(const RawStateDev* __restrict__ raw, const float* __restrict__ prev_action,
                       float* __restrict__ vel_cmd, float* __restrict__ obs, long long B, CtrlConst cc,
-                      int32_t* __restrict__ button0_out) {
+                      int32_t* __restrict__ button0_out, const uint8_t* __restrict__ reset) {
   __shared__ uint32_t s_raw[kAsmWarps][32 * kAsmRawWords];
   __shared__ float s_new[kAsmWarps][32 * kFrame];
   const int H = cc.H, n_obs = kFrame * H;
@@ -225,6 +228,8 @@ assemble_batch_kernel(const RawStateDev* __restrict__ raw, const float* __restri
     // 1. raw states of the group -> shared memory (contiguous words, coalesced)
     const uint32_t* gr = reinterpret_cast<const uint32_t*>(raw + row0);
     for (int i = lane; i < rows * kAsmRawWords; i += 32) my_raw[i] = gr[i];
+    const bool rst = reset != nullptr && lane < rows && reset[row0 + lane] != 0;   // lane r: row r's flag
+    const uint32_t rst_rows = __ballot_sync(0xffffffffu, rst);                      // bit r: row r is reset
     __syncwarp();
     // 2. newest frame of robot (row0 + lane)
     if (lane < rows) {
@@ -244,6 +249,9 @@ assemble_batch_kernel(const RawStateDev* __restrict__ raw, const float* __restri
       if (joy_valid) {
 #pragma unroll
         for (int c = 0; c < 3; ++c) { cmd[c] = vel_cmd_component(axes, c); vel_cmd[row * 3 + c] = cmd[c]; }
+      } else if (rst) {
+#pragma unroll
+        for (int c = 0; c < 3; ++c) { cmd[c] = 0.f; vel_cmd[row * 3 + c] = 0.f; }
       } else {
 #pragma unroll
         for (int c = 0; c < 3; ++c) cmd[c] = vel_cmd[row * 3 + c];
@@ -254,7 +262,7 @@ assemble_batch_kernel(const RawStateDev* __restrict__ raw, const float* __restri
       for (int c = 0; c < kDof; ++c) nf[9 + c] = __double2float_rn(__dsub_rn((double)rf[7 + c], cc.q0[c]));
 #pragma unroll
       for (int c = 0; c < kDof; ++c) nf[21 + c] = rf[19 + c];
-      if (prev_action) {
+      if (prev_action && !rst) {
         const float4* pa = reinterpret_cast<const float4*>(prev_action + row * kDof);
 #pragma unroll
         for (int q = 0; q < 3; ++q) { const float4 t4 = pa[q]; nf[33 + 4 * q] = t4.x; nf[34 + 4 * q] = t4.y; nf[35 + 4 * q] = t4.z; nf[36 + 4 * q] = t4.w; }
@@ -279,10 +287,11 @@ assemble_batch_kernel(const RawStateDev* __restrict__ raw, const float* __restri
         const int r = r0 + i;
         if (r < rows) {
           const float* o = obs + (row0 + r) * n_obs;
+          const bool old_zero = (rst_rows >> r) & 1u;              // reset row: its old frames are not read
 #pragma unroll
           for (int e = 0; e < kPerLane; ++e) {
             const int mt = meta[e];
-            v[i][e] = mt < 0 ? 0.f : ((mt & 0x100) ? o[e * 32 + lane + (mt & 0xff)] : my_new[r * kFrame + mt]);
+            v[i][e] = mt < 0 ? 0.f : ((mt & 0x100) ? (old_zero ? 0.f : o[e * 32 + lane + (mt & 0xff)]) : my_new[r * kFrame + mt]);
           }
         }
       }
@@ -304,13 +313,14 @@ assemble_batch_kernel(const RawStateDev* __restrict__ raw, const float* __restri
 
 // n_obs = 49*H floats per row: 4 elements per lane serve H <= 2, 13 serve H <= 8
 inline void launch_assemble_batch(const RawStateDev* raw, const float* prev_action, float* vel_cmd, float* obs, long long B,
-                                  const CtrlConst& cc, int32_t* button0_out, int sm_count, cudaStream_t st) {
+                                  const CtrlConst& cc, int32_t* button0_out, int sm_count, cudaStream_t st,
+                                  const uint8_t* reset = nullptr) {
   const long long groups = (B + 31) / 32;
   const unsigned grid = (unsigned)std::min<long long>((groups + kAsmWarps - 1) / kAsmWarps, (long long)sm_count * 16);
   if (kFrame * cc.H <= 128)
-    assemble_batch_kernel<4><<<grid, kAsmWarps * 32, 0, st>>>(raw, prev_action, vel_cmd, obs, B, cc, button0_out);
+    assemble_batch_kernel<4><<<grid, kAsmWarps * 32, 0, st>>>(raw, prev_action, vel_cmd, obs, B, cc, button0_out, reset);
   else
-    assemble_batch_kernel<(kFrame * kMaxHistory + 31) / 32><<<grid, kAsmWarps * 32, 0, st>>>(raw, prev_action, vel_cmd, obs, B, cc, button0_out);
+    assemble_batch_kernel<(kFrame * kMaxHistory + 31) / 32><<<grid, kAsmWarps * 32, 0, st>>>(raw, prev_action, vel_cmd, obs, B, cc, button0_out, reset);
 }
 
 }  // namespace go2p

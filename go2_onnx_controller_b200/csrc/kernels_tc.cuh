@@ -75,6 +75,10 @@ struct TcArgs {
   float* vel_cmd;            // [B, 3] last joystick command (in/out)
   int H, foot_threshold;
   unsigned long long* trace;   // debug timeline (GO2P_TC_TRACE): [0] = count, then (event, clock64) pairs; CTA 0 only
+  // fused step with resets (tc_mlp_kernel<., true, true>): [B] per-robot flags.  A robot whose byte is non-zero starts
+  // this step from the controller's initial state (controller.hpp:132-162): older frames, previous action and stored
+  // joystick command 0
+  const uint8_t* reset;
 };
 
 #ifdef GO2P_TC_TRACE
@@ -120,13 +124,14 @@ __device__ __forceinline__ bool any_saturated_f16x2(const uint32_t (&w)[kN]) {
 }
 
 // ---- fused A1-A6: history shift + newest frame of one observation term, in place in the row's shared-memory copy
-// (term-major layout, oldest frame first inside a term: controller.hpp:45-68, controller.cpp:200-212)
+// (term-major layout, oldest frame first inside a term: controller.hpp:45-68, controller.cpp:200-212).  rst: the
+// older frames are the initial state's zeros instead (selected, so whatever the row held -- NaN included -- is dropped)
 template <int kW>
-__device__ __forceinline__ void tc_shift_append(float* term, int H, const float (&cur)[kW]) {
+__device__ __forceinline__ void tc_shift_append(float* term, int H, const float (&cur)[kW], bool rst) {
 #pragma unroll 1
   for (int f = 0; f + 1 < H; ++f) {
 #pragma unroll
-    for (int j = 0; j < kW; ++j) term[f * kW + j] = term[(f + 1) * kW + j];
+    for (int j = 0; j < kW; ++j) term[f * kW + j] = rst ? 0.f : term[(f + 1) * kW + j];
   }
 #pragma unroll
   for (int j = 0; j < kW; ++j) term[(H - 1) * kW + j] = cur[j];
@@ -136,8 +141,10 @@ __device__ __forceinline__ void tc_shift_append(float* term, int H, const float 
 // joystick command, cb 1 joint positions, cb 2 joint velocities, cb 3 previous action / foot contacts (+ the dead-man
 // button for the output job).  Bit-exact rules as in kernels_b1.cuh (same device functions).
 // pa4 (cb 3) / vc (cb 0): the row's previous published action / last joystick command, loaded one job ahead.
+// rst: the row's reset flag (every column block shifts terms, so every one needs it); a reset row's previous action
+// and stored joystick command are 0, and without joystick input the 0 is written back as the row's command.
 __device__ __forceinline__ void tc_update_terms(const TcArgs& a, int cb, float* srow, const uint32_t* rw, long long grow, int* button_out,
-                                                const float4 (&pa4)[3], const float (&vc)[3]) {
+                                                const float4 (&pa4)[3], const float (&vc)[3], bool rst) {
   const float* rf = reinterpret_cast<const float*>(rw);     // this robot's raw state: 39 words (shared-memory stage, or global for a ragged tile)
   const int H = a.H;
   if (cb == 0) {
@@ -152,25 +159,33 @@ __device__ __forceinline__ void tc_update_terms(const TcArgs& a, int cb, float* 
       for (int c = 0; c < 3; ++c) { cmd[c] = vel_cmd_component(axes, c); a.vel_cmd[grow * 3 + c] = cmd[c]; }
     } else {
 #pragma unroll
-      for (int c = 0; c < 3; ++c) cmd[c] = vc[c];
+      for (int c = 0; c < 3; ++c) cmd[c] = rst ? 0.f : vc[c];
+      if (rst) {
+#pragma unroll
+        for (int c = 0; c < 3; ++c) a.vel_cmd[grow * 3 + c] = 0.f;
+      }
     }
-    tc_shift_append<3>(srow, H, g);
-    tc_shift_append<3>(srow + 3 * H, H, w);
-    tc_shift_append<3>(srow + 6 * H, H, cmd);
+    tc_shift_append<3>(srow, H, g, rst);
+    tc_shift_append<3>(srow + 3 * H, H, w, rst);
+    tc_shift_append<3>(srow + 6 * H, H, cmd, rst);
   } else if (cb == 1) {
     float q[kDof];
 #pragma unroll
     for (int c = 0; c < kDof; ++c) q[c] = __double2float_rn(__dsub_rn((double)rf[7 + c], a.q0[c]));   // controller.cpp:194-197
-    tc_shift_append<kDof>(srow + 9 * H, H, q);
+    tc_shift_append<kDof>(srow + 9 * H, H, q, rst);
   } else if (cb == 2) {
     float dq[kDof];
 #pragma unroll
     for (int c = 0; c < kDof; ++c) dq[c] = rf[19 + c];
-    tc_shift_append<kDof>(srow + 21 * H, H, dq);
+    tc_shift_append<kDof>(srow + 21 * H, H, dq, rst);
   } else {
     float pa[kDof];                                                               // previous published action
 #pragma unroll
     for (int q = 0; q < 3; ++q) { const float4 t = pa4[q]; pa[4 * q] = t.x; pa[4 * q + 1] = t.y; pa[4 * q + 2] = t.z; pa[4 * q + 3] = t.w; }
+    if (rst) {
+#pragma unroll
+      for (int c = 0; c < kDof; ++c) pa[c] = 0.f;
+    }
     float ct[4];
 #pragma unroll
     for (int c = 0; c < 4; ++c) {
@@ -178,8 +193,8 @@ __device__ __forceinline__ void tc_update_terms(const TcArgs& a, int cb, float* 
       const int force = (int)(int16_t)(uint16_t)(rw[35 + (p >> 1)] >> (16 * (p & 1)));
       ct[c] = (force >= a.foot_threshold) ? 1.0f : 0.0f;
     }
-    tc_shift_append<kDof>(srow + 33 * H, H, pa);
-    tc_shift_append<4>(srow + 45 * H, H, ct);
+    tc_shift_append<kDof>(srow + 33 * H, H, pa, rst);
+    tc_shift_append<4>(srow + 45 * H, H, ct, rst);
     *button_out = (int)rw[38];
   }
 }
@@ -298,8 +313,11 @@ __device__ __noinline__ void tc_out_generic(const TcArgs& a, uint32_t o_t, long 
   if ((a.flags & 4u) && a.cmd) store_gains(a.cmd, row, b0, a.kp, a.kd, a.kp_deadman);
 }
 
-template <bool kFp16, bool kFused>
+// kReset (fused step only): the step reads a.reset.  A separate instantiation, so that the step without a mask runs
+// exactly the code it ran before resets existed (the per-element selects cost 2 % even when every flag is 0).
+template <bool kFp16, bool kFused, bool kReset = false>
 __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_constant__ TcArgs a) {
+  static_assert(kFused || !kReset, "resets belong to the fused controller step");
   extern __shared__ __align__(128) uint8_t smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 
@@ -500,9 +518,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
     // NEXT conversion job, requested in the output job that precedes it (global loads, ~1 us under load)
     float4 pf_act[3] = {make_float4(0.f, 0.f, 0.f, 0.f), make_float4(0.f, 0.f, 0.f, 0.f), make_float4(0.f, 0.f, 0.f, 0.f)};
     float pf_vel[3] = {0.f, 0.f, 0.f};
+    bool pf_rst = false;                                  // kReset: the row's reset flag (every column block)
     auto prefetch_state = [&](int pair, int s) {          // for conv_job(pair, s)
       const long long row = (blockIdx.x + (long long)(pair * 2 + s) * gridDim.x) * kTcTileM + m;
+      pf_rst = false;
       if (row < a.B) {
+        if constexpr (kReset) pf_rst = a.reset[row] != 0;
         if (cb == 3) {
           const float4* p4 = reinterpret_cast<const float4*>(a.act + row * kDof);
 #pragma unroll
@@ -537,7 +558,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
           tc_term_range(cb, a.H, lo, hi);
           if (!full) for (int k = lo; k < hi; ++k) srow[k] = a.obs_rw[(row0 + m) * a.in_dim + k];   // ragged tile: no bulk load
           const uint32_t* rw = full ? s_raw + m * kTcRawWords : reinterpret_cast<const uint32_t*>(a.raw + row0 + m);
-          tc_update_terms(a, cb, srow, rw, row0 + m, &s_button[(s * 2 + (pair & 1)) * kTcTileM + m], pf_act, pf_vel);
+          tc_update_terms(a, cb, srow, rw, row0 + m, &s_button[(s * 2 + (pair & 1)) * kTcTileM + m], pf_act, pf_vel,
+                          pf_rst);
           if (!full) for (int k = lo; k < hi; ++k) a.obs_rw[(row0 + m) * a.in_dim + k] = srow[k];
         }
         TC_TRACE(0xB00u | (uint32_t)s);

@@ -213,6 +213,17 @@ int go2p_infer_batch_cmd(go2p_handle* h, const float* d_obs, const int32_t* d_bu
 int go2p_step_batch_cmd(go2p_handle* h, const go2p_raw_state* d_raw, float* d_vel_cmd, float* d_obs,
                         float* d_action, double* d_qdes, go2p_motor_cmd* d_cmd, int64_t B,
                         int precision, void* stream);
+/* go2p_step_batch_cmd with per-robot resets, for fleets whose robots end their episodes at different times.
+ * d_reset [B] uint8 on the device (NULL = no resets, any alignment; a torch.bool tensor qualifies).  A robot whose
+ * byte is non-zero starts this step from the controller's initial state (controller.hpp:132-162): its H-1 older frames
+ * of every term are 0, its previous action is 0 and its stored joystick command is 0; then the step runs as usual (the
+ * newest frame is appended; without joy_valid its command is 0, and 0 is written back to d_vel_cmd).  Its outputs do not
+ * depend on what its rows of d_obs / d_vel_cmd / d_action held on entry (NaN included).  Robots with a zero byte step
+ * exactly as with go2p_step_batch_cmd, which is this call with d_reset = NULL.  Same argument rules and launch count
+ * as go2p_step_batch_cmd. */
+int go2p_step_batch_ex(go2p_handle* h, const go2p_raw_state* d_raw, const uint8_t* d_reset, float* d_vel_cmd,
+                       float* d_obs, float* d_action, double* d_qdes, go2p_motor_cmd* d_cmd, int64_t B,
+                       int precision, void* stream);
 /* go2p_step_fused + the same step's send_command arguments in motor order (out may be NULL) */
 int go2p_step_fused_cmd(go2p_handle* h, const go2p_raw_state* raw, go2p_step_out* out, go2p_motor_cmd* cmd);
 /* isaac_of_motor[u] = Isaac joint index of Unitree motor u */
@@ -224,6 +235,10 @@ int go2p_motor_order(int32_t isaac_of_motor[GO2P_DOF]);
 int go2p_step_batch_host(go2p_handle* h, const go2p_raw_state* h_raw, float* h_action, go2p_motor_cmd* h_cmd,
                          int64_t B, int precision);
 int go2p_step_batch_host_reset(go2p_handle* h);
+/* go2p_step_batch_host with per-robot resets (the rule of go2p_step_batch_ex) applied to the state the handle keeps:
+ * h_reset [B] uint8 in host memory, NULL = no resets.  1 B more per robot on the way in. */
+int go2p_step_batch_host_ex(go2p_handle* h, const go2p_raw_state* h_raw, const uint8_t* h_reset, float* h_action,
+                            go2p_motor_cmd* h_cmd, int64_t B, int precision);
 /* fp16 operands saturate at +-65504 where the fp32 reference does not.  Launches with GO2P_F_SAT_COUNT count the
  * (row, 32-column operand block) pairs in which an observation or a hidden activation was clipped on its way into a
  * Gemm; this reads (and optionally resets) the total once `stream` has drained.  0 means the fp16 path never left the
@@ -253,6 +268,9 @@ int go2p_shard_rows(int64_t B, int n, int i, int64_t* begin, int64_t* end);
 int go2p_fleet_infer_host(go2p_fleet* f, const float* h_obs, float* h_act, int64_t B, int precision);
 int go2p_fleet_step_host(go2p_fleet* f, const go2p_raw_state* h_raw, float* h_action, go2p_motor_cmd* h_cmd,
                          int64_t B, int precision);
+/* + per-robot resets (go2p_step_batch_host_ex): h_reset [B] uint8 in host memory, NULL = no resets, sharded like h_raw */
+int go2p_fleet_step_host_ex(go2p_fleet* f, const go2p_raw_state* h_raw, const uint8_t* h_reset, float* h_action,
+                            go2p_motor_cmd* h_cmd, int64_t B, int precision);
 
 /* ---- small device / pinned-memory helpers so non-CUDA hosts can drive the batched path ---- */
 int go2p_dev_alloc(go2p_handle* h, size_t bytes, void** dptr);

@@ -1,5 +1,6 @@
 """Timeline of one CTA of tc_mlp_kernel (trace build: -DGO2P_TC_TRACE, lib/libgo2policy_trace.so).
-usage: tc_trace.py [rows] [first event] [count] [warps, comma separated]"""
+usage: tc_trace.py [rows] [first event] [count] [warps, comma separated]
+GO2P_TRACE_STEP=1 traces the fused controller step; GO2P_TRACE_RESET=p adds a mask resetting a fraction p of the robots."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -31,11 +32,15 @@ if FUSED:
     d_raw = torch.from_numpy(np.tile(raw_np, (B // 4096, 1)).copy()).cuda()
     d_obs = torch.zeros((B, 98), device="cuda"); d_vel = torch.zeros((B, 3), device="cuda")
     d_act = torch.zeros((B, 12), device="cuda"); d_q = torch.zeros((B, 12), device="cuda", dtype=torch.float64)
+    # GO2P_TRACE_RESET=p: the step with per-robot resets (go2p_step_batch_ex), a fraction p of the robots reset
+    RESET = float(os.environ["GO2P_TRACE_RESET"]) if os.environ.get("GO2P_TRACE_RESET") else None
+    d_rst = (torch.rand(B, device="cuda", generator=torch.Generator(device="cuda").manual_seed(5)) < RESET) if RESET is not None else None
 for _ in range(3):
     trace.zero_()
     torch.cuda.synchronize()
     if FUSED:
-        pb.step_device(d_raw.data_ptr(), d_vel.data_ptr(), d_obs.data_ptr(), d_act.data_ptr(), d_q.data_ptr(), B, capi.PREC_FP16)
+        pb.step_device(d_raw.data_ptr(), d_vel.data_ptr(), d_obs.data_ptr(), d_act.data_ptr(), d_q.data_ptr(), B, capi.PREC_FP16,
+                       d_reset=None if d_rst is None else d_rst.data_ptr())
     else:
         pb.infer_device(d_obs.data_ptr(), d_act.data_ptr(), B, capi.PREC_FP16)
     torch.cuda.synchronize()
