@@ -47,6 +47,16 @@ class _Handle:
         self.output_name = info.output_name.decode()
         self.dims = [info.dims[i] for i in range(info.n_layers + 1)]
 
+    def set_weights(self, weights, biases, obs_mean, obs_std, stream: int, host_only: bool) -> None:
+        kind = weight_arrays(self.dims, weights, biases, obs_mean, obs_std, device=self.cfg.device)
+        if host_only and kind != "host":
+            raise TypeError("this form takes numpy arrays (host memory)")
+        w, b = _ptr_array(weights), (_ptr_array(biases) if biases is not None else None)
+        if kind == "host":
+            capi.check(self.lib.go2p_set_weights_host(self.h, w, b, len(weights), _ptr(obs_mean), _ptr(obs_std)))
+        else:
+            capi.check(self.lib.go2p_set_weights(self.h, w, b, len(weights), _ptr(obs_mean), _ptr(obs_std), stream or None))
+
     def close(self):
         if self.h:
             self.lib.go2p_destroy(self.h)
@@ -70,6 +80,69 @@ def host_reset_mask(reset, B: int) -> np.ndarray:
     if not reset.flags.c_contiguous:
         raise ValueError("reset must be C-contiguous")
     return reset
+
+
+def _is_device_tensor(a) -> bool:
+    """A torch-like tensor (duck-typed: this package does not import torch)."""
+    return all(hasattr(a, x) for x in ("data_ptr", "is_contiguous", "device"))
+
+
+def weight_arrays(dims, weights, biases=None, obs_mean=None, obs_std=None, device: int | None = None) -> str:
+    """Validates a set_weights() argument list against a policy's layer widths ``dims`` ([in, h1, ..., out]) before any
+    native call.  weights[l]: float32 [dims[l+1], dims[l]] (torch nn.Linear.weight layout), biases: None or a list with
+    float32 [dims[l+1]] or None per layer, obs_mean / obs_std: float32 [dims[0]], both or neither.  Every array is a
+    C-contiguous numpy array (host form) or every one a contiguous CUDA tensor on device ``device`` (device form);
+    the two are not mixed.  Returns "host" or "device"; raises TypeError / ValueError."""
+    n = len(dims) - 1
+    if not isinstance(weights, (list, tuple)):
+        raise TypeError(f"weights must be a list of {n} arrays, got {type(weights).__name__}")
+    if len(weights) != n:
+        raise ValueError(f"weights has {len(weights)} layers, the policy has {n}")
+    if biases is not None:
+        if not isinstance(biases, (list, tuple)):
+            raise TypeError(f"biases must be None or a list of {n} arrays, got {type(biases).__name__}")
+        if len(biases) != n:
+            raise ValueError(f"biases has {len(biases)} layers, the policy has {n}")
+    if (obs_mean is None) != (obs_std is None):
+        raise ValueError("obs_mean and obs_std go together")
+    named = [(f"weights[{l}]", w, (dims[l + 1], dims[l])) for l, w in enumerate(weights)]
+    named += [(f"biases[{l}]", b, (dims[l + 1],)) for l, b in enumerate(biases or []) if b is not None]
+    if obs_mean is not None:
+        named += [("obs_mean", obs_mean, (dims[0],)), ("obs_std", obs_std, (dims[0],))]
+    kinds = set()
+    for name, a, shape in named:
+        if isinstance(a, np.ndarray):
+            kinds.add("host")
+            if a.dtype != np.float32:
+                raise TypeError(f"{name} must be float32, got {a.dtype}")
+            contiguous = a.flags.c_contiguous
+        elif _is_device_tensor(a):
+            kinds.add("device")
+            if str(a.dtype) != "torch.float32":
+                raise TypeError(f"{name} must be float32, got {a.dtype}")
+            if getattr(a.device, "type", None) != "cuda":
+                raise TypeError(f"{name} is a tensor on {a.device}: pass a CUDA tensor or a numpy array")
+            if device is not None and a.device.index != device:
+                raise ValueError(f"{name} is on cuda:{a.device.index}, the handle on cuda:{device}")
+            contiguous = a.is_contiguous()
+        else:
+            raise TypeError(f"{name} must be a numpy array or a CUDA tensor, got {type(a).__name__}")
+        if tuple(a.shape) != shape:
+            raise ValueError(f"{name} must have shape {shape}, got {tuple(a.shape)}")
+        if not contiguous:
+            raise ValueError(f"{name} must be C-contiguous")
+    if len(kinds) > 1:
+        raise TypeError("host (numpy) and device (CUDA tensor) arrays cannot be mixed in one update")
+    return kinds.pop()
+
+
+def _ptr(a):
+    return None if a is None else (a.ctypes.data if isinstance(a, np.ndarray) else a.data_ptr())
+
+
+def _ptr_array(arrays):
+    """Host array of pointers (NULL for None), as go2p_set_weights* read them."""
+    return (C.c_void_p * len(arrays))(*[_ptr(a) for a in arrays])
 
 
 class ONNXActor:
@@ -168,6 +241,11 @@ class Go2Controller:
 
     def set_gains(self, kp: float, kd: float) -> None:
         capi.check(self._hd.lib.go2p_set_gains(self._hd.h, kp, kd))
+
+    def set_weights(self, weights, biases=None, obs_mean=None, obs_std=None) -> None:
+        """Replace the policy's weights (numpy float32 arrays; see PolicyBatch.set_weights).  The controller's history,
+        previous action, joystick command and gains carry over to the next step."""
+        self._hd.set_weights(weights, biases, obs_mean, obs_std, 0, host_only=True)
 
     def stop(self) -> None:
         capi.check(self._hd.lib.go2p_persistent_stop(self._hd.h))
@@ -272,6 +350,15 @@ class PolicyBatch:
     def step_host_reset(self) -> None:
         capi.check(self._hd.lib.go2p_step_batch_host_reset(self._hd.h))
 
+    def set_weights(self, weights, biases=None, obs_mean=None, obs_std=None, stream: int = 0) -> None:
+        """Replace the weights of every layer; the topology stays.  weights[l]: float32 [dims[l+1], dims[l]] (the layout
+        of torch nn.Linear.weight), biases: None or float32 [dims[l+1]] (None) per layer, obs_mean / obs_std: float32
+        [in_dim], both or neither, an observation normaliser (x - mean) / std folded into the first layer.
+        numpy arrays: synchronous (go2p_set_weights_host).  CUDA tensors on the handle's device: packed on the device,
+        ordered on ``stream`` (go2p_set_weights); keep them alive until the stream has passed the update.  Robot state
+        kept by the handle (step_host, the batch-1 controller) carries over."""
+        self._hd.set_weights(weights, biases, obs_mean, obs_std, stream, host_only=False)
+
     def close(self) -> None:
         self._hd.close()
 
@@ -287,6 +374,7 @@ class Fleet:
         dev = (C.c_int32 * len(devices))(*devices)
         capi.check(self.lib.go2p_fleet_create(os.fspath(model_path).encode(), C.byref(c), dev, len(devices), C.byref(self.f)))
         self.n_devices = len(devices)
+        self.model_path = os.fspath(model_path)
 
     def infer_host(self, obs: np.ndarray, act: np.ndarray, precision: int = capi.PREC_FP32) -> None:
         capi.check(self.lib.go2p_fleet_infer_host(self.f, obs.ctypes.data, act.ctypes.data, obs.shape[0], precision))
@@ -301,6 +389,16 @@ class Fleet:
             reset = host_reset_mask(reset, raw.shape[0])
             capi.check(self.lib.go2p_fleet_step_host_ex(self.f, raw.ctypes.data, reset.ctypes.data, action.ctypes.data, cmd_p,
                                                         raw.shape[0], precision))
+
+    def set_weights(self, weights, biases=None, obs_mean=None, obs_std=None) -> None:
+        """PolicyBatch.set_weights with numpy arrays, on every device of the fleet (go2p_fleet_set_weights_host)."""
+        info = capi.ModelInfo()
+        capi.check(self.lib.go2p_inspect_model(self.model_path.encode(), C.byref(info), None))
+        if weight_arrays([info.dims[i] for i in range(info.n_layers + 1)], weights, biases, obs_mean, obs_std) != "host":
+            raise TypeError("Fleet.set_weights takes numpy arrays (host memory)")
+        capi.check(self.lib.go2p_fleet_set_weights_host(self.f, _ptr_array(weights),
+                                                        _ptr_array(biases) if biases is not None else None, len(weights),
+                                                        _ptr(obs_mean), _ptr(obs_std)))
 
     def close(self) -> None:
         if self.f:

@@ -114,6 +114,12 @@ SIGNATURES = {
     "go2p_fleet_infer_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int]),
     "go2p_fleet_step_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int]),
     "go2p_fleet_step_host_ex": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int]),
+    "go2p_set_weights": (C.c_int, [_H, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_int, C.c_void_p, C.c_void_p,
+                                   C.c_void_p]),
+    "go2p_set_weights_host": (C.c_int, [_H, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_int, C.c_void_p,
+                                        C.c_void_p]),
+    "go2p_fleet_set_weights_host": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_int,
+                                              C.c_void_p, C.c_void_p]),
     "go2p_dev_alloc": (C.c_int, [_H, C.c_size_t, C.POINTER(C.c_void_p)]),
     "go2p_dev_free": (C.c_int, [_H, C.c_void_p]),
     "go2p_host_alloc": (C.c_int, [_H, C.c_size_t, C.POINTER(C.c_void_p)]),

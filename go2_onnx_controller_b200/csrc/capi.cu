@@ -25,6 +25,7 @@
 #include "kernels_fp32.cuh"
 #include "kernels_tc.cuh"
 #include "kernels_wide.cuh"
+#include "kernels_pack.cuh"   // after the step-path kernels: their instantiation order (and SASS) stays as it was
 #include "onnx_reader.hpp"
 
 using namespace go2p;
@@ -72,6 +73,9 @@ struct go2p_handle {
   bool wide_ok = false;
   uint16_t* d_wpack[2] = {nullptr, nullptr};   // [0] bf16, [1] fp16
   int k0p = 0;
+  size_t tc_off[kMaxLayers] = {};              // layer l's image starts tc_off[l] elements into d_wpack[0] / [1]
+  int tc_kp[kMaxLayers] = {};
+  double tc_wscale[kMaxLayers] = {}, tc_bscale[kMaxLayers] = {};   // the scales pack_umma_kmajor applied
   size_t tc_attr_smem[6] = {};                 // dynamic shared memory opted in for tc_mlp_kernel<bf16|fp16, plain|fused|fused+reset> on this device
   bool b1_attr_set = false;                    // same for the one-shot batch-1 kernel
   size_t so_attr_smem = 0;                     // same for small_out_kernel
@@ -106,6 +110,13 @@ struct go2p_handle {
   float* pipe_out[kPipeDepth] = {};
   int last_launches = 0;
   unsigned long long* d_sat = nullptr;         // GO2P_F_SAT_COUNT: saturated fp16 operand blocks since the last read
+  // go2p_set_weights: w_gen counts updates; tc_w_gen is the update the first tensor-core launch on w_stream (the
+  // stream of the last update) has seen.  w_event marks the end of the last update's packer.
+  uint64_t w_gen = 0, tc_w_gen = 0;
+  cudaStream_t w_stream = nullptr;
+  cudaEvent_t w_event = nullptr;
+  float* w_fold = nullptr;                     // layer 0 with the observation normaliser folded in
+  float* w_stage = nullptr;                    // go2p_set_weights_host: the caller's tensors on the device
   // ObservationAction ring (go2p_log_enable)
   LogRing* d_log = nullptr;
   uint32_t log_capacity = 0;
@@ -241,6 +252,8 @@ int upload_model(go2p_handle* h) {
       const int Kp = l == 0 ? h->k0p : kTcHidden + kTcBiasK;
       const int Np = l == dm.n_layers - 1 ? kTcOutPad : kTcHidden;
       const double out_scale = m.layers[l].has_elu ? kLog2e : 1.0;
+      h->tc_off[l] = wb.size(); h->tc_kp[l] = Kp;
+      h->tc_wscale[l] = out_scale / in_scale; h->tc_bscale[l] = out_scale;
       pack_umma_kmajor(m.layers[l], Np, Kp, false, out_scale / in_scale, out_scale, wb);
       pack_umma_kmajor(m.layers[l], Np, Kp, true, out_scale / in_scale, out_scale, wf);
       in_scale = out_scale;
@@ -470,14 +483,19 @@ int launch_tc_t(go2p_handle* h, const TcArgs& a, cudaStream_t st) {
   const long long tiles = (a.B + kTcTileM - 1) / kTcTileM;
   int grid = (int)std::min<long long>(tiles, h->sm_count - (h->resident ? 1 : 0));
   // programmatic stream serialization: the kernel's prologue may overlap the tail of the previous kernel of the stream
-  // (it waits for that kernel before touching observations / actions: griddepcontrol.wait in tc_mlp_kernel)
+  // (it waits for that kernel before touching observations / actions: griddepcontrol.wait in tc_mlp_kernel).  The
+  // prologue also issues the weights' bulk copies, so the first launch on the stream of a weight update goes without
+  // it: its previous kernel may be the packer (go2p_set_weights).  Other streams reach the new weights through an
+  // event or a host synchronisation, which programmatic serialization does not relax.
+  const bool after_update = h->tc_w_gen != h->w_gen && st == h->w_stream;
   cudaLaunchConfig_t lc{};
   lc.gridDim = dim3((unsigned)grid); lc.blockDim = dim3(kTcThreads); lc.dynamicSmemBytes = smem; lc.stream = st;
   cudaLaunchAttribute attr{};
   attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr.val.programmaticStreamSerializationAllowed = 1;
-  lc.attrs = &attr; lc.numAttrs = 1;
+  lc.attrs = &attr; lc.numAttrs = after_update ? 0 : 1;
   CU_TRY(cudaLaunchKernelEx(&lc, kernel, a));
+  if (after_update) h->tc_w_gen = h->w_gen;
   h->last_launches++;
   CU_TRY(cudaGetLastError());
   return GO2P_OK;
@@ -666,6 +684,7 @@ int go2p_destroy(go2p_handle* h) {
     if (h->pipe_out[i]) cudaFree(h->pipe_out[i]);
   }
   if (h->b1_stream) cudaStreamDestroy(h->b1_stream);
+  if (h->w_event) cudaEventDestroy(h->w_event);
   for (void* p : h->dev_owned) cudaFree(p);
   wide_release(&h->wide);
   for (auto& sc : h->scratch_sets)
@@ -1189,6 +1208,136 @@ int go2p_step_batch_host_reset(go2p_handle* h) {
   return GO2P_OK;
 }
 
+// ------------------------------------------------------------------------------------- weight updates
+namespace {
+int check_weight_args(const char* fn, const go2p_handle* h, const float* const* w, int n_layers, const float* mean,
+                      const float* stdv) {
+  const std::string f(fn);
+  if (!h) return fail(GO2P_ERR_INVALID, f + ": null handle");
+  if (n_layers != h->dm.n_layers)
+    return fail(GO2P_ERR_INVALID, f + ": n_layers " + std::to_string(n_layers) + " does not match the handle's " +
+                                      std::to_string(h->dm.n_layers));
+  if (!w) return fail(GO2P_ERR_INVALID, f + ": null weight array");
+  for (int l = 0; l < n_layers; ++l)
+    if (!w[l]) return fail(GO2P_ERR_INVALID, f + ": null weight pointer for layer " + std::to_string(l));
+  if ((mean == nullptr) != (stdv == nullptr)) return fail(GO2P_ERR_INVALID, f + ": obs_mean and obs_std go together");
+  return GO2P_OK;
+}
+
+// Before the packer touches the images: the resident batch-1 kernel (which holds the weights in registers or shared
+// memory) is stopped -- it saves its state to d_state and is relaunched lazily by the next batch-1 call -- and `st`
+// waits for whatever the handle's own streams have queued, the previous update's packer included.
+int begin_update(go2p_handle* h, cudaStream_t st) {
+  if (h->resident) { const int rc = go2p_persistent_stop(h); if (rc) return rc; }
+  if (!h->w_event) CU_TRY(cudaEventCreateWithFlags(&h->w_event, cudaEventDisableTiming));
+  cudaStream_t own[1 + kPipeDepth] = {h->b1_stream};
+  for (int i = 0; i < kPipeDepth; ++i) own[1 + i] = h->pipe_stream[i];
+  for (cudaStream_t s : own) {
+    if (s == st) continue;
+    CU_TRY(cudaEventRecord(h->w_event, s));
+    CU_TRY(cudaStreamWaitEvent(st, h->w_event, 0));
+  }
+  return GO2P_OK;
+}
+
+// The packer (kernels_pack.cuh) on `st`, then the handle's own streams wait for it: a batch-1 call or a host-buffer
+// step issued after this returns computes with the new weights without a host synchronisation.
+int pack_and_publish(go2p_handle* h, const float* const* w, const float* const* b, const float* mean, const float* stdv,
+                     cudaStream_t st) {
+  const DevModel& dm = h->dm;
+  PackArgs pa{};
+  pa.n_layers = dm.n_layers;
+  long long widest = 0;
+  for (int l = 0; l < dm.n_layers; ++l) {
+    const DevLayer& D = dm.L[l];
+    PackLayer& P = pa.L[l];
+    P.w = w[l]; P.b = b ? b[l] : nullptr;
+    P.K = D.K; P.N = D.N; P.Kp = D.Kp; P.Np = D.Np;
+    P.w_rm = const_cast<float*>(D.w_rm); P.w_k4 = const_cast<float*>(D.w_k4);
+    P.w_kn = const_cast<float*>(D.w_kn); P.bias = const_cast<float*>(D.bias);
+    if (h->tc_ok) {
+      for (int f = 0; f < 2; ++f) P.tc[f] = h->d_wpack[f] + h->tc_off[l];
+      P.tc_Kp = h->tc_kp[l]; P.wscale = h->tc_wscale[l]; P.bscale = h->tc_bscale[l];
+    }
+    if (h->wide_ok) {
+      const WideLayerDev& W = h->wide.L[l];
+      for (int f = 0; f < 2; ++f) P.wd[f] = const_cast<uint16_t*>(W.w[f]);
+      P.wd_bias = const_cast<float*>(W.bias); P.wd_NT = W.NT; P.wd_Kp = W.Kp;
+    }
+    widest = std::max<long long>(widest, (long long)D.N * (D.K + 1));
+  }
+  if (mean) {
+    const int K = dm.L[0].K, N = dm.L[0].N;
+    if (!h->w_fold) {
+      CU_TRY(cudaMalloc((void**)&h->w_fold, ((size_t)N * K + N) * sizeof(float)));
+      h->dev_owned.push_back(h->w_fold);
+    }
+    fold_normaliser_kernel<<<(N + 127) / 128, 128, 0, st>>>(w[0], b ? b[0] : nullptr, mean, stdv, K, N, h->w_fold,
+                                                           h->w_fold + (size_t)N * K);
+    CU_TRY(cudaGetLastError());
+    pa.L[0].w = h->w_fold;
+    pa.L[0].b = h->w_fold + (size_t)N * K;
+  }
+  const int blocks = (int)std::min<long long>((widest + 255) / 256, (long long)h->sm_count * 4);
+  pack_weights_kernel<<<dim3((unsigned)blocks, (unsigned)dm.n_layers), 256, 0, st>>>(pa);
+  CU_TRY(cudaGetLastError());
+  CU_TRY(cudaEventRecord(h->w_event, st));
+  cudaStream_t own[1 + kPipeDepth] = {h->b1_stream};
+  for (int i = 0; i < kPipeDepth; ++i) own[1 + i] = h->pipe_stream[i];
+  for (cudaStream_t s : own)
+    if (s != st) CU_TRY(cudaStreamWaitEvent(s, h->w_event, 0));
+  ++h->w_gen;
+  h->w_stream = st;
+  return GO2P_OK;
+}
+}  // namespace
+
+int go2p_set_weights(go2p_handle* h, const float* const* d_weight, const float* const* d_bias, int n_layers,
+                     const float* d_obs_mean, const float* d_obs_std, void* stream) {
+  int rc = check_weight_args("go2p_set_weights", h, d_weight, n_layers, d_obs_mean, d_obs_std);
+  if (rc) return rc;
+  DeviceGuard g(h->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if ((rc = begin_update(h, st))) return rc;
+  return pack_and_publish(h, d_weight, d_bias, d_obs_mean, d_obs_std, st);
+}
+
+int go2p_set_weights_host(go2p_handle* h, const float* const* h_weight, const float* const* h_bias, int n_layers,
+                          const float* h_obs_mean, const float* h_obs_std) {
+  int rc = check_weight_args("go2p_set_weights_host", h, h_weight, n_layers, h_obs_mean, h_obs_std);
+  if (rc) return rc;
+  DeviceGuard g(h->device);
+  const DevModel& dm = h->dm;
+  size_t floats = 2 * (size_t)dm.in_dim;
+  for (int l = 0; l < dm.n_layers; ++l) floats += (size_t)dm.L[l].N * dm.L[l].K + dm.L[l].N;
+  if (!h->w_stage) {       // the topology is fixed, so is the size
+    CU_TRY(cudaMalloc((void**)&h->w_stage, floats * sizeof(float)));
+    h->dev_owned.push_back(h->w_stage);
+  }
+  cudaStream_t st = h->pipe_stream[0];
+  if ((rc = begin_update(h, st))) return rc;
+  const float* dw[kMaxLayers] = {};
+  const float* db[kMaxLayers] = {};
+  float* p = h->w_stage;
+  auto stage = [&](const float* src, size_t n, const float** dst) -> int {
+    CU_TRY(cudaMemcpyAsync(p, src, n * sizeof(float), cudaMemcpyHostToDevice, st));
+    *dst = p;
+    p += n;
+    return GO2P_OK;
+  };
+  for (int l = 0; l < dm.n_layers; ++l) {
+    if ((rc = stage(h_weight[l], (size_t)dm.L[l].N * dm.L[l].K, &dw[l]))) return rc;
+    if (h_bias && h_bias[l] && (rc = stage(h_bias[l], (size_t)dm.L[l].N, &db[l]))) return rc;
+  }
+  const float *dmean = nullptr, *dstd = nullptr;
+  if (h_obs_mean && ((rc = stage(h_obs_mean, (size_t)dm.in_dim, &dmean)) || (rc = stage(h_obs_std, (size_t)dm.in_dim, &dstd))))
+    return rc;
+  if ((rc = pack_and_publish(h, dw, db, dmean, dstd, st))) return rc;
+  CU_TRY(cudaStreamSynchronize(st));
+  h->tc_w_gen = h->w_gen;   // the packer has completed: no later launch can overlap it
+  return GO2P_OK;
+}
+
 // ------------------------------------------------------------------------------------- ObservationAction log
 int go2p_log_enable(go2p_handle* h, int capacity) {
   if (!h || capacity < 0) return fail(GO2P_ERR_INVALID, "go2p_log_enable: bad argument");
@@ -1299,6 +1448,16 @@ int go2p_fleet_step_host_ex(go2p_fleet* f, const go2p_raw_state* h_raw, const ui
 int go2p_fleet_step_host(go2p_fleet* f, const go2p_raw_state* h_raw, float* h_action, go2p_motor_cmd* h_cmd, int64_t B,
                          int precision) {
   return go2p_fleet_step_host_ex(f, h_raw, nullptr, h_action, h_cmd, B, precision);
+}
+
+int go2p_fleet_set_weights_host(go2p_fleet* f, const float* const* h_weight, const float* const* h_bias, int n_layers,
+                                const float* h_obs_mean, const float* h_obs_std) {
+  if (!f || f->handles.empty()) return fail(GO2P_ERR_INVALID, "go2p_fleet_set_weights_host: null fleet");
+  for (size_t i = 0; i < f->handles.size(); ++i) {
+    const int rc = go2p_set_weights_host(f->handles[i], h_weight, h_bias, n_layers, h_obs_mean, h_obs_std);
+    if (rc) return fail(rc, "device " + std::to_string(i) + ": " + g_err);
+  }
+  return GO2P_OK;
 }
 
 // ------------------------------------------------------------------------------------- helpers

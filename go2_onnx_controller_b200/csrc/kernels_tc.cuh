@@ -366,9 +366,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
   block_sync();
   ptx::tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
-  // Programmatic dependent launch: everything above (barriers, TMEM, the weights' bulk copies -- the weights never
-  // change after go2p_create) may run while the previous kernel of the stream drains; observations are read and
-  // actions written only after that kernel has completed.  The next launch may start its own prologue as soon as
+  // Programmatic dependent launch: everything above (barriers, TMEM, the weights' bulk copies) may run while the
+  // previous kernel of the stream drains; observations are read and actions written only after that kernel has
+  // completed.  The weights are read before the wait, so the previous kernel must not be one that writes them: the
+  // host launches the first tensor-core kernel after a weight update (go2p_set_weights) on the update's stream without
+  // programmatic serialization (capi.cu: launch_tc_t).  The next launch may start its own prologue as soon as
   // this CTA's SM is free (a short batch per GPU, e.g. 1/8 of a sharded step, is otherwise launch-gap bound).
 #if GO2P_TC_WARM_L2
   // While the previous kernel drains, pull this CTA's first two observation slabs into L2 (prefetch only: L2 is the

@@ -181,7 +181,10 @@ __global__ void __launch_bounds__(kWdThreads, 1) wide_gemm_kernel(const WideGemm
   // Programmatic dependent launch: barriers and TMEM are set up while the previous layer's launch drains; its
   // activations are read (and the buffer two layers back is overwritten) only after that launch has completed.  The
   // next layer's launch may begin its own set-up as soon as this CTA's SM is free.  (5 launches per 18,944-row pass:
-  // the gaps between them were a quarter of the wide policy's time.)
+  // the gaps between them were a quarter of the wide policy's time.)  Weights and biases, like activations, are read
+  // only after the wait (the producer warp's bulk copies and the epilogue's bias loads below), so a launch may follow
+  // the weight packer of go2p_set_weights on the same stream with programmatic serialization; obs_to_blocked_kernel
+  // reads no weights at all.
   ptx::grid_dependency_wait();
   ptx::grid_launch_dependents();
 

@@ -239,6 +239,34 @@ int go2p_step_batch_host_reset(go2p_handle* h);
  * h_reset [B] uint8 in host memory, NULL = no resets.  1 B more per robot on the way in. */
 int go2p_step_batch_host_ex(go2p_handle* h, const go2p_raw_state* h_raw, const uint8_t* h_reset, float* h_action,
                             go2p_motor_cmd* h_cmd, int64_t B, int precision);
+/* ---- replacing the policy weights of a live handle (a new checkpoint, a running observation normaliser, an A/B
+ * comparison) without losing robot state.
+ * Replace the weights and biases of every layer.  The topology of the handle is fixed at create: n_layers, dims,
+ * activations and ELU alpha must match.
+ * weight[l]: [dims[l+1]][dims[l]] fp32 row-major (the layout of torch nn.Linear.weight and of ONNX Gemm transB=1).
+ * bias[l]: [dims[l+1]] fp32, or NULL for zeros (the bias array itself may be NULL: every bias zero).
+ * obs_mean / obs_std: [in_dim] fp32 or both NULL.  They describe an observation normaliser x' = (x - mean) / std and are
+ *   folded into layer 0 exactly as the reader folds a Sub(mean) -> Div(std) prefix.
+ * After the call, every path computes what a handle created from an .onnx holding these tensors would compute, bit for
+ *   bit.  Robot state is untouched: batch-1 history, the host-step fleet state, caller buffers, gains, log ring and
+ *   saturation counter.
+ * The pointer arrays are host arrays.  GO2P_ERR_INVALID: null handle, n_layers that does not match, a null weight
+ * pointer, or exactly one of mean / std given.
+ *
+ * go2p_set_weights: the tensors are on the handle's device; the weight images are rebuilt in place by a device packer
+ *   on `stream`, so "step, update, step" can be written on one stream.  The caller's tensors may be reused once
+ *   `stream` has passed the update.  A resident batch-1 kernel is stopped first (its state is saved; the next batch-1
+ *   call relaunches it), so the call may wait on the host for that.  The handle's own streams (batch-1, host-buffer
+ *   steps) wait for the update: every go2p_* call issued after this returns sees the new weights.  Kernels the caller
+ *   queued on OTHER streams are the caller's to order, as for any stream-ordered write: work that may still read the
+ *   handle's weights must complete before `stream` reaches the update, and work that must see the new weights has to
+ *   wait for `stream` (an event) -- the images are rewritten in place, not double-buffered. */
+int go2p_set_weights(go2p_handle* h, const float* const* d_weight, const float* const* d_bias, int n_layers,
+                     const float* d_obs_mean, const float* d_obs_std, void* stream);
+/* the same from host memory; synchronous (the packer has completed when it returns) */
+int go2p_set_weights_host(go2p_handle* h, const float* const* h_weight, const float* const* h_bias, int n_layers,
+                          const float* h_obs_mean, const float* h_obs_std);
+
 /* fp16 operands saturate at +-65504 where the fp32 reference does not.  Launches with GO2P_F_SAT_COUNT count the
  * (row, 32-column operand block) pairs in which an observation or a hidden activation was clipped on its way into a
  * Gemm; this reads (and optionally resets) the total once `stream` has drained.  0 means the fp16 path never left the
@@ -271,6 +299,10 @@ int go2p_fleet_step_host(go2p_fleet* f, const go2p_raw_state* h_raw, float* h_ac
 /* + per-robot resets (go2p_step_batch_host_ex): h_reset [B] uint8 in host memory, NULL = no resets, sharded like h_raw */
 int go2p_fleet_step_host_ex(go2p_fleet* f, const go2p_raw_state* h_raw, const uint8_t* h_reset, float* h_action,
                             go2p_motor_cmd* h_cmd, int64_t B, int precision);
+/* go2p_set_weights_host on every device of the fleet, one after the other.  On failure the devices before the failing
+ * one already hold the new weights; the message names the device. */
+int go2p_fleet_set_weights_host(go2p_fleet* f, const float* const* h_weight, const float* const* h_bias, int n_layers,
+                                const float* h_obs_mean, const float* h_obs_std);
 
 /* ---- small device / pinned-memory helpers so non-CUDA hosts can drive the batched path ---- */
 int go2p_dev_alloc(go2p_handle* h, size_t bytes, void** dptr);
