@@ -8,6 +8,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <array>
 #include <atomic>
 #include <chrono>
 #include <cstdio>
@@ -65,7 +66,7 @@ struct go2p_handle {
   go2p_config cfg{};
   MlpModel model;
   int device = 0, sm_count = 0, cc_major = 0, cc_minor = 0;
-  std::vector<void*> dev_owned;
+  std::vector<void*> dev_owned;                // every device buffer of the handle (owned_alloc), freed by go2p_destroy
   DevModel dm{};
   CtrlConst cc{};
   // tensor-core path
@@ -80,11 +81,11 @@ struct go2p_handle {
   bool b1_attr_set = false;                    // same for the one-shot batch-1 kernel
   size_t so_attr_smem = 0;                     // same for small_out_kernel
   WideModel wide{};
-  // fp32 path scratch (activations between the per-layer launches): set 0 serves the device-pointer API,
-  // sets 1..kPipeDepth the streams of the host-buffer pipeline (which run concurrently)
-  struct Scratch { float* buf[2] = {nullptr, nullptr}; int64_t rows = 0; };
-  Scratch scratch_sets[1 + kPipeDepth];
-  int scratch_sel = 0;
+  // activation ping-pong buffers between the per-layer launches of the fp32 path and of the wide path, one pair per
+  // stream set: set 0 serves the device-pointer API, sets 1..kPipeDepth the streams of the host-buffer pipeline (which
+  // run concurrently)
+  struct Scratch { void* buf[2] = {nullptr, nullptr}; int64_t rows = 0; };
+  Scratch fp32_scratch[1 + kPipeDepth], wide_scratch[1 + kPipeDepth];
   // batch-1
   B1State* d_state = nullptr;
   int32_t* d_step_button = nullptr;   // go2p_step_batch: dead-man buttons extracted by the assembly kernel
@@ -147,13 +148,32 @@ struct DeviceGuard {
   }
 };
 
+// Device memory of the handle.  owned_alloc gives p `bytes` of device memory unless p is already set, and records the
+// buffer in dev_owned, which go2p_destroy frees.  To retire an outgrown buffer, clear its member; do not free it:
+// cudaFree synchronises the device and would never return while the resident batch-1 kernel runs, and kernels of other
+// streams may still read the buffer.  owned_free frees a buffer at once, where no kernel can still use it.
+template <class T>
+int owned_alloc(go2p_handle* h, T*& p, size_t bytes) {
+  if (p) return GO2P_OK;
+  void* d = nullptr;
+  CU_TRY(cudaMalloc(&d, bytes));
+  h->dev_owned.push_back(d);
+  p = static_cast<T*>(d);
+  return GO2P_OK;
+}
+
+void owned_free(go2p_handle* h, void* p) {
+  if (!p) return;
+  h->dev_owned.erase(std::remove(h->dev_owned.begin(), h->dev_owned.end(), p), h->dev_owned.end());
+  cudaFree(p);
+}
+
 template <class T>
 int dev_upload(go2p_handle* h, const std::vector<T>& v, T** out) {
-  void* p = nullptr;
-  CU_TRY(cudaMalloc(&p, std::max<size_t>(v.size() * sizeof(T), 16)));
-  h->dev_owned.push_back(p);
+  T* p = nullptr;
+  if (const int rc = owned_alloc(h, p, std::max<size_t>(v.size() * sizeof(T), 16))) return rc;
   CU_TRY(cudaMemcpy(p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
-  *out = static_cast<T*>(p);
+  *out = p;
   return GO2P_OK;
 }
 
@@ -267,7 +287,8 @@ int upload_model(go2p_handle* h) {
     }
   }
   if (!h->tc_ok) {
-    int rc = wide_prepare(m, h->dev_owned, &h->wide, g_err);
+    auto alloc = [h](size_t bytes) { void* p = nullptr; return owned_alloc(h, p, bytes) ? nullptr : p; };
+    int rc = wide_prepare(m, alloc, &h->wide, g_err);
     if (rc == 0) h->wide_ok = true;
     else if (rc > 0) return rc;   // CUDA failure; rc < 0 means "shape not served"
   }
@@ -309,6 +330,18 @@ B1Args make_b1_args(const go2p_handle* h, bool weights_in_smem) {
   a.epoch = h->epoch;
   a.log = h->d_log;
   return a;
+}
+
+// one raw state as the kRawWords words of a MSG_STEP message (and of b1_selfdriven_kernel's input)
+void raw_to_words(const go2p_raw_state& r, uint32_t* w) {
+  std::memcpy(&w[0], r.quat, 16);
+  std::memcpy(&w[4], r.gyro, 12);
+  std::memcpy(&w[7], r.q, 48);
+  std::memcpy(&w[19], r.dq, 48);
+  std::memcpy(&w[31], r.axes, 16);
+  for (int i = 0; i < 4; ++i) w[35 + i] = (uint32_t)(int32_t)r.foot_force[i];
+  w[39] = (uint32_t)(r.joy_valid != 0);
+  w[40] = (uint32_t)r.button0;
 }
 
 void mail_send(go2p_handle* h, uint32_t type, const uint32_t* words, int n, uint32_t* tag_out) {
@@ -401,31 +434,26 @@ int simple_message(go2p_handle* h, uint32_t type, const uint32_t* words, int n) 
   return mail_wait(h, tag, 1);
 }
 
-int ensure_scratch(go2p_handle* h, int64_t rows) {
-  go2p_handle::Scratch& sc = h->scratch_sets[h->scratch_sel];
+// grows both buffers of sc to `rows` rows of `row_bytes`; outgrown buffers retire (owned_alloc)
+int ensure_scratch(go2p_handle* h, go2p_handle::Scratch& sc, int64_t rows, size_t row_bytes) {
   if (sc.rows >= rows) return GO2P_OK;
-  for (int i = 0; i < 2; ++i) {
-    // outgrown buffers are retired, not freed: cudaFree synchronises the device and would never return while the
-    // resident batch-1 kernel runs, and kernels of other streams may still read them; go2p_destroy frees them
-    if (sc.buf[i]) h->dev_owned.push_back(sc.buf[i]);
-    sc.buf[i] = nullptr;
-  }
+  sc.buf[0] = sc.buf[1] = nullptr;
   sc.rows = 0;
-  const size_t bytes = (size_t)rows * h->dm.max_width * sizeof(float);
-  CU_TRY(cudaMalloc((void**)&sc.buf[0], bytes));
-  CU_TRY(cudaMalloc((void**)&sc.buf[1], bytes));
+  for (void*& b : sc.buf)
+    if (const int rc = owned_alloc(h, b, (size_t)rows * row_bytes)) return rc;
   sc.rows = rows;
   return GO2P_OK;
 }
 
-int launch_fp32(go2p_handle* h, const float* d_obs, const int32_t* d_button0, float* d_act, double* d_qdes,
+int launch_fp32(go2p_handle* h, int set, const float* d_obs, const int32_t* d_button0, float* d_act, double* d_qdes,
                 MotorCmdDev* d_cmd, int64_t B, uint32_t flags, cudaStream_t st) {
   const DevModel& dm = h->dm;
   // the GEMM epilogue stores float4 where the row pitch allows it: the output base has to be 16-byte aligned
   if ((reinterpret_cast<uintptr_t>(d_act) & 15) || (d_qdes && (reinterpret_cast<uintptr_t>(d_qdes) & 15)))
     return fail(GO2P_ERR_INVALID, "fp32 path needs 16-byte aligned act/qdes device pointers");
   const int64_t chunk = std::min<int64_t>(B, kFp32ChunkRows);
-  int rc = ensure_scratch(h, chunk);
+  go2p_handle::Scratch& sc = h->fp32_scratch[set];
+  int rc = ensure_scratch(h, sc, chunk, (size_t)dm.max_width * sizeof(float));
   if (rc) return rc;
   for (int64_t r0 = 0; r0 < B; r0 += chunk) {
     const int64_t rows = std::min(chunk, B - r0);
@@ -434,7 +462,7 @@ int launch_fp32(go2p_handle* h, const float* d_obs, const int32_t* d_button0, fl
     for (int l = 0; l < dm.n_layers; ++l) {
       const DevLayer& L = dm.L[l];
       const bool last = l == dm.n_layers - 1;
-      float* out = last ? d_act + r0 * dm.out_dim : h->scratch_sets[h->scratch_sel].buf[l & 1];
+      float* out = last ? d_act + r0 * dm.out_dim : static_cast<float*>(sc.buf[l & 1]);
       const int ldc = L.N;
       // the narrow output kernel stages 128 whole rows in shared memory: it serves last hidden widths up to ~440;
       // wider ones take the generic GEMM + the elementwise A9/A11 kernel
@@ -515,7 +543,7 @@ int launch_tc(go2p_handle* h, const float* d_obs, const int32_t* d_button0, floa
   a.sat_count = nullptr;
   if (flags & GO2P_F_SAT_COUNT) {
     if (!h->d_sat) {
-      CU_TRY(cudaMalloc((void**)&h->d_sat, sizeof(unsigned long long)));
+      if (const int rc = owned_alloc(h, h->d_sat, sizeof(unsigned long long))) return rc;
       CU_TRY(cudaMemsetAsync(h->d_sat, 0, sizeof(unsigned long long), st));
     }
     a.sat_count = h->d_sat;
@@ -565,6 +593,24 @@ int fleet_run(go2p_fleet* f, int64_t B, Fn&& per_shard) {
   }
   for (auto& t : threads) t.join();
   for (int i = 0; i < n; ++i) if (rc[i]) return fail(rc[i], "device shard " + std::to_string(i) + ": " + msg[i]);
+  return GO2P_OK;
+}
+
+// The host-buffer pipeline: B rows in chunks of kHostChunkRows, round robin over the kPipeDepth pipe streams, so one
+// chunk's copies overlap another's kernels.  per_chunk(slot, r0, rows, stream) queues the chunk's copy in, its kernels
+// on stream set 1 + slot and its copy out; last_launches ends as the sum over the chunks.
+// Not re-entrant: one host thread per handle (the reference's single-threaded executor, controller.cpp:282).
+template <class Fn>
+int host_pipeline(go2p_handle* h, int64_t B, Fn&& per_chunk) {
+  const int64_t chunk = std::min<int64_t>(B, kHostChunkRows);
+  int launches = 0, slot = 0;
+  for (int64_t r0 = 0; r0 < B; r0 += chunk, slot = (slot + 1) % kPipeDepth) {
+    const int rc = per_chunk(slot, r0, std::min(chunk, B - r0), h->pipe_stream[slot]);
+    if (rc) return rc;
+    launches += h->last_launches;
+  }
+  for (int i = 0; i < kPipeDepth; ++i) CU_TRY(cudaStreamSynchronize(h->pipe_stream[i]));
+  h->last_launches = launches;
   return GO2P_OK;
 }
 }  // namespace
@@ -652,7 +698,7 @@ int go2p_create(const char* onnx_path, const go2p_config* cfg_in, go2p_handle** 
     CU_TRY(cudaHostAlloc((void**)&h->outbox, sizeof(MailWord) * kOutSlots, cudaHostAllocMapped));
     std::memset(h->inbox, 0, sizeof(MailWord) * kB1Threads);
     std::memset(h->outbox, 0, sizeof(MailWord) * kOutSlots);
-    CU_TRY(cudaMalloc((void**)&h->d_state, sizeof(B1State)));
+    if (const int e = owned_alloc(h, h->d_state, sizeof(B1State))) return e;
     B1State init{};
     init.kp = h->cfg.kp;
     init.kd = h->cfg.kd;
@@ -678,28 +724,11 @@ int go2p_destroy(go2p_handle* h) {
   if (h->b1_stream) cudaStreamSynchronize(h->b1_stream);
   if (h->graph_exec) cudaGraphExecDestroy(h->graph_exec);
   if (h->graph) cudaGraphDestroy(h->graph);
-  for (int i = 0; i < kPipeDepth; ++i) {
-    if (h->pipe_stream[i]) { cudaStreamSynchronize(h->pipe_stream[i]); cudaStreamDestroy(h->pipe_stream[i]); }
-    if (h->pipe_in[i]) cudaFree(h->pipe_in[i]);
-    if (h->pipe_out[i]) cudaFree(h->pipe_out[i]);
-  }
+  for (cudaStream_t s : h->pipe_stream)
+    if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); }
   if (h->b1_stream) cudaStreamDestroy(h->b1_stream);
   if (h->w_event) cudaEventDestroy(h->w_event);
   for (void* p : h->dev_owned) cudaFree(p);
-  wide_release(&h->wide);
-  for (auto& sc : h->scratch_sets)
-    for (int i = 0; i < 2; ++i) if (sc.buf[i]) cudaFree(sc.buf[i]);
-  if (h->d_state) cudaFree(h->d_state);
-  if (h->d_step_button) cudaFree(h->d_step_button);
-  if (h->d_log) cudaFree(h->d_log);
-  if (h->d_sat) cudaFree(h->d_sat);
-  for (void* p : {(void*)h->fleet.obs, (void*)h->fleet.vel, (void*)h->fleet.act}) if (p) cudaFree(p);
-  for (int i = 0; i < kPipeDepth; ++i) {
-    if (h->fleet.raw[i]) cudaFree(h->fleet.raw[i]);
-    if (h->fleet.cmd[i]) cudaFree(h->fleet.cmd[i]);
-    if (h->fleet.button[i]) cudaFree(h->fleet.button[i]);
-    if (h->fleet.reset[i]) cudaFree(h->fleet.reset[i]);
-  }
   if (h->inbox) cudaFreeHost(h->inbox);
   if (h->outbox) cudaFreeHost(h->outbox);
   delete h;
@@ -834,14 +863,7 @@ int go2p_step_fused(go2p_handle* h, const go2p_raw_state* raw, go2p_step_out* ou
     return fail(GO2P_ERR_UNSUPPORTED, "fused step needs a policy with 49*history inputs and 12 outputs");
   DeviceGuard g(h->device);
   uint32_t w[kRawWords];
-  std::memcpy(&w[0], raw->quat, 16);
-  std::memcpy(&w[4], raw->gyro, 12);
-  std::memcpy(&w[7], raw->q, 48);
-  std::memcpy(&w[19], raw->dq, 48);
-  std::memcpy(&w[31], raw->axes, 16);
-  for (int i = 0; i < 4; ++i) w[35 + i] = (uint32_t)(int32_t)raw->foot_force[i];
-  w[39] = (uint32_t)(raw->joy_valid != 0);
-  w[40] = (uint32_t)raw->button0;
+  raw_to_words(*raw, w);
   uint32_t tag;
   mail_send(h, MSG_STEP, w, kRawWords, &tag);
   int rc = b1_dispatch(h);
@@ -904,47 +926,46 @@ int go2p_b1_selfdriven(go2p_handle* h, const go2p_raw_state* raws, int n_raws, i
   const bool regs = b1_regs_ok(h);
   if (!fit && !regs) return fail(GO2P_ERR_UNSUPPORTED, "weights fit neither the register file nor shared memory");
   std::vector<uint32_t> words((size_t)n_raws * kRawWords);
-  for (int r = 0; r < n_raws; ++r) {
-    uint32_t* w = &words[(size_t)r * kRawWords];
-    std::memcpy(&w[0], raws[r].quat, 16); std::memcpy(&w[4], raws[r].gyro, 12);
-    std::memcpy(&w[7], raws[r].q, 48); std::memcpy(&w[19], raws[r].dq, 48); std::memcpy(&w[31], raws[r].axes, 16);
-    for (int i = 0; i < 4; ++i) w[35 + i] = (uint32_t)(int32_t)raws[r].foot_force[i];
-    w[39] = (uint32_t)(raws[r].joy_valid != 0);
-    w[40] = (uint32_t)raws[r].button0;
-  }
+  for (int r = 0; r < n_raws; ++r) raw_to_words(raws[r], &words[(size_t)r * kRawWords]);
   uint32_t* d_raws = nullptr;
   float* d_out = nullptr;
   B1State* d_st = nullptr;
-  CU_TRY(cudaMalloc((void**)&d_raws, words.size() * 4));
-  CU_TRY(cudaMalloc((void**)&d_out, 64));
-  CU_TRY(cudaMalloc((void**)&d_st, sizeof(B1State)));
-  B1State init{};
-  init.kp = h->cfg.kp; init.kd = h->cfg.kd;
-  CU_TRY(cudaMemcpy(d_st, &init, sizeof(init), cudaMemcpyHostToDevice));
-  CU_TRY(cudaMemcpy(d_raws, words.data(), words.size() * 4, cudaMemcpyHostToDevice));
-  if (regs) CU_TRY(cudaFuncSetAttribute(b1_selfdriven_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  else CU_TRY(cudaFuncSetAttribute(b1_selfdriven_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  B1Args a = make_b1_args(h, true);
-  a.gstate = d_st;
-  cudaEvent_t e0, e1;
-  CU_TRY(cudaEventCreate(&e0));
-  CU_TRY(cudaEventCreate(&e1));
-  CU_TRY(cudaEventRecord(e0, h->pipe_stream[0]));
-  if (regs) b1_selfdriven_kernel<true><<<1, kB1Threads, smem, h->pipe_stream[0]>>>(a, d_raws, n_raws, steps, d_out);
-  else b1_selfdriven_kernel<false><<<1, kB1Threads, smem, h->pipe_stream[0]>>>(a, d_raws, n_raws, steps, d_out);
-  CU_TRY(cudaGetLastError());
-  CU_TRY(cudaEventRecord(e1, h->pipe_stream[0]));
-  CU_TRY(cudaEventSynchronize(e1));
-  float ms = 0.f;
-  CU_TRY(cudaEventElapsedTime(&ms, e0, e1));
-  if (elapsed_ms) *elapsed_ms = ms;
-  if (last_action) CU_TRY(cudaMemcpyAsync(last_action, d_out, 48, cudaMemcpyDeviceToHost, h->pipe_stream[0]));
-  CU_TRY(cudaStreamSynchronize(h->pipe_stream[0]));
-  cudaEventDestroy(e0); cudaEventDestroy(e1);
-  if (!h->resident) { cudaFree(d_raws); cudaFree(d_out); cudaFree(d_st); }
-  else { h->dev_owned.push_back(d_raws); h->dev_owned.push_back(d_out); h->dev_owned.push_back(d_st); }   // cudaFree would block on the resident kernel: retired, freed by go2p_destroy
-  h->last_launches = 1;
-  return GO2P_OK;
+  cudaEvent_t e0 = nullptr, e1 = nullptr;
+  auto run = [&]() -> int {
+    int rc;
+    if ((rc = owned_alloc(h, d_raws, words.size() * 4)) || (rc = owned_alloc(h, d_out, 64)) ||
+        (rc = owned_alloc(h, d_st, sizeof(B1State))))
+      return rc;
+    B1State init{};
+    init.kp = h->cfg.kp; init.kd = h->cfg.kd;
+    CU_TRY(cudaMemcpy(d_st, &init, sizeof(init), cudaMemcpyHostToDevice));
+    CU_TRY(cudaMemcpy(d_raws, words.data(), words.size() * 4, cudaMemcpyHostToDevice));
+    if (regs) CU_TRY(cudaFuncSetAttribute(b1_selfdriven_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    else CU_TRY(cudaFuncSetAttribute(b1_selfdriven_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    B1Args a = make_b1_args(h, true);
+    a.gstate = d_st;
+    CU_TRY(cudaEventCreate(&e0));
+    CU_TRY(cudaEventCreate(&e1));
+    CU_TRY(cudaEventRecord(e0, h->pipe_stream[0]));
+    if (regs) b1_selfdriven_kernel<true><<<1, kB1Threads, smem, h->pipe_stream[0]>>>(a, d_raws, n_raws, steps, d_out);
+    else b1_selfdriven_kernel<false><<<1, kB1Threads, smem, h->pipe_stream[0]>>>(a, d_raws, n_raws, steps, d_out);
+    CU_TRY(cudaGetLastError());
+    CU_TRY(cudaEventRecord(e1, h->pipe_stream[0]));
+    CU_TRY(cudaEventSynchronize(e1));
+    float ms = 0.f;
+    CU_TRY(cudaEventElapsedTime(&ms, e0, e1));
+    if (elapsed_ms) *elapsed_ms = ms;
+    if (last_action) CU_TRY(cudaMemcpyAsync(last_action, d_out, 48, cudaMemcpyDeviceToHost, h->pipe_stream[0]));
+    CU_TRY(cudaStreamSynchronize(h->pipe_stream[0]));
+    return GO2P_OK;
+  };
+  const int rc = run();
+  if (e0) cudaEventDestroy(e0);
+  if (e1) cudaEventDestroy(e1);
+  // while the resident kernel runs, cudaFree would block on it: the buffers then stay until go2p_destroy
+  if (!h->resident) for (void* p : {(void*)d_raws, (void*)d_out, (void*)d_st}) owned_free(h, p);
+  if (rc == GO2P_OK) h->last_launches = 1;
+  return rc;
 }
 
 int go2p_reset_history(go2p_handle* h) {
@@ -971,8 +992,10 @@ int go2p_b1_stats_get(go2p_handle* h, go2p_b1_stats* out, int reset) {
 }
 
 // ------------------------------------------------------------------------------------- batched
-int go2p_infer_batch_cmd(go2p_handle* h, const float* d_obs, const int32_t* d_button0, float* d_act, double* d_qdes,
-                         go2p_motor_cmd* d_cmd, int64_t B, int precision, uint32_t flags, void* stream) {
+namespace {
+// go2p_infer_batch_cmd with the activation scratch of stream set `set`
+int infer_batch_on(go2p_handle* h, int set, const float* d_obs, const int32_t* d_button0, float* d_act, double* d_qdes,
+                   go2p_motor_cmd* d_cmd, int64_t B, int precision, uint32_t flags, cudaStream_t st) {
   if (!h) return fail(GO2P_ERR_INVALID, "go2p_infer_batch: null handle");
   if (B < 0) return fail(GO2P_ERR_INVALID, "negative batch");
   if (B == 0) { h->last_launches = 0; return GO2P_OK; }   // empty batch: nothing is read, nothing is launched
@@ -985,21 +1008,30 @@ int go2p_infer_batch_cmd(go2p_handle* h, const float* d_obs, const int32_t* d_bu
     return fail(GO2P_ERR_INVALID, "d_cmd must be 16-byte aligned");
   h->last_launches = 0;
   DeviceGuard g(h->device);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
   MotorCmdDev* cmd = reinterpret_cast<MotorCmdDev*>(d_cmd);
   switch (precision) {
-    case GO2P_PREC_FP32: return launch_fp32(h, d_obs, d_button0, d_act, d_qdes, cmd, B, flags, st);
+    case GO2P_PREC_FP32: return launch_fp32(h, set, d_obs, d_button0, d_act, d_qdes, cmd, B, flags, st);
     case GO2P_PREC_BF16:
     case GO2P_PREC_FP16:
       if (h->tc_ok) return launch_tc(h, d_obs, d_button0, d_act, d_qdes, cmd, B, precision == GO2P_PREC_FP16, flags, st);
       if (h->wide_ok) {
-        int rc = wide_launch(h->wide, d_obs, d_button0, d_act, d_qdes, cmd, B, precision == GO2P_PREC_FP16, flags, h->cc,
-                             h->sm_count, st, &h->last_launches, g_err, h->scratch_sel);
+        go2p_handle::Scratch& sc = h->wide_scratch[set];
+        if (ensure_scratch(h, sc, wide_act_rows(B), (size_t)h->wide.max_kp * sizeof(uint16_t)))
+          return fail(GO2P_ERR_CUDA, "wide_launch: cudaMalloc of the activation buffers failed");
+        uint16_t* const act[2] = {static_cast<uint16_t*>(sc.buf[0]), static_cast<uint16_t*>(sc.buf[1])};
+        int rc = wide_launch(h->wide, act, d_obs, d_button0, d_act, d_qdes, cmd, B, precision == GO2P_PREC_FP16, flags, h->cc,
+                             h->sm_count, st, &h->last_launches, g_err);
         return rc ? fail(rc, g_err.c_str()) : GO2P_OK;
       }
       return fail(GO2P_ERR_UNSUPPORTED, "tensor-core kernels do not serve this layer shape; use GO2P_PREC_FP32");
     default: return fail(GO2P_ERR_INVALID, "unknown precision");
   }
+}
+}  // namespace
+
+int go2p_infer_batch_cmd(go2p_handle* h, const float* d_obs, const int32_t* d_button0, float* d_act, double* d_qdes,
+                         go2p_motor_cmd* d_cmd, int64_t B, int precision, uint32_t flags, void* stream) {
+  return infer_batch_on(h, 0, d_obs, d_button0, d_act, d_qdes, d_cmd, B, precision, flags, static_cast<cudaStream_t>(stream));
 }
 
 int go2p_infer_batch_ex(go2p_handle* h, const float* d_obs, const int32_t* d_button0, float* d_act, double* d_qdes,
@@ -1042,31 +1074,19 @@ int go2p_infer_batch_host(go2p_handle* h, const float* h_obs, float* h_act, int6
   if (B <= 0) return B == 0 ? GO2P_OK : fail(GO2P_ERR_INVALID, "negative batch");
   DeviceGuard g(h->device);
   const int in = h->dm.in_dim, out = h->dm.out_dim;
-  const int64_t chunk = std::min<int64_t>(B, kHostChunkRows);
   for (int i = 0; i < kPipeDepth; ++i) {
-    if (!h->pipe_in[i]) {
-      CU_TRY(cudaMalloc((void**)&h->pipe_in[i], (size_t)kHostChunkRows * in * sizeof(float)));
-      CU_TRY(cudaMalloc((void**)&h->pipe_out[i], (size_t)kHostChunkRows * out * sizeof(float)));
-    }
+    int rc;
+    if ((rc = owned_alloc(h, h->pipe_in[i], (size_t)kHostChunkRows * in * sizeof(float))) ||
+        (rc = owned_alloc(h, h->pipe_out[i], (size_t)kHostChunkRows * out * sizeof(float))))
+      return rc;
   }
-  int launches = 0;
-  int slot = 0;
-  // Not re-entrant: one host thread per handle (the reference's single-threaded executor, controller.cpp:282);
-  // scratch_sel routes every stream of the pipeline to its own activation scratch.
-  for (int64_t r0 = 0; r0 < B; r0 += chunk, slot = (slot + 1) % kPipeDepth) {
-    const int64_t rows = std::min(chunk, B - r0);
-    cudaStream_t st = h->pipe_stream[slot];
+  return host_pipeline(h, B, [&](int slot, int64_t r0, int64_t rows, cudaStream_t st) -> int {
     CU_TRY(cudaMemcpyAsync(h->pipe_in[slot], h_obs + r0 * in, (size_t)rows * in * sizeof(float), cudaMemcpyHostToDevice, st));
-    h->scratch_sel = 1 + slot;
-    int rc = go2p_infer_batch_cmd(h, h->pipe_in[slot], nullptr, h->pipe_out[slot], nullptr, nullptr, rows, precision, 0u, st);
-    h->scratch_sel = 0;
+    const int rc = infer_batch_on(h, 1 + slot, h->pipe_in[slot], nullptr, h->pipe_out[slot], nullptr, nullptr, rows, precision, 0u, st);
     if (rc) return rc;
-    launches += h->last_launches;
     CU_TRY(cudaMemcpyAsync(h_act + r0 * out, h->pipe_out[slot], (size_t)rows * out * sizeof(float), cudaMemcpyDeviceToHost, st));
-  }
-  for (int i = 0; i < kPipeDepth; ++i) CU_TRY(cudaStreamSynchronize(h->pipe_stream[i]));
-  h->last_launches = launches;
-  return GO2P_OK;
+    return GO2P_OK;
+  });
 }
 
 int go2p_assemble_batch(go2p_handle* h, const go2p_raw_state* d_raw, const float* d_prev_action, float* d_vel_cmd,
@@ -1085,7 +1105,8 @@ namespace {
 // publish() for B robots on device buffers; button_scratch [B] receives the dead-man buttons for the epilogue.
 // d_reset [B] (may be null): robots to start from the initial state, applied by whichever kernel assembles the
 // observations (the fused kernel's conversion job or assemble_batch_kernel); the path choice does not depend on it.
-int step_batch_on(go2p_handle* h, const go2p_raw_state* d_raw, const uint8_t* d_reset, float* d_vel_cmd, float* d_obs,
+// `set`: the stream set whose activation scratch the policy uses.
+int step_batch_on(go2p_handle* h, int set, const go2p_raw_state* d_raw, const uint8_t* d_reset, float* d_vel_cmd, float* d_obs,
                   float* d_action, double* d_qdes, go2p_motor_cmd* d_cmd, int32_t* button_scratch, int64_t B, int precision,
                   cudaStream_t st) {
   const uint32_t all_flags = GO2P_F_CLAMP_MASK | (d_qdes ? GO2P_F_QDES : 0u) | (d_cmd ? GO2P_F_MOTOR_CMD : 0u);
@@ -1107,7 +1128,7 @@ int step_batch_on(go2p_handle* h, const go2p_raw_state* d_raw, const uint8_t* d_
   CU_TRY(cudaGetLastError());
   // A7 + A9 + A11
   const uint32_t flags = GO2P_F_CLAMP_MASK | (d_qdes ? GO2P_F_QDES : 0u) | (d_cmd ? GO2P_F_MOTOR_CMD : 0u);
-  const int rc = go2p_infer_batch_cmd(h, d_obs, button_scratch, d_action, d_qdes, d_cmd, B, precision, flags, st);
+  const int rc = infer_batch_on(h, set, d_obs, button_scratch, d_action, d_qdes, d_cmd, B, precision, flags, st);
   if (rc == GO2P_OK) h->last_launches += 1;
   return rc;
 }
@@ -1122,11 +1143,12 @@ int go2p_step_batch_ex(go2p_handle* h, const go2p_raw_state* d_raw, const uint8_
     return fail(GO2P_ERR_INVALID, "go2p_step_batch: the policy is not a 49*H -> 12 controller policy");
   DeviceGuard g(h->device);
   if (h->step_button_rows < B) {
-    if (h->d_step_button) { h->dev_owned.push_back(h->d_step_button); h->d_step_button = nullptr; }   // retired, see ensure_scratch
-    CU_TRY(cudaMalloc((void**)&h->d_step_button, (size_t)B * sizeof(int32_t)));
+    h->d_step_button = nullptr;   // retire (owned_alloc)
+    h->step_button_rows = 0;
+    if (const int rc = owned_alloc(h, h->d_step_button, (size_t)B * sizeof(int32_t))) return rc;
     h->step_button_rows = B;
   }
-  return step_batch_on(h, d_raw, d_reset, d_vel_cmd, d_obs, d_action, d_qdes, d_cmd, h->d_step_button, B, precision,
+  return step_batch_on(h, 0, d_raw, d_reset, d_vel_cmd, d_obs, d_action, d_qdes, d_cmd, h->d_step_button, B, precision,
                        static_cast<cudaStream_t>(stream));
 }
 
@@ -1154,13 +1176,15 @@ int go2p_step_batch_host_ex(go2p_handle* h, const go2p_raw_state* h_raw, const u
   DeviceGuard g(h->device);
   go2p_handle::Fleet& f = h->fleet;
   const int n_obs = h->dm.in_dim;
+  int rc;
   if (f.robots != B) {
-    // (re)create the fleet state: histories 0, joystick command 0, previous action 0 (controller.hpp:132-162)
-    for (void* p : {(void*)f.obs, (void*)f.vel, (void*)f.act}) if (p) h->dev_owned.push_back(p);
+    // (re)create the fleet state: histories 0, joystick command 0, previous action 0 (controller.hpp:132-162); the
+    // old buffers retire (owned_alloc)
+    f.robots = 0;
     f.obs = f.vel = f.act = nullptr;
-    CU_TRY(cudaMalloc((void**)&f.obs, (size_t)B * n_obs * sizeof(float)));
-    CU_TRY(cudaMalloc((void**)&f.vel, (size_t)B * 3 * sizeof(float)));
-    CU_TRY(cudaMalloc((void**)&f.act, (size_t)B * kDof * sizeof(float)));
+    if ((rc = owned_alloc(h, f.obs, (size_t)B * n_obs * sizeof(float))) || (rc = owned_alloc(h, f.vel, (size_t)B * 3 * sizeof(float))) ||
+        (rc = owned_alloc(h, f.act, (size_t)B * kDof * sizeof(float))))
+      return rc;
     CU_TRY(cudaMemsetAsync(f.obs, 0, (size_t)B * n_obs * sizeof(float), h->pipe_stream[0]));
     CU_TRY(cudaMemsetAsync(f.vel, 0, (size_t)B * 3 * sizeof(float), h->pipe_stream[0]));
     CU_TRY(cudaMemsetAsync(f.act, 0, (size_t)B * kDof * sizeof(float), h->pipe_stream[0]));
@@ -1168,33 +1192,23 @@ int go2p_step_batch_host_ex(go2p_handle* h, const go2p_raw_state* h_raw, const u
     f.robots = B;
   }
   for (int i = 0; i < kPipeDepth; ++i) {
-    if (!f.raw[i]) {
-      CU_TRY(cudaMalloc((void**)&f.raw[i], (size_t)kHostChunkRows * sizeof(go2p_raw_state)));
-      CU_TRY(cudaMalloc((void**)&f.cmd[i], (size_t)kHostChunkRows * sizeof(MotorCmdDev)));
-      CU_TRY(cudaMalloc((void**)&f.button[i], (size_t)kHostChunkRows * sizeof(int32_t)));
-    }
-    if (h_reset && !f.reset[i]) CU_TRY(cudaMalloc((void**)&f.reset[i], (size_t)kHostChunkRows));
+    if ((rc = owned_alloc(h, f.raw[i], (size_t)kHostChunkRows * sizeof(go2p_raw_state))) ||
+        (rc = owned_alloc(h, f.cmd[i], (size_t)kHostChunkRows * sizeof(MotorCmdDev))) ||
+        (rc = owned_alloc(h, f.button[i], (size_t)kHostChunkRows * sizeof(int32_t))) ||
+        (h_reset && (rc = owned_alloc(h, f.reset[i], (size_t)kHostChunkRows))))
+      return rc;
   }
-  const int64_t chunk = std::min<int64_t>(B, kHostChunkRows);
-  int launches = 0, slot = 0;
-  for (int64_t r0 = 0; r0 < B; r0 += chunk, slot = (slot + 1) % kPipeDepth) {
-    const int64_t rows = std::min(chunk, B - r0);
-    cudaStream_t st = h->pipe_stream[slot];
+  return host_pipeline(h, B, [&](int slot, int64_t r0, int64_t rows, cudaStream_t st) -> int {
     CU_TRY(cudaMemcpyAsync(f.raw[slot], h_raw + r0, (size_t)rows * sizeof(go2p_raw_state), cudaMemcpyHostToDevice, st));
     if (h_reset) CU_TRY(cudaMemcpyAsync(f.reset[slot], h_reset + r0, (size_t)rows, cudaMemcpyHostToDevice, st));
-    h->scratch_sel = 1 + slot;
-    int rc = step_batch_on(h, f.raw[slot], h_reset ? f.reset[slot] : nullptr, f.vel + r0 * 3, f.obs + r0 * n_obs,
-                           f.act + r0 * kDof, nullptr, h_cmd ? reinterpret_cast<go2p_motor_cmd*>(f.cmd[slot]) : nullptr,
-                           f.button[slot], rows, precision, st);
-    h->scratch_sel = 0;
+    const int rc = step_batch_on(h, 1 + slot, f.raw[slot], h_reset ? f.reset[slot] : nullptr, f.vel + r0 * 3, f.obs + r0 * n_obs,
+                                 f.act + r0 * kDof, nullptr, h_cmd ? reinterpret_cast<go2p_motor_cmd*>(f.cmd[slot]) : nullptr,
+                                 f.button[slot], rows, precision, st);
     if (rc) return rc;
-    launches += h->last_launches;
     CU_TRY(cudaMemcpyAsync(h_action + r0 * kDof, f.act + r0 * kDof, (size_t)rows * kDof * sizeof(float), cudaMemcpyDeviceToHost, st));
     if (h_cmd) CU_TRY(cudaMemcpyAsync(h_cmd + r0, f.cmd[slot], (size_t)rows * sizeof(MotorCmdDev), cudaMemcpyDeviceToHost, st));
-  }
-  for (int i = 0; i < kPipeDepth; ++i) CU_TRY(cudaStreamSynchronize(h->pipe_stream[i]));
-  h->last_launches = launches;
-  return GO2P_OK;
+    return GO2P_OK;
+  });
 }
 
 int go2p_step_batch_host(go2p_handle* h, const go2p_raw_state* h_raw, float* h_action, go2p_motor_cmd* h_cmd, int64_t B,
@@ -1224,15 +1238,20 @@ int check_weight_args(const char* fn, const go2p_handle* h, const float* const* 
   return GO2P_OK;
 }
 
+// the handle's own streams: the batch-1 stream and the host pipeline's
+std::array<cudaStream_t, 1 + kPipeDepth> own_streams(const go2p_handle* h) {
+  std::array<cudaStream_t, 1 + kPipeDepth> own = {h->b1_stream};
+  for (int i = 0; i < kPipeDepth; ++i) own[1 + i] = h->pipe_stream[i];
+  return own;
+}
+
 // Before the packer touches the images: the resident batch-1 kernel (which holds the weights in registers or shared
 // memory) is stopped -- it saves its state to d_state and is relaunched lazily by the next batch-1 call -- and `st`
 // waits for whatever the handle's own streams have queued, the previous update's packer included.
 int begin_update(go2p_handle* h, cudaStream_t st) {
   if (h->resident) { const int rc = go2p_persistent_stop(h); if (rc) return rc; }
   if (!h->w_event) CU_TRY(cudaEventCreateWithFlags(&h->w_event, cudaEventDisableTiming));
-  cudaStream_t own[1 + kPipeDepth] = {h->b1_stream};
-  for (int i = 0; i < kPipeDepth; ++i) own[1 + i] = h->pipe_stream[i];
-  for (cudaStream_t s : own) {
+  for (cudaStream_t s : own_streams(h)) {
     if (s == st) continue;
     CU_TRY(cudaEventRecord(h->w_event, s));
     CU_TRY(cudaStreamWaitEvent(st, h->w_event, 0));
@@ -1268,10 +1287,7 @@ int pack_and_publish(go2p_handle* h, const float* const* w, const float* const* 
   }
   if (mean) {
     const int K = dm.L[0].K, N = dm.L[0].N;
-    if (!h->w_fold) {
-      CU_TRY(cudaMalloc((void**)&h->w_fold, ((size_t)N * K + N) * sizeof(float)));
-      h->dev_owned.push_back(h->w_fold);
-    }
+    if (const int rc = owned_alloc(h, h->w_fold, ((size_t)N * K + N) * sizeof(float))) return rc;
     fold_normaliser_kernel<<<(N + 127) / 128, 128, 0, st>>>(w[0], b ? b[0] : nullptr, mean, stdv, K, N, h->w_fold,
                                                            h->w_fold + (size_t)N * K);
     CU_TRY(cudaGetLastError());
@@ -1282,9 +1298,7 @@ int pack_and_publish(go2p_handle* h, const float* const* w, const float* const* 
   pack_weights_kernel<<<dim3((unsigned)blocks, (unsigned)dm.n_layers), 256, 0, st>>>(pa);
   CU_TRY(cudaGetLastError());
   CU_TRY(cudaEventRecord(h->w_event, st));
-  cudaStream_t own[1 + kPipeDepth] = {h->b1_stream};
-  for (int i = 0; i < kPipeDepth; ++i) own[1 + i] = h->pipe_stream[i];
-  for (cudaStream_t s : own)
+  for (cudaStream_t s : own_streams(h))
     if (s != st) CU_TRY(cudaStreamWaitEvent(s, h->w_event, 0));
   ++h->w_gen;
   h->w_stream = st;
@@ -1310,10 +1324,7 @@ int go2p_set_weights_host(go2p_handle* h, const float* const* h_weight, const fl
   const DevModel& dm = h->dm;
   size_t floats = 2 * (size_t)dm.in_dim;
   for (int l = 0; l < dm.n_layers; ++l) floats += (size_t)dm.L[l].N * dm.L[l].K + dm.L[l].N;
-  if (!h->w_stage) {       // the topology is fixed, so is the size
-    CU_TRY(cudaMalloc((void**)&h->w_stage, floats * sizeof(float)));
-    h->dev_owned.push_back(h->w_stage);
-  }
+  if ((rc = owned_alloc(h, h->w_stage, floats * sizeof(float)))) return rc;   // the topology is fixed, so is the size
   cudaStream_t st = h->pipe_stream[0];
   if ((rc = begin_update(h, st))) return rc;
   const float* dw[kMaxLayers] = {};
@@ -1344,11 +1355,12 @@ int go2p_log_enable(go2p_handle* h, int capacity) {
   DeviceGuard g(h->device);
   const bool was_resident = h->resident;
   if (was_resident) { int rc = go2p_persistent_stop(h); if (rc) return rc; }   // the ring pointer is a launch argument
-  if (h->d_log) { cudaFree(h->d_log); h->d_log = nullptr; }
+  owned_free(h, h->d_log);
+  h->d_log = nullptr;
   h->log_capacity = 0; h->log_tail = 0;
   if (capacity > 0) {
     const size_t bytes = sizeof(LogRing) + (size_t)capacity * kLogRecFloats * sizeof(float);
-    CU_TRY(cudaMalloc((void**)&h->d_log, bytes));
+    if (const int rc = owned_alloc(h, h->d_log, bytes)) return rc;
     CU_TRY(cudaMemset(h->d_log, 0, bytes));
     LogRing hdr{};
     hdr.head = 0; hdr.capacity = (uint32_t)capacity; hdr.n_obs = (uint32_t)h->dm.in_dim;

@@ -67,12 +67,6 @@ struct WideModel {
   int in_dim = 0, out_dim = 0;
   WideLayerDev L[kMaxLayers];
   int max_kp = 0;          // widest blocked activation (in K columns)
-  // activation ping-pong buffers (allocated lazily by wide_launch for a chunk of rows)
-  // one pair per stream set (capi.cu: scratch_sel; the host-buffer pipeline runs several streams concurrently)
-  static constexpr int kSets = 4;
-  mutable uint16_t* act[kSets][2] = {};
-  mutable long long act_rows[kSets] = {};
-  mutable std::vector<void*> retired;     // outgrown buffers: freed with the model (cudaFree would synchronise the device)
 };
 
 struct WideGemmArgs {
@@ -391,16 +385,17 @@ inline void wd_pack_weights(const MlpLayer& L, int NT, int Np, int Kp, bool fp16
     }
 }
 
-// returns 0 = ok, > 0 = go2p_status (CUDA failure), < 0 = this shape is not served by the wide path
-inline int wide_prepare(const MlpModel& m, std::vector<void*>& dev_owned, WideModel* wm, std::string& err) {
+// returns 0 = ok, > 0 = go2p_status (CUDA failure), < 0 = this shape is not served by the wide path.
+// alloc(bytes) returns device memory that the caller owns, or null.
+template <class Alloc>
+inline int wide_prepare(const MlpModel& m, Alloc&& alloc, WideModel* wm, std::string& err) {
   const int nl = (int)m.layers.size();
   if (nl < 2 || nl > kMaxLayers || m.layers.back().out > 16) return -1;
   for (int l = 0; l + 1 < nl; ++l) if (m.layers[l].out % 64 != 0) return -1;
   wm->n_layers = nl; wm->in_dim = m.layers.front().in; wm->out_dim = m.layers.back().out; wm->max_kp = 0;
   auto upload = [&](const void* src, size_t bytes, void** out) -> bool {
-    void* p = nullptr;
-    if (cudaMalloc(&p, bytes) != cudaSuccess) { err = "wide_prepare: cudaMalloc failed"; return false; }
-    dev_owned.push_back(p);
+    void* p = alloc(bytes);
+    if (!p) { err = "wide_prepare: cudaMalloc failed"; return false; }
     if (cudaMemcpy(p, src, bytes, cudaMemcpyHostToDevice) != cudaSuccess) { err = "wide_prepare: cudaMemcpy failed"; return false; }
     *out = p; return true;
   };
@@ -484,15 +479,6 @@ inline cudaError_t wd_launch_gemm(const WideGemmArgs& a, int sm_count, cudaStrea
   return cudaLaunchKernelEx(&cfg, kernel, a);
 }
 
-inline void wide_release(WideModel* wm) {
-  for (int s = 0; s < WideModel::kSets; ++s) {
-    for (int i = 0; i < 2; ++i) { if (wm->act[s][i]) cudaFree(wm->act[s][i]); wm->act[s][i] = nullptr; }
-    wm->act_rows[s] = 0;
-  }
-  for (void* p : wm->retired) cudaFree(p);
-  wm->retired.clear();
-}
-
 // rows per pass: a multiple of 148 row tiles, so every layer's job count is a whole number of waves over the 148 SMs.
 // Round 1 used ONE wave of row tiles (18,944 rows: the widest activation, 39 MB, stays in the 126 MB L2); measured in
 // round 2 (scripts/gpu_wide_variants.sh, 606,208 rows, fp16 / bf16): 1 wave 1.86 / 1.85 ms, 2 waves 1.62 / 1.66 ms,
@@ -504,20 +490,16 @@ inline void wide_release(WideModel* wm) {
 #endif
 constexpr long long kWdChunkRows = 148 * kWdTileM * GO2P_WD_PASS_WAVES;
 
-inline int wide_launch(const WideModel& wm, const float* d_obs, const int32_t* d_button0, float* d_act, double* d_qdes, MotorCmdDev* d_cmd, long long B,
-                       bool fp16, uint32_t flags, const CtrlConst& cc, int sm_count, cudaStream_t st, int* launches, std::string& err, int set = 0) {
-  if (set < 0 || set >= WideModel::kSets) { err = "wide_launch: bad stream set"; return 2; }
-  uint16_t** act = wm.act[set];
+// rows of one pass of wide_launch over B rows, in whole row tiles
+inline long long wide_act_rows(long long B) {
+  return (std::min<long long>(B, kWdChunkRows) + kWdTileM - 1) / kWdTileM * kWdTileM;
+}
+
+// act: the two blocked activation buffers (ping-pong), each of wide_act_rows(B) rows x wm.max_kp 16-bit columns
+inline int wide_launch(const WideModel& wm, uint16_t* const act[2], const float* d_obs, const int32_t* d_button0, float* d_act, double* d_qdes,
+                       MotorCmdDev* d_cmd, long long B, bool fp16, uint32_t flags, const CtrlConst& cc, int sm_count, cudaStream_t st,
+                       int* launches, std::string& err) {
   const long long chunk = std::min<long long>(B, kWdChunkRows);
-  const long long chunk_tiles = (chunk + kWdTileM - 1) / kWdTileM;
-  if (wm.act_rows[set] < chunk_tiles * kWdTileM) {
-    for (int i = 0; i < 2; ++i) { if (act[i]) wm.retired.push_back(act[i]); act[i] = nullptr; }
-    const size_t bytes = (size_t)chunk_tiles * kWdTileM * wm.max_kp * 2;
-    if (cudaMalloc((void**)&act[0], bytes) != cudaSuccess || cudaMalloc((void**)&act[1], bytes) != cudaSuccess) {
-      err = "wide_launch: cudaMalloc of the activation buffers failed"; return 4;
-    }
-    wm.act_rows[set] = chunk_tiles * kWdTileM;
-  }
   for (long long r0 = 0; r0 < B; r0 += chunk) {
     const long long rows = std::min(chunk, B - r0);
     const int m_tiles = (int)((rows + kWdTileM - 1) / kWdTileM);
