@@ -136,6 +136,51 @@ def weight_arrays(dims, weights, biases=None, obs_mean=None, obs_std=None, devic
     return kinds.pop()
 
 
+RAW_FIELDS = (("quat", 4), ("gyro", 3), ("q", 12), ("dq", 12), ("axes", 4), ("foot_force", 4), ("joy_valid", None),
+              ("button0", None))
+_FLAG_DTYPES = ("torch.bool", "torch.uint8")
+
+
+def step_field_tensors(in_dim: int, device: int, fields: dict, vel_cmd, obs, action, qdes=None, cmd=None, reset=None) -> int:
+    """Validates the arguments of PolicyBatch.step_fields before any native call.  fields: the eight raw-state tensors by
+    name (RAW_FIELDS): float32 [B,w], foot_force int16 [B,4], joy_valid / button0 bool or uint8 [B].  vel_cmd float32
+    [B,3], obs float32 [B,in_dim], action float32 [B,12], qdes float64 [B,12] or None, cmd uint8 [B,112] or None (not
+    both None), reset bool / uint8 [B] or None.  Every tensor is a contiguous CUDA tensor on device ``device`` (duck-typed:
+    this package does not import torch).  Returns B; raises TypeError / ValueError."""
+    if qdes is None and cmd is None:
+        raise ValueError("qdes and cmd are both None: the step needs at least one output")
+    quat = fields["quat"]
+    if not _is_device_tensor(quat):
+        raise TypeError(f"quat must be a CUDA tensor, got {type(quat).__name__}")
+    if len(quat.shape) != 2:
+        raise ValueError(f"quat must have shape (B, 4), got {tuple(quat.shape)}")
+    B = int(quat.shape[0])
+    named = [(name, fields[name], (B, w) if w else (B,), "torch.int16" if name == "foot_force" else
+              _FLAG_DTYPES if w is None else "torch.float32") for name, w in RAW_FIELDS]
+    named += [("vel_cmd", vel_cmd, (B, 3), "torch.float32"), ("obs", obs, (B, in_dim), "torch.float32"),
+              ("action", action, (B, 12), "torch.float32")]
+    if qdes is not None:
+        named.append(("qdes", qdes, (B, 12), "torch.float64"))
+    if cmd is not None:
+        named.append(("cmd", cmd, (B, C.sizeof(capi.MotorCmd)), "torch.uint8"))
+    if reset is not None:
+        named.append(("reset", reset, (B,), _FLAG_DTYPES))
+    for name, a, shape, dtypes in named:
+        if not _is_device_tensor(a):
+            raise TypeError(f"{name} must be a CUDA tensor, got {type(a).__name__}")
+        if str(a.dtype) not in ((dtypes,) if isinstance(dtypes, str) else dtypes):
+            raise TypeError(f"{name} must be {' or '.join((dtypes,) if isinstance(dtypes, str) else dtypes)}, got {a.dtype}")
+        if getattr(a.device, "type", None) != "cuda":
+            raise TypeError(f"{name} is a tensor on {a.device}: pass a CUDA tensor")
+        if a.device.index != device:
+            raise ValueError(f"{name} is on cuda:{a.device.index}, the handle on cuda:{device}")
+        if tuple(a.shape) != shape:
+            raise ValueError(f"{name} must have shape {shape}, got {tuple(a.shape)}")
+        if not a.is_contiguous():
+            raise ValueError(f"{name} must be contiguous")
+    return B
+
+
 def _ptr(a):
     return None if a is None else (a.ctypes.data if isinstance(a, np.ndarray) else a.data_ptr())
 
@@ -332,6 +377,24 @@ class PolicyBatch:
         else:
             capi.check(self._hd.lib.go2p_step_batch_ex(self._hd.h, d_raw, d_reset, d_vel_cmd, d_obs, d_action, d_qdes, d_cmd,
                                                        B, precision, stream or None))
+
+    def step_fields(self, quat, gyro, q, dq, axes, foot_force, joy_valid, button0, vel_cmd, obs, action, qdes=None,
+                    cmd=None, precision: int = capi.PREC_FP32, stream: int = 0, reset=None) -> None:
+        """step_device_cmd with the raw states as one CUDA tensor per field, the way a GPU simulator keeps them
+        (go2p_step_batch_fields): quat [B,4], gyro [B,3], q [B,12], dq [B,12], axes [B,4] float32, foot_force [B,4]
+        int16 (Unitree order), joy_valid / button0 [B] bool or uint8.  vel_cmd [B,3], obs [B,in_dim] and action [B,12]
+        (previous published action on entry) are the robots' state, updated in place; qdes float64 [B,12] and / or cmd
+        uint8 [B,112] receive the outputs; reset: bool / uint8 [B] or None.  Every tensor contiguous and on the handle's
+        device; a slice of a wider tensor must be made contiguous first.  B = 0 does nothing."""
+        fields = dict(quat=quat, gyro=gyro, q=q, dq=dq, axes=axes, foot_force=foot_force, joy_valid=joy_valid,
+                      button0=button0)
+        B = step_field_tensors(self.in_dim, self._hd.cfg.device, fields, vel_cmd, obs, action, qdes, cmd, reset)
+        if B == 0:
+            return
+        f = capi.RawFields(*[fields[name].data_ptr() for name, _ in RAW_FIELDS])
+        capi.check(self._hd.lib.go2p_step_batch_fields(self._hd.h, C.byref(f), _ptr(reset), vel_cmd.data_ptr(),
+                                                       obs.data_ptr(), action.data_ptr(), _ptr(qdes), _ptr(cmd), B,
+                                                       precision, stream or None))
 
     def step_host(self, raw: np.ndarray, action: np.ndarray, cmd: np.ndarray | None = None,
                   precision: int = capi.PREC_FP32, reset: np.ndarray | None = None) -> None:

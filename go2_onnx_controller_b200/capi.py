@@ -35,6 +35,11 @@ class RawState(C.Structure):
     ]
 
 
+class RawFields(C.Structure):
+    """Device pointers to the per-field raw states of B robots (include/go2policy.h: go2p_raw_fields)."""
+    _fields_ = [(name, C.c_void_p) for name in ("quat", "gyro", "q", "dq", "axes", "foot_force", "joy_valid", "button0")]
+
+
 class StepOut(C.Structure):
     _fields_ = [
         ("observation", C.c_float * (GO2P_FRAME * GO2P_MAX_HISTORY)), ("action_raw", C.c_float * 12),
@@ -100,6 +105,8 @@ SIGNATURES = {
                                        C.c_int, C.c_void_p]),
     "go2p_step_batch_ex": (C.c_int, [_H, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                       C.c_int64, C.c_int, C.c_void_p]),
+    "go2p_step_batch_fields": (C.c_int, [_H, C.POINTER(RawFields), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                          C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
     "go2p_step_fused_cmd": (C.c_int, [_H, C.POINTER(RawState), C.POINTER(StepOut), C.POINTER(MotorCmd)]),
     "go2p_motor_order": (C.c_int, [C.POINTER(C.c_int32)]),
     "go2p_step_batch_host": (C.c_int, [_H, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int]),

@@ -17,6 +17,7 @@
 #include <stdexcept>
 #include <thread>
 #include <string>
+#include <utility>
 #include <vector>
 #if defined(__x86_64__)
 #include <immintrin.h>
@@ -77,7 +78,8 @@ struct go2p_handle {
   size_t tc_off[kMaxLayers] = {};              // layer l's image starts tc_off[l] elements into d_wpack[0] / [1]
   int tc_kp[kMaxLayers] = {};
   double tc_wscale[kMaxLayers] = {}, tc_bscale[kMaxLayers] = {};   // the scales pack_umma_kmajor applied
-  size_t tc_attr_smem[6] = {};                 // dynamic shared memory opted in for tc_mlp_kernel<bf16|fp16, plain|fused|fused+reset> on this device
+  size_t tc_attr_smem[10] = {};                // dynamic shared memory opted in for tc_mlp_kernel<bf16|fp16, plain|fused|fused+reset,
+                                               // records|fields> on this device
   bool b1_attr_set = false;                    // same for the one-shot batch-1 kernel
   size_t so_attr_smem = 0;                     // same for small_out_kernel
   WideModel wide{};
@@ -498,12 +500,12 @@ int launch_fp32(go2p_handle* h, int set, const float* d_obs, const int32_t* d_bu
   return GO2P_OK;
 }
 
-template <bool kFp16, bool kFused, bool kReset = false>
+template <bool kFp16, bool kFused, bool kReset = false, bool kFields = false>
 int launch_tc_t(go2p_handle* h, const TcArgs& a, cudaStream_t st) {
   const size_t smem = tc_smem_bytes(a);
-  auto kernel = tc_mlp_kernel<kFp16, kFused, kReset>;
+  auto kernel = tc_mlp_kernel<kFp16, kFused, kReset, kFields>;
   // the opt-in is a per-device function attribute: remembered per handle (one handle = one device)
-  size_t& configured = h->tc_attr_smem[(kFp16 ? 1 : 0) + (kFused ? 2 : 0) + (kReset ? 2 : 0)];
+  size_t& configured = h->tc_attr_smem[(kFp16 ? 1 : 0) + (kFused ? 2 : 0) + (kReset ? 2 : 0) + (kFields ? 4 : 0)];
   if (configured != smem) {
     CU_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     configured = smem;
@@ -529,11 +531,12 @@ int launch_tc_t(go2p_handle* h, const TcArgs& a, cudaStream_t st) {
   return GO2P_OK;
 }
 
-// raw != null: the fused controller step (A1-A6 in the conversion job): d_obs is the robots' history, updated in place;
-// d_reset (may be null) the robots' reset flags
+// raw or fields != null: the fused controller step (A1-A6 in the conversion job) from records or per-field arrays: d_obs
+// is the robots' history, updated in place; d_reset (may be null) the robots' reset flags
 int launch_tc(go2p_handle* h, const float* d_obs, const int32_t* d_button0, float* d_act, double* d_qdes,
               MotorCmdDev* d_cmd, int64_t B, bool fp16, uint32_t flags, cudaStream_t st,
-              const RawStateDev* raw = nullptr, float* d_vel_cmd = nullptr, const uint8_t* d_reset = nullptr) {
+              const RawStateDev* raw = nullptr, float* d_vel_cmd = nullptr, const uint8_t* d_reset = nullptr,
+              const RawFieldsDev* fields = nullptr) {
   if ((reinterpret_cast<uintptr_t>(d_obs) & 15) || (reinterpret_cast<uintptr_t>(d_act) & 15) ||
       (d_qdes && (reinterpret_cast<uintptr_t>(d_qdes) & 15)))
     return fail(GO2P_ERR_INVALID, "tensor-core path needs 16-byte aligned obs/act/qdes device pointers");
@@ -564,7 +567,12 @@ int launch_tc(go2p_handle* h, const float* d_obs, const int32_t* d_button0, floa
   if (const char* e = std::getenv("GO2P_TC_TRACE_PTR")) a.trace = reinterpret_cast<unsigned long long*>(std::strtoull(e, nullptr, 0));
 #endif
   a.raw = raw; a.obs_rw = const_cast<float*>(d_obs); a.vel_cmd = d_vel_cmd; a.H = h->cc.H; a.foot_threshold = h->cc.foot_threshold;
-  a.reset = raw ? d_reset : nullptr;
+  a.reset = raw || fields ? d_reset : nullptr;
+  if (fields) {
+    a.fields = *fields;
+    if (d_reset) return fp16 ? launch_tc_t<true, true, true, true>(h, a, st) : launch_tc_t<false, true, true, true>(h, a, st);
+    return fp16 ? launch_tc_t<true, true, false, true>(h, a, st) : launch_tc_t<false, true, false, true>(h, a, st);
+  }
   if (raw && d_reset) return fp16 ? launch_tc_t<true, true, true>(h, a, st) : launch_tc_t<false, true, true>(h, a, st);
   if (raw) return fp16 ? launch_tc_t<true, true>(h, a, st) : launch_tc_t<false, true>(h, a, st);
   return fp16 ? launch_tc_t<true, false>(h, a, st) : launch_tc_t<false, false>(h, a, st);
@@ -1102,29 +1110,38 @@ int go2p_assemble_batch(go2p_handle* h, const go2p_raw_state* d_raw, const float
 }
 
 namespace {
+bool aligned16(const void* p) { return !(reinterpret_cast<uintptr_t>(p) & 15); }
+
 // publish() for B robots on device buffers; button_scratch [B] receives the dead-man buttons for the epilogue.
+// The raw states are records (d_raw) or per-field arrays (fields); exactly one of the two is non-null.
 // d_reset [B] (may be null): robots to start from the initial state, applied by whichever kernel assembles the
 // observations (the fused kernel's conversion job or assemble_batch_kernel); the path choice does not depend on it.
 // `set`: the stream set whose activation scratch the policy uses.
-int step_batch_on(go2p_handle* h, int set, const go2p_raw_state* d_raw, const uint8_t* d_reset, float* d_vel_cmd, float* d_obs,
-                  float* d_action, double* d_qdes, go2p_motor_cmd* d_cmd, int32_t* button_scratch, int64_t B, int precision,
-                  cudaStream_t st) {
+int step_batch_on(go2p_handle* h, int set, const go2p_raw_state* d_raw, const RawFieldsDev* fields, const uint8_t* d_reset,
+                  float* d_vel_cmd, float* d_obs, float* d_action, double* d_qdes, go2p_motor_cmd* d_cmd,
+                  int32_t* button_scratch, int64_t B, int precision, cudaStream_t st) {
   const uint32_t all_flags = GO2P_F_CLAMP_MASK | (d_qdes ? GO2P_F_QDES : 0u) | (d_cmd ? GO2P_F_MOTOR_CMD : 0u);
   TcArgs probe{};
   probe.n_layers = h->dm.n_layers; probe.in_dim = h->dm.in_dim; probe.k0p = h->k0p;
   probe.raw = reinterpret_cast<const RawStateDev*>(d_raw);          // the fused kernel also stages the raw states
+  if (fields) probe.fields = *fields;
+  // the fused kernel bulk-copies a full tile of records, or of every field, into shared memory
+  const bool raw_aligned = fields ? aligned16(fields->quat) && aligned16(fields->gyro) && aligned16(fields->q) &&
+                                        aligned16(fields->dq) && aligned16(fields->axes) && aligned16(fields->foot_force) &&
+                                        aligned16(fields->joy_valid) && aligned16(fields->button0)
+                                  : aligned16(d_raw);
   if (h->tc_ok && (precision == GO2P_PREC_FP16 || precision == GO2P_PREC_BF16) && (h->dm.in_dim & 1) == 0 &&
-      tc_smem_bytes(probe) <= (size_t)227 * 1024 && !(reinterpret_cast<uintptr_t>(d_raw) & 15) &&
+      tc_smem_bytes(probe) <= (size_t)227 * 1024 && raw_aligned &&
       !(reinterpret_cast<uintptr_t>(d_obs) & 15) && !(reinterpret_cast<uintptr_t>(d_action) & 15) &&
       !(d_qdes && (reinterpret_cast<uintptr_t>(d_qdes) & 15)) && !(d_cmd && (reinterpret_cast<uintptr_t>(d_cmd) & 15))) {
     // ONE launch: A1-A6 run inside the policy kernel's conversion job, the newest frame never round-trips HBM
     h->last_launches = 0;
     return launch_tc(h, d_obs, nullptr, d_action, d_qdes, reinterpret_cast<MotorCmdDev*>(d_cmd), B, precision == GO2P_PREC_FP16,
-                     all_flags, st, reinterpret_cast<const RawStateDev*>(d_raw), d_vel_cmd, d_reset);
+                     all_flags, st, reinterpret_cast<const RawStateDev*>(d_raw), d_vel_cmd, d_reset, fields);
   }
   // A1-A6: d_action still holds the previous published action here
   launch_assemble_batch(reinterpret_cast<const RawStateDev*>(d_raw), d_action, d_vel_cmd, d_obs, B, h->cc, button_scratch,
-                        h->sm_count, st, d_reset);
+                        h->sm_count, st, d_reset, fields);
   CU_TRY(cudaGetLastError());
   // A7 + A9 + A11
   const uint32_t flags = GO2P_F_CLAMP_MASK | (d_qdes ? GO2P_F_QDES : 0u) | (d_cmd ? GO2P_F_MOTOR_CMD : 0u);
@@ -1132,15 +1149,14 @@ int step_batch_on(go2p_handle* h, int set, const go2p_raw_state* d_raw, const ui
   if (rc == GO2P_OK) h->last_launches += 1;
   return rc;
 }
-}  // namespace
 
-int go2p_step_batch_ex(go2p_handle* h, const go2p_raw_state* d_raw, const uint8_t* d_reset, float* d_vel_cmd, float* d_obs,
-                       float* d_action, double* d_qdes, go2p_motor_cmd* d_cmd, int64_t B, int precision, void* stream) {
-  if (!h || !d_raw || !d_vel_cmd || !d_obs || !d_action || (!d_qdes && !d_cmd))
-    return fail(GO2P_ERR_INVALID, "go2p_step_batch: null argument");
+// the device-buffer step after its pointer checks: batch and policy checks, the button scratch, stream set 0
+int step_batch_device(go2p_handle* h, const char* fn, const go2p_raw_state* d_raw, const RawFieldsDev* fields,
+                      const uint8_t* d_reset, float* d_vel_cmd, float* d_obs, float* d_action, double* d_qdes,
+                      go2p_motor_cmd* d_cmd, int64_t B, int precision, void* stream) {
   if (B <= 0) return B == 0 ? GO2P_OK : fail(GO2P_ERR_INVALID, "negative batch");
   if (h->dm.in_dim != kFrame * h->cc.H || h->dm.out_dim != kDof)
-    return fail(GO2P_ERR_INVALID, "go2p_step_batch: the policy is not a 49*H -> 12 controller policy");
+    return fail(GO2P_ERR_INVALID, std::string(fn) + ": the policy is not a 49*H -> 12 controller policy");
   DeviceGuard g(h->device);
   if (h->step_button_rows < B) {
     h->d_step_button = nullptr;   // retire (owned_alloc)
@@ -1148,8 +1164,38 @@ int go2p_step_batch_ex(go2p_handle* h, const go2p_raw_state* d_raw, const uint8_
     if (const int rc = owned_alloc(h, h->d_step_button, (size_t)B * sizeof(int32_t))) return rc;
     h->step_button_rows = B;
   }
-  return step_batch_on(h, 0, d_raw, d_reset, d_vel_cmd, d_obs, d_action, d_qdes, d_cmd, h->d_step_button, B, precision,
-                       static_cast<cudaStream_t>(stream));
+  return step_batch_on(h, 0, d_raw, fields, d_reset, d_vel_cmd, d_obs, d_action, d_qdes, d_cmd, h->d_step_button, B,
+                       precision, static_cast<cudaStream_t>(stream));
+}
+}  // namespace
+
+int go2p_step_batch_ex(go2p_handle* h, const go2p_raw_state* d_raw, const uint8_t* d_reset, float* d_vel_cmd, float* d_obs,
+                       float* d_action, double* d_qdes, go2p_motor_cmd* d_cmd, int64_t B, int precision, void* stream) {
+  if (!h || !d_raw || !d_vel_cmd || !d_obs || !d_action || (!d_qdes && !d_cmd))
+    return fail(GO2P_ERR_INVALID, "go2p_step_batch: null argument");
+  return step_batch_device(h, "go2p_step_batch", d_raw, nullptr, d_reset, d_vel_cmd, d_obs, d_action, d_qdes, d_cmd, B,
+                           precision, stream);
+}
+
+int go2p_step_batch_fields(go2p_handle* h, const go2p_raw_fields* f, const uint8_t* d_reset, float* d_vel_cmd,
+                           float* d_obs, float* d_action, double* d_qdes, go2p_motor_cmd* d_cmd, int64_t B,
+                           int precision, void* stream) {
+  const char* fn = "go2p_step_batch_fields";
+  if (!h) return fail(GO2P_ERR_INVALID, std::string(fn) + ": null handle");
+  if (!f) return fail(GO2P_ERR_INVALID, std::string(fn) + ": null go2p_raw_fields");
+  const std::pair<const void*, const char*> ptrs[] = {
+      {f->quat, "quat"}, {f->gyro, "gyro"}, {f->q, "q"}, {f->dq, "dq"}, {f->axes, "axes"}, {f->foot_force, "foot_force"},
+      {f->joy_valid, "joy_valid"}, {f->button0, "button0"}, {d_vel_cmd, "d_vel_cmd"}, {d_obs, "d_obs"},
+      {d_action, "d_action"}};
+  for (const auto& p : ptrs)
+    if (!p.first) return fail(GO2P_ERR_INVALID, std::string(fn) + ": null " + p.second);
+  if (!d_qdes && !d_cmd) return fail(GO2P_ERR_INVALID, std::string(fn) + ": d_qdes and d_cmd are both null");
+  // the two-kernel chain reads the fields at any alignment of their element type
+  const auto addr = [](const void* p) { return reinterpret_cast<uintptr_t>(p); };
+  if (((addr(f->quat) | addr(f->gyro) | addr(f->q) | addr(f->dq) | addr(f->axes)) & 3) || (addr(f->foot_force) & 1))
+    return fail(GO2P_ERR_INVALID, std::string(fn) + ": a field is not aligned to its element size");
+  const RawFieldsDev fd{f->quat, f->gyro, f->q, f->dq, f->axes, f->foot_force, f->joy_valid, f->button0};
+  return step_batch_device(h, fn, nullptr, &fd, d_reset, d_vel_cmd, d_obs, d_action, d_qdes, d_cmd, B, precision, stream);
 }
 
 int go2p_step_batch_cmd(go2p_handle* h, const go2p_raw_state* d_raw, float* d_vel_cmd, float* d_obs, float* d_action,
@@ -1201,7 +1247,7 @@ int go2p_step_batch_host_ex(go2p_handle* h, const go2p_raw_state* h_raw, const u
   return host_pipeline(h, B, [&](int slot, int64_t r0, int64_t rows, cudaStream_t st) -> int {
     CU_TRY(cudaMemcpyAsync(f.raw[slot], h_raw + r0, (size_t)rows * sizeof(go2p_raw_state), cudaMemcpyHostToDevice, st));
     if (h_reset) CU_TRY(cudaMemcpyAsync(f.reset[slot], h_reset + r0, (size_t)rows, cudaMemcpyHostToDevice, st));
-    const int rc = step_batch_on(h, 1 + slot, f.raw[slot], h_reset ? f.reset[slot] : nullptr, f.vel + r0 * 3, f.obs + r0 * n_obs,
+    const int rc = step_batch_on(h, 1 + slot, f.raw[slot], nullptr, h_reset ? f.reset[slot] : nullptr, f.vel + r0 * 3, f.obs + r0 * n_obs,
                                  f.act + r0 * kDof, nullptr, h_cmd ? reinterpret_cast<go2p_motor_cmd*>(f.cmd[slot]) : nullptr,
                                  f.button[slot], rows, precision, st);
     if (rc) return rc;

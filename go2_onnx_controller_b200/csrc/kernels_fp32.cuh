@@ -175,12 +175,14 @@ __global__ void post_kernel(float* __restrict__ act, long long total, int out_di
 }
 
 // A1-A6 for B robots: one thread per observation element, history kept in the obs rows themselves
-// (term-major, oldest frame first; reference: controller.cpp:200-212).  raw words as in kernels_b1.cuh.
-// (RawStateDev: policy_dev.cuh)
+// (term-major, oldest frame first; reference: controller.cpp:200-212).  The raw states are records (raw, kFields =
+// false) or one array per field (fields, kFields = true; any natural alignment); both are read through the row
+// accessors of policy_dev.cuh.
 
 // button0_out (optional): the dead-man button of every robot as int32 [B], the form the batched epilogue reads.
 // A warp takes 32 robots at a time:
-//   1. their raw states (32 x 156 B, contiguous) are copied to shared memory with coalesced loads;
+//   1. their raw states (32 x 156 B of records, or 32 rows of every field) are copied to shared memory with coalesced
+//      loads;
 //   2. lane r evaluates the newest frame of robot r (49 values: gravity projection, gyro, command, q - q0, dq,
 //      previous action, contacts) -- one robot per lane, so the scalar work of a robot is not replicated over a warp --
 //      with the same device functions as the batch-1 kernel (kernels_b1.cuh), i.e. bit-identical results;
@@ -193,13 +195,19 @@ __global__ void post_kernel(float* __restrict__ act, long long total, int out_di
 constexpr int kAsmWarps = 4;
 constexpr int kAsmRawWords = 39;                        // sizeof(RawStateDev) / 4
 constexpr int kAsmRowsInFlight = 4;
+static_assert(raw_fields_tile_bytes(32) <= 32 * kAsmRawWords * 4, "a warp's per-field tile fits its record stage");
 
-template <int kPerLane>
+template <class T>
+__device__ __forceinline__ void asm_copy_rows(T* dst, const T* src, int n, int lane) {
+  for (int i = lane; i < n; i += 32) dst[i] = src[i];
+}
+
+template <int kPerLane, bool kFields = false>
 __global__ void __launch_bounds__(kAsmWarps * 32)
 assemble_batch_kernel(const RawStateDev* __restrict__ raw, const float* __restrict__ prev_action,
                       float* __restrict__ vel_cmd, float* __restrict__ obs, long long B, CtrlConst cc,
-                      int32_t* __restrict__ button0_out, const uint8_t* __restrict__ reset) {
-  __shared__ uint32_t s_raw[kAsmWarps][32 * kAsmRawWords];
+                      int32_t* __restrict__ button0_out, const uint8_t* __restrict__ reset, const RawFieldsDev fields) {
+  __shared__ __align__(16) uint32_t s_raw[kAsmWarps][32 * kAsmRawWords];
   __shared__ float s_new[kAsmWarps][32 * kFrame];
   const int H = cc.H, n_obs = kFrame * H;
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -225,26 +233,40 @@ assemble_batch_kernel(const RawStateDev* __restrict__ raw, const float* __restri
   for (long long grp = (long long)blockIdx.x * kAsmWarps + wid; grp < n_groups; grp += (long long)gridDim.x * kAsmWarps) {
     const long long row0 = grp * 32;
     const int rows = (int)min(32LL, B - row0);
-    // 1. raw states of the group -> shared memory (contiguous words, coalesced)
-    const uint32_t* gr = reinterpret_cast<const uint32_t*>(raw + row0);
-    for (int i = lane; i < rows * kAsmRawWords; i += 32) my_raw[i] = gr[i];
+    // 1. raw states of the group -> shared memory (contiguous words, coalesced; per field: a raw_fields_tile of 32 rows)
+    if constexpr (kFields) {
+      const RawFieldsDev t = raw_fields_tile(my_raw, 32);
+      asm_copy_rows(const_cast<float*>(t.quat), fields.quat + row0 * 4, rows * 4, lane);
+      asm_copy_rows(const_cast<float*>(t.gyro), fields.gyro + row0 * 3, rows * 3, lane);
+      asm_copy_rows(const_cast<float*>(t.q), fields.q + row0 * kDof, rows * kDof, lane);
+      asm_copy_rows(const_cast<float*>(t.dq), fields.dq + row0 * kDof, rows * kDof, lane);
+      asm_copy_rows(const_cast<float*>(t.axes), fields.axes + row0 * 4, rows * 4, lane);
+      asm_copy_rows(const_cast<int16_t*>(t.foot_force), fields.foot_force + row0 * 4, rows * 4, lane);
+      asm_copy_rows(const_cast<uint8_t*>(t.joy_valid), fields.joy_valid + row0, rows, lane);
+      asm_copy_rows(const_cast<uint8_t*>(t.button0), fields.button0 + row0, rows, lane);
+    } else {
+      const uint32_t* gr = reinterpret_cast<const uint32_t*>(raw + row0);
+      for (int i = lane; i < rows * kAsmRawWords; i += 32) my_raw[i] = gr[i];
+    }
     const bool rst = reset != nullptr && lane < rows && reset[row0 + lane] != 0;   // lane r: row r's flag
     const uint32_t rst_rows = __ballot_sync(0xffffffffu, rst);                      // bit r: row r is reset
     __syncwarp();
     // 2. newest frame of robot (row0 + lane)
     if (lane < rows) {
       const long long row = row0 + lane;
-      const uint32_t* rw = my_raw + lane * kAsmRawWords;          // stride 39 words: conflict-free
-      const float* rf = reinterpret_cast<const float*>(rw);
+      const auto rr = [&] {                                        // records: stride 39 words, conflict-free
+        if constexpr (kFields) return RawFieldRow<32>{my_raw, lane};
+        else return RawRecordRow{my_raw + lane * kAsmRawWords};
+      }();
       float* nf = my_new + lane * kFrame;                          // stride 49 words: conflict-free
-      float quat[4] = {rf[0], rf[1], rf[2], rf[3]};
+      float quat[4] = {rr.quat(0), rr.quat(1), rr.quat(2), rr.quat(3)};
       float g[3];
       gravity_all(quat, g);
       nf[0] = g[0]; nf[1] = g[1]; nf[2] = g[2];
 #pragma unroll
-      for (int c = 0; c < 3; ++c) nf[3 + c] = rf[4 + c];
-      const int joy_valid = (int)rw[37];
-      float axes[4] = {rf[31], rf[32], rf[33], rf[34]};
+      for (int c = 0; c < 3; ++c) nf[3 + c] = rr.gyro(c);
+      const int joy_valid = (int)rr.joy_valid();
+      float axes[4] = {rr.axes(0), rr.axes(1), rr.axes(2), rr.axes(3)};
       float cmd[3];
       if (joy_valid) {
 #pragma unroll
@@ -259,9 +281,9 @@ assemble_batch_kernel(const RawStateDev* __restrict__ raw, const float* __restri
 #pragma unroll
       for (int c = 0; c < 3; ++c) nf[6 + c] = cmd[c];
 #pragma unroll
-      for (int c = 0; c < kDof; ++c) nf[9 + c] = __double2float_rn(__dsub_rn((double)rf[7 + c], cc.q0[c]));
+      for (int c = 0; c < kDof; ++c) nf[9 + c] = __double2float_rn(__dsub_rn((double)rr.q(c), cc.q0[c]));
 #pragma unroll
-      for (int c = 0; c < kDof; ++c) nf[21 + c] = rf[19 + c];
+      for (int c = 0; c < kDof; ++c) nf[21 + c] = rr.dq(c);
       if (prev_action && !rst) {
         const float4* pa = reinterpret_cast<const float4*>(prev_action + row * kDof);
 #pragma unroll
@@ -273,10 +295,9 @@ assemble_batch_kernel(const RawStateDev* __restrict__ raw, const float* __restri
 #pragma unroll
       for (int c = 0; c < 4; ++c) {
         const int p = c ^ 1;                                       // [1,0,3,2] (controller.hpp:99-103)
-        const int force = (int)(int16_t)(uint16_t)(rw[35 + (p >> 1)] >> (16 * (p & 1)));
-        nf[45 + c] = (force >= cc.foot_threshold) ? 1.0f : 0.0f;
+        nf[45 + c] = (rr.foot_force(p) >= cc.foot_threshold) ? 1.0f : 0.0f;
       }
-      if (button0_out) button0_out[row] = (int32_t)rw[38];
+      if (button0_out) button0_out[row] = (int32_t)rr.button0();
     }
     __syncwarp();
     // 3. shift + append, row by row, kAsmRowsInFlight rows of loads in flight
@@ -312,15 +333,18 @@ assemble_batch_kernel(const RawStateDev* __restrict__ raw, const float* __restri
 }
 
 // n_obs = 49*H floats per row: 4 elements per lane serve H <= 2, 13 serve H <= 8
+// fields != null: the raw states come from these arrays instead of raw
 inline void launch_assemble_batch(const RawStateDev* raw, const float* prev_action, float* vel_cmd, float* obs, long long B,
                                   const CtrlConst& cc, int32_t* button0_out, int sm_count, cudaStream_t st,
-                                  const uint8_t* reset = nullptr) {
+                                  const uint8_t* reset = nullptr, const RawFieldsDev* fields = nullptr) {
   const long long groups = (B + 31) / 32;
   const unsigned grid = (unsigned)std::min<long long>((groups + kAsmWarps - 1) / kAsmWarps, (long long)sm_count * 16);
-  if (kFrame * cc.H <= 128)
-    assemble_batch_kernel<4><<<grid, kAsmWarps * 32, 0, st>>>(raw, prev_action, vel_cmd, obs, B, cc, button0_out, reset);
-  else
-    assemble_batch_kernel<(kFrame * kMaxHistory + 31) / 32><<<grid, kAsmWarps * 32, 0, st>>>(raw, prev_action, vel_cmd, obs, B, cc, button0_out, reset);
+  constexpr int kWide = (kFrame * kMaxHistory + 31) / 32;
+  const RawFieldsDev f = fields ? *fields : RawFieldsDev{};
+  const bool narrow = kFrame * cc.H <= 128;
+  auto kernel = fields ? (narrow ? assemble_batch_kernel<4, true> : assemble_batch_kernel<kWide, true>)
+                       : (narrow ? assemble_batch_kernel<4> : assemble_batch_kernel<kWide>);
+  kernel<<<grid, kAsmWarps * 32, 0, st>>>(raw, prev_action, vel_cmd, obs, B, cc, button0_out, reset, f);
 }
 
 }  // namespace go2p

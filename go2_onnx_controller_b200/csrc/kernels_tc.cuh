@@ -79,6 +79,8 @@ struct TcArgs {
   // this step from the controller's initial state (controller.hpp:132-162): older frames, previous action and stored
   // joystick command 0
   const uint8_t* reset;
+  // fused step from per-field arrays (tc_mlp_kernel<., true, ., true>): read instead of raw, every pointer 16-byte aligned
+  RawFieldsDev fields;
 };
 
 #ifdef GO2P_TC_TRACE
@@ -109,8 +111,9 @@ __host__ __device__ inline size_t tc_weight_bytes(const TcArgs& a) {
 __host__ __device__ inline size_t tc_stage_bytes(const TcArgs& a) { return ((size_t)kTcTileM * a.in_dim * 4 + 127) & ~(size_t)127; }
 constexpr int kTcRawWords = 39;                               // sizeof(RawStateDev) / 4
 constexpr int kTcRawStageBytes = kTcTileM * kTcRawWords * 4;    // fused step: one tile's raw states (128 x 156 B, contiguous)
+static_assert(raw_fields_tile_bytes(kTcTileM) <= kTcRawStageBytes, "the per-field tile shares the raw stage");
 __host__ __device__ inline size_t tc_smem_bytes(const TcArgs& a) {
-  return tc_weight_bytes(a) + 2 * tc_stage_bytes(a) + 256 + 4 * kTcTileM * 4 + (a.raw ? kTcRawStageBytes : 0);
+  return tc_weight_bytes(a) + 2 * tc_stage_bytes(a) + 256 + 4 * kTcTileM * 4 + (a.raw || a.fields.quat ? kTcRawStageBytes : 0);
 }
 
 // does any half of these packed fp16 words sit at the largest finite magnitude (0x7BFF)?  (h & 0x7FFF) + 0x0401 reaches
@@ -143,18 +146,19 @@ __device__ __forceinline__ void tc_shift_append(float* term, int H, const float 
 // pa4 (cb 3) / vc (cb 0): the row's previous published action / last joystick command, loaded one job ahead.
 // rst: the row's reset flag (every column block shifts terms, so every one needs it); a reset row's previous action
 // and stored joystick command are 0, and without joystick input the 0 is written back as the row's command.
-__device__ __forceinline__ void tc_update_terms(const TcArgs& a, int cb, float* srow, const uint32_t* rw, long long grow, int* button_out,
+// rr: this robot's raw state (RawRecordRow: in the raw stage or, for a ragged tile, global memory; RawFieldRow: in the stage)
+template <class Row>
+__device__ __forceinline__ void tc_update_terms(const TcArgs& a, int cb, float* srow, const Row& rr, long long grow, int* button_out,
                                                 const float4 (&pa4)[3], const float (&vc)[3], bool rst) {
-  const float* rf = reinterpret_cast<const float*>(rw);     // this robot's raw state: 39 words (shared-memory stage, or global for a ragged tile)
   const int H = a.H;
   if (cb == 0) {
-    const float quat[4] = {rf[0], rf[1], rf[2], rf[3]};
+    const float quat[4] = {rr.quat(0), rr.quat(1), rr.quat(2), rr.quat(3)};
     float g[3];
     gravity_all(quat, g);
-    const float w[3] = {rf[4], rf[5], rf[6]};
+    const float w[3] = {rr.gyro(0), rr.gyro(1), rr.gyro(2)};
     float cmd[3];
-    if (rw[37]) {                                        // joy_ && !axes.empty() (controller.cpp:173)
-      const float axes[4] = {rf[31], rf[32], rf[33], rf[34]};
+    if (rr.joy_valid()) {                                // joy_ && !axes.empty() (controller.cpp:173)
+      const float axes[4] = {rr.axes(0), rr.axes(1), rr.axes(2), rr.axes(3)};
 #pragma unroll
       for (int c = 0; c < 3; ++c) { cmd[c] = vel_cmd_component(axes, c); a.vel_cmd[grow * 3 + c] = cmd[c]; }
     } else {
@@ -171,12 +175,12 @@ __device__ __forceinline__ void tc_update_terms(const TcArgs& a, int cb, float* 
   } else if (cb == 1) {
     float q[kDof];
 #pragma unroll
-    for (int c = 0; c < kDof; ++c) q[c] = __double2float_rn(__dsub_rn((double)rf[7 + c], a.q0[c]));   // controller.cpp:194-197
+    for (int c = 0; c < kDof; ++c) q[c] = __double2float_rn(__dsub_rn((double)rr.q(c), a.q0[c]));   // controller.cpp:194-197
     tc_shift_append<kDof>(srow + 9 * H, H, q, rst);
   } else if (cb == 2) {
     float dq[kDof];
 #pragma unroll
-    for (int c = 0; c < kDof; ++c) dq[c] = rf[19 + c];
+    for (int c = 0; c < kDof; ++c) dq[c] = rr.dq(c);
     tc_shift_append<kDof>(srow + 21 * H, H, dq, rst);
   } else {
     float pa[kDof];                                                               // previous published action
@@ -190,14 +194,30 @@ __device__ __forceinline__ void tc_update_terms(const TcArgs& a, int cb, float* 
 #pragma unroll
     for (int c = 0; c < 4; ++c) {
       const int p = c ^ 1;                                                          // [1,0,3,2] (controller.hpp:99-103)
-      const int force = (int)(int16_t)(uint16_t)(rw[35 + (p >> 1)] >> (16 * (p & 1)));
-      ct[c] = (force >= a.foot_threshold) ? 1.0f : 0.0f;
+      ct[c] = (rr.foot_force(p) >= a.foot_threshold) ? 1.0f : 0.0f;
     }
     tc_shift_append<kDof>(srow + 33 * H, H, pa, rst);
     tc_shift_append<4>(srow + 45 * H, H, ct, rst);
-    *button_out = (int)rw[38];
+    *button_out = (int)rr.button0();
   }
 }
+// L2 prefetch of one tile's per-field raw states (rows row0.. of a.fields, up to a.B): thread m of the tile's 128 takes
+// the m-th 128-byte line of every field's range (a field holds at most 48 B per row: 49 lines with misalignment).
+// A rolled loop over the fields, the pointers read from the kernel parameters: it runs where the pool holds the most
+// registers.
+__device__ __forceinline__ void tc_prefetch_fields(const TcArgs& a, long long row0, int m) {
+  const long long rows = min((long long)kTcTileM, a.B - row0);
+  static_assert(sizeof(RawFieldsDev) == 8 * sizeof(void*), "eight field pointers");
+#pragma unroll 1
+  for (int f = 0; f < 8; ++f) {
+    // bytes per row, one byte per field: quat 16, gyro 12, q 48, dq 48, axes 16, foot_force 8, joy_valid 1, button0 1
+    const long long row_bytes = (long long)((0x0101081030300C10ull >> (8 * f)) & 0xFFu);
+    const uintptr_t lo = reinterpret_cast<uintptr_t>(reinterpret_cast<const void* const*>(&a.fields)[f]) + (uintptr_t)(row0 * row_bytes);
+    const uintptr_t line = (lo & ~(uintptr_t)127) + (uintptr_t)m * 128u;
+    if (line < lo + (uintptr_t)(rows * row_bytes)) ptx::prefetch_l2(reinterpret_cast<const void*>(line));
+  }
+}
+
 // the term ranges (floats) column block cb owns in a row: [lo, hi)
 __device__ __forceinline__ void tc_term_range(int cb, int H, int& lo, int& hi) {
   lo = cb == 0 ? 0 : cb == 1 ? 9 * H : cb == 2 ? 21 * H : 33 * H;
@@ -270,6 +290,25 @@ __device__ __forceinline__ void elu_pack16(const uint32_t (&v)[16], bool has_elu
 // (measured: with everything inlined the kernel was 40 KB of SASS, above the 32 KB L1.5 instruction cache, and
 // every phase of the 18-warp pipeline paid instruction-fetch misses: ~1000 cycles for a backward branch)
 
+// ragged last tile, per-field raw states: row `grow`'s fields that column block cb reads (tc_update_terms), from global
+// memory into row m of the raw stage, which then serves the row as for a full tile (the same thread reads them back)
+__device__ __noinline__ void tc_stage_fields_row(const TcArgs& a, int cb, uint32_t* s_raw, long long grow, int m) {
+  const RawFieldsDev t = raw_fields_tile(s_raw, kTcTileM), &g = a.fields;
+  if (cb == 0) {
+    const_cast<float4*>(reinterpret_cast<const float4*>(t.quat))[m] = reinterpret_cast<const float4*>(g.quat)[grow];
+    for (int c = 0; c < 3; ++c) const_cast<float*>(t.gyro)[m * 3 + c] = g.gyro[grow * 3 + c];
+    const_cast<float4*>(reinterpret_cast<const float4*>(t.axes))[m] = reinterpret_cast<const float4*>(g.axes)[grow];
+    const_cast<uint8_t*>(t.joy_valid)[m] = g.joy_valid[grow];
+  } else if (cb == 1 || cb == 2) {
+    const float4* src = reinterpret_cast<const float4*>(cb == 1 ? g.q : g.dq) + grow * 3;
+    float4* dst = const_cast<float4*>(reinterpret_cast<const float4*>(cb == 1 ? t.q : t.dq)) + m * 3;
+    for (int j = 0; j < 3; ++j) dst[j] = src[j];
+  } else {
+    const_cast<short4*>(reinterpret_cast<const short4*>(t.foot_force))[m] = reinterpret_cast<const short4*>(g.foot_force)[grow];
+    const_cast<uint8_t*>(t.button0)[m] = g.button0[grow];
+  }
+}
+
 // layer-0 A operand of one row for a ragged last tile (read from global memory) or an odd input width
 template <bool kFp16>
 __device__ __noinline__ void tc_conv_slow(const TcArgs& a, const float* rowp, bool live, int c8_lo, int c8_hi, uint32_t a0_t) {
@@ -315,9 +354,11 @@ __device__ __noinline__ void tc_out_generic(const TcArgs& a, uint32_t o_t, long 
 
 // kReset (fused step only): the step reads a.reset.  A separate instantiation, so that the step without a mask runs
 // exactly the code it ran before resets existed (the per-element selects cost 2 % even when every flag is 0).
-template <bool kFp16, bool kFused, bool kReset = false>
+// kFields (fused step only): the raw states come from a.fields (one array per field) instead of a.raw (records).
+template <bool kFp16, bool kFused, bool kReset = false, bool kFields = false>
 __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_constant__ TcArgs a) {
   static_assert(kFused || !kReset, "resets belong to the fused controller step");
+  static_assert(kFused || !kFields, "per-field raw states belong to the fused controller step");
   extern __shared__ __align__(128) uint8_t smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 
@@ -419,13 +460,27 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
         ptx::mbar_arrive(&obs_full[s]);      // ragged last tile: the pool reads global memory directly
       }
     };
-    // fused step: tile i's raw states (contiguous 19,968 B) -> the raw stage; issued when conversion i-1 (the other
-    // slot's) has signalled, i.e. when every warp is done with the stage
+    // fused step: tile i's raw states (contiguous 19,968 B, or one bulk copy per field: 19,200 B laid out as
+    // raw_fields_tile) -> the raw stage; issued when conversion i-1 (the other slot's) has signalled, i.e. when every
+    // warp is done with the stage
     auto load_raw = [&](int i) {
       const long long row0 = (blockIdx.x + (long long)i * gridDim.x) * kTcTileM;
       if (a.B - row0 >= kTcTileM) {
-        ptx::mbar_arrive_expect_tx(raw_full, (uint32_t)kTcRawStageBytes);
-        ptx::bulk_g2s(s_raw, a.raw + row0, (uint32_t)kTcRawStageBytes, raw_full);
+        if constexpr (kFields) {
+          const RawFieldsDev t = raw_fields_tile(s_raw, kTcTileM);
+          ptx::mbar_arrive_expect_tx(raw_full, (uint32_t)raw_fields_tile_bytes(kTcTileM));
+          ptx::bulk_g2s(const_cast<float*>(t.quat), a.fields.quat + row0 * 4, kTcTileM * 4 * 4, raw_full);
+          ptx::bulk_g2s(const_cast<float*>(t.gyro), a.fields.gyro + row0 * 3, kTcTileM * 3 * 4, raw_full);
+          ptx::bulk_g2s(const_cast<float*>(t.q), a.fields.q + row0 * kDof, kTcTileM * kDof * 4, raw_full);
+          ptx::bulk_g2s(const_cast<float*>(t.dq), a.fields.dq + row0 * kDof, kTcTileM * kDof * 4, raw_full);
+          ptx::bulk_g2s(const_cast<float*>(t.axes), a.fields.axes + row0 * 4, kTcTileM * 4 * 4, raw_full);
+          ptx::bulk_g2s(const_cast<int16_t*>(t.foot_force), a.fields.foot_force + row0 * 4, kTcTileM * 4 * 2, raw_full);
+          ptx::bulk_g2s(const_cast<uint8_t*>(t.joy_valid), a.fields.joy_valid + row0, kTcTileM, raw_full);
+          ptx::bulk_g2s(const_cast<uint8_t*>(t.button0), a.fields.button0 + row0, kTcTileM, raw_full);
+        } else {
+          ptx::mbar_arrive_expect_tx(raw_full, (uint32_t)kTcRawStageBytes);
+          ptx::bulk_g2s(s_raw, a.raw + row0, (uint32_t)kTcRawStageBytes, raw_full);
+        }
       } else {
         ptx::mbar_arrive(raw_full);          // ragged last tile: the pool reads global memory directly
       }
@@ -559,9 +614,15 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
           int lo, hi;
           tc_term_range(cb, a.H, lo, hi);
           if (!full) for (int k = lo; k < hi; ++k) srow[k] = a.obs_rw[(row0 + m) * a.in_dim + k];   // ragged tile: no bulk load
-          const uint32_t* rw = full ? s_raw + m * kTcRawWords : reinterpret_cast<const uint32_t*>(a.raw + row0 + m);
-          tc_update_terms(a, cb, srow, rw, row0 + m, &s_button[(s * 2 + (pair & 1)) * kTcTileM + m], pf_act, pf_vel,
-                          pf_rst);
+          if constexpr (kFields) {
+            if (!full) tc_stage_fields_row(a, cb, s_raw, row0 + m, m);
+            tc_update_terms(a, cb, srow, RawFieldRow<kTcTileM>{s_raw, m}, row0 + m, &s_button[(s * 2 + (pair & 1)) * kTcTileM + m], pf_act,
+                            pf_vel, pf_rst);
+          } else {
+            const RawRecordRow rr{full ? s_raw + m * kTcRawWords : reinterpret_cast<const uint32_t*>(a.raw + row0 + m)};
+            tc_update_terms(a, cb, srow, rr, row0 + m, &s_button[(s * 2 + (pair & 1)) * kTcTileM + m], pf_act, pf_vel,
+                            pf_rst);
+          }
           if (!full) for (int k = lo; k < hi; ++k) a.obs_rw[(row0 + m) * a.in_dim + k] = srow[k];
         }
         TC_TRACE(0xB00u | (uint32_t)s);
@@ -692,7 +753,10 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
             // two layers ahead (no registers held, nothing waited for)
             const long long r0 = (blockIdx.x + (long long)(pair * 2 + 2 + (cb & 1)) * gridDim.x) * kTcTileM + m;
             if (r0 < a.B) {
-              if (cb < 2) { ptx::prefetch_l2(a.raw + r0); ptx::prefetch_l2(reinterpret_cast<const uint8_t*>(a.raw + r0) + sizeof(RawStateDev) - 1); }
+              if (cb < 2) {
+                if constexpr (kFields) tc_prefetch_fields(a, r0 - m, m);
+                else { ptx::prefetch_l2(a.raw + r0); ptx::prefetch_l2(reinterpret_cast<const uint8_t*>(a.raw + r0) + sizeof(RawStateDev) - 1); }
+              }
               else { ptx::prefetch_l2(a.act + r0 * kDof); ptx::prefetch_l2(a.vel_cmd + r0 * 3); }
             }
           }

@@ -37,13 +37,76 @@ struct CtrlConst {
 };
 
 // Everything publish() reads from the outside world for one robot and one control step (include/go2policy.h:
-// go2p_raw_state); as 32-bit words: quat 0-3, gyro 4-6, q 7-18, dq 19-30, axes 31-34, foot_force 35-36 (4 x int16),
-// joy_valid 37, button0 38.
+// go2p_raw_state), read through RawRecordRow below.
 struct RawStateDev {
   float quat[4]; float gyro[3]; float q[12]; float dq[12]; float axes[4];
   int16_t foot_force[4]; int32_t joy_valid; int32_t button0;
 };
 static_assert(sizeof(RawStateDev) == 4 * 35 + 8 + 8, "must match go2p_raw_state");
+
+// The same quantities as one array per field (include/go2policy.h: go2p_raw_fields), row-major, B rows each.  The flags
+// are one byte: every reader compares them with 0.
+struct RawFieldsDev {
+  const float* quat;            // [B,4]
+  const float* gyro;            // [B,3]
+  const float* q;               // [B,12]
+  const float* dq;              // [B,12]
+  const float* axes;            // [B,4]
+  const int16_t* foot_force;    // [B,4]
+  const uint8_t* joy_valid;     // [B]
+  const uint8_t* button0;       // [B]
+};
+// a tile of `rows` robots' fields packed one field after the other (quat, gyro, q, dq, axes, foot_force, joy_valid,
+// button0): the shared-memory form.  For rows a multiple of 4 every field starts 16-byte aligned.
+__host__ __device__ constexpr int raw_fields_tile_bytes(int rows) { return rows * (35 * 4 + 4 * 2 + 2); }
+__host__ __device__ inline RawFieldsDev raw_fields_tile(const void* base, int rows) {
+  const uint8_t* p = static_cast<const uint8_t*>(base);
+  RawFieldsDev f;
+  f.quat = reinterpret_cast<const float*>(p);
+  f.gyro = f.quat + rows * 4;
+  f.q = f.gyro + rows * 3;
+  f.dq = f.q + rows * kDof;
+  f.axes = f.dq + rows * kDof;
+  f.foot_force = reinterpret_cast<const int16_t*>(f.axes + rows * 4);
+  f.joy_valid = reinterpret_cast<const uint8_t*>(f.foot_force + rows * 4);
+  f.button0 = f.joy_valid + rows;
+  return f;
+}
+
+// One robot's raw state, read field by field: the only code that knows where a field sits in either layout.
+// RawRecordRow: a go2p_raw_state record as 39 words (quat 0-3, gyro 4-6, q 7-18, dq 19-30, axes 31-34, foot_force 35-36
+// as 4 x int16, joy_valid 37, button0 38); any 4-byte alignment.
+struct RawRecordRow {
+  const uint32_t* w;
+  __device__ __forceinline__ float quat(int i) const { return reinterpret_cast<const float*>(w)[i]; }
+  __device__ __forceinline__ float gyro(int i) const { return reinterpret_cast<const float*>(w)[4 + i]; }
+  __device__ __forceinline__ float q(int i) const { return reinterpret_cast<const float*>(w)[7 + i]; }
+  __device__ __forceinline__ float dq(int i) const { return reinterpret_cast<const float*>(w)[19 + i]; }
+  __device__ __forceinline__ float axes(int i) const { return reinterpret_cast<const float*>(w)[31 + i]; }
+  __device__ __forceinline__ int foot_force(int i) const { return (int)(int16_t)(uint16_t)(w[35 + (i >> 1)] >> (16 * (i & 1))); }
+  __device__ __forceinline__ uint32_t joy_valid() const { return w[37]; }
+  __device__ __forceinline__ uint32_t button0() const { return w[38]; }
+};
+// RawFieldRow: row r of a raw_fields_tile of kRows rows in shared memory; each group of 4 floats is one 16-byte load
+// and the foot forces one 8-byte load (the compiler merges the loads of one group).
+template <int kRows>
+struct RawFieldRow {
+  const void* tile;
+  int r;
+  __device__ __forceinline__ RawFieldsDev f() const { return raw_fields_tile(tile, kRows); }
+  __device__ __forceinline__ static float pick(const float4& t, int i) { return (i & 3) == 0 ? t.x : (i & 3) == 1 ? t.y : (i & 3) == 2 ? t.z : t.w; }
+  __device__ __forceinline__ float quat(int i) const { return pick(reinterpret_cast<const float4*>(f().quat)[r], i); }
+  __device__ __forceinline__ float gyro(int i) const { return f().gyro[r * 3 + i]; }
+  __device__ __forceinline__ float q(int i) const { return pick(reinterpret_cast<const float4*>(f().q)[r * 3 + (i >> 2)], i); }
+  __device__ __forceinline__ float dq(int i) const { return pick(reinterpret_cast<const float4*>(f().dq)[r * 3 + (i >> 2)], i); }
+  __device__ __forceinline__ float axes(int i) const { return pick(reinterpret_cast<const float4*>(f().axes)[r], i); }
+  __device__ __forceinline__ int foot_force(int i) const {
+    const short4 t = reinterpret_cast<const short4*>(f().foot_force)[r];
+    return (int)((i & 3) == 0 ? t.x : (i & 3) == 1 ? t.y : (i & 3) == 2 ? t.z : t.w);
+  }
+  __device__ __forceinline__ uint32_t joy_valid() const { return f().joy_valid[r]; }
+  __device__ __forceinline__ uint32_t button0() const { return f().button0[r]; }
+};
 
 // What Go2RobotInterface::send_command receives from publish() (controller.cpp:235-251), in UNITREE motor order:
 // motor u = leg_u*3 + joint with legs FR, FL, RR, RL and joints hip, thigh, calf, while the policy works in Isaac order

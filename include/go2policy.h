@@ -224,6 +224,26 @@ int go2p_step_batch_cmd(go2p_handle* h, const go2p_raw_state* d_raw, float* d_ve
 int go2p_step_batch_ex(go2p_handle* h, const go2p_raw_state* d_raw, const uint8_t* d_reset, float* d_vel_cmd,
                        float* d_obs, float* d_action, double* d_qdes, go2p_motor_cmd* d_cmd, int64_t B,
                        int precision, void* stream);
+/* The raw states of B robots as one DEVICE array per field, the way a GPU simulator keeps them: row-major, contiguous,
+ * B rows each, every pointer aligned to its element type.  Meaning of each field as in go2p_raw_state. */
+typedef struct go2p_raw_fields {
+  const float* quat;           /* [B,4]  w,x,y,z                                              */
+  const float* gyro;           /* [B,3]                                                       */
+  const float* q;              /* [B,12]                                                      */
+  const float* dq;             /* [B,12]                                                      */
+  const float* axes;           /* [B,4]                                                       */
+  const int16_t* foot_force;   /* [B,4]  unitree order                                        */
+  const uint8_t* joy_valid;    /* [B]    non-zero = joy_ && !axes.empty() (a torch.bool qualifies) */
+  const uint8_t* button0;      /* [B]    non-zero = dead-man button pressed                  */
+} go2p_raw_fields;
+/* go2p_step_batch_ex with the raw states read from per-field device arrays instead of go2p_raw_state records: it
+ * computes exactly what go2p_step_batch_ex computes from records that hold the same values (flags compared with 0), with
+ * the same argument rules, reset rule and launch count.  The one-launch path (fp16 / bf16) needs every field pointer
+ * 16-byte aligned where the record form needs d_raw so; otherwise the step takes the two-kernel chain, as records do.
+ * A NULL handle, f or field is GO2P_ERR_INVALID. */
+int go2p_step_batch_fields(go2p_handle* h, const go2p_raw_fields* f, const uint8_t* d_reset, float* d_vel_cmd,
+                           float* d_obs, float* d_action, double* d_qdes, go2p_motor_cmd* d_cmd, int64_t B,
+                           int precision, void* stream);
 /* go2p_step_fused + the same step's send_command arguments in motor order (out may be NULL) */
 int go2p_step_fused_cmd(go2p_handle* h, const go2p_raw_state* raw, go2p_step_out* out, go2p_motor_cmd* cmd);
 /* isaac_of_motor[u] = Isaac joint index of Unitree motor u */
