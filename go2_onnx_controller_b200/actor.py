@@ -305,7 +305,11 @@ class Go2Controller:
 
 
 class PolicyBatch:
-    """Batched inference.  Device tensors are passed as raw pointers (torch ``.data_ptr()`` or go2p_dev_alloc)."""
+    """Batched inference.  Device tensors are passed as raw pointers (torch ``.data_ptr()`` or go2p_dev_alloc).
+
+    ``precision`` of every method: capi.PREC_FP32 (the default: CUDA cores, the reference's 1e-5 contract),
+    capi.PREC_FP32_TC (the same 1e-5 contract on the tensor cores, each operand split into three bf16 pieces; not
+    bit-identical to PREC_FP32), capi.PREC_FP16 or capi.PREC_BF16 (16-bit operands, looser tolerances)."""
 
     def __init__(self, model_path: str = DEFAULT_MODEL, device: int = 0, **cfg):
         self._hd = _Handle(model_path, default_config(device=device, **cfg))
@@ -317,7 +321,8 @@ class PolicyBatch:
 
     def infer_device(self, d_obs: int, d_act: int, B: int, precision: int = capi.PREC_FP32, stream: int = 0,
                      d_button0: int | None = None, d_qdes: int | None = None, flags: int = 0, d_cmd: int | None = None) -> None:
-        """precision defaults to the reference's (fp32, 1e-5 contract); the tensor-core precisions are opt-in."""
+        """precision defaults to the reference's (fp32, 1e-5 contract); the tensor-core precisions are opt-in, and
+        PREC_FP32_TC keeps the 1e-5 contract."""
         capi.check(self._hd.lib.go2p_infer_batch_cmd(self._hd.h, d_obs, d_button0, d_act, d_qdes, d_cmd, B, precision, flags,
                                                      stream or None))
 
@@ -428,7 +433,8 @@ class PolicyBatch:
 
 class Fleet:
     """One process, several GPUs: rows are split into contiguous shards, one handle + host thread per device
-    (include/go2policy.h: go2p_fleet_*).  No data crosses between devices."""
+    (include/go2policy.h: go2p_fleet_*).  No data crosses between devices.  ``precision`` as in PolicyBatch: PREC_FP32
+    by default, PREC_FP32_TC for the same accuracy on the tensor cores, PREC_FP16 / PREC_BF16."""
 
     def __init__(self, model_path: str = DEFAULT_MODEL, devices=(0,), **cfg):
         self.lib = capi.load()

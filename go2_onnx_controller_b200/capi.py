@@ -13,6 +13,7 @@ GO2P_MAX_LAYERS = 8
 
 OK, ERR_INVALID, ERR_IO, ERR_MODEL, ERR_CUDA, ERR_NO_DEVICE, ERR_UNSUPPORTED, ERR_STATE, ERR_TIMEOUT = range(9)
 PREC_FP32, PREC_BF16, PREC_FP16 = 0, 1, 2
+PREC_FP32_TC = 4               # fp32 accuracy on the tensor cores (three bf16 pieces per operand); 3 is rejected
 B1_PERSISTENT, B1_GRAPH, B1_LAUNCH = 0, 1, 2
 F_CLAMP_MASK, F_QDES, F_MOTOR_CMD, F_SAT_COUNT = 1, 2, 4, 8
 

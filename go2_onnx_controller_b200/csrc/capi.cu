@@ -72,7 +72,8 @@ struct go2p_handle {
   CtrlConst cc{};
   // tensor-core path
   bool tc_ok = false;
-  bool wide_ok = false;
+  bool wide_ok = false;                        // bf16 / fp16 on the per-layer GEMMs
+  bool split_ok = false;                       // GO2P_PREC_FP32_TC on the per-layer GEMMs (wide.L[l].w3)
   uint16_t* d_wpack[2] = {nullptr, nullptr};   // [0] bf16, [1] fp16
   int k0p = 0;
   size_t tc_off[kMaxLayers] = {};              // layer l's image starts tc_off[l] elements into d_wpack[0] / [1]
@@ -82,12 +83,13 @@ struct go2p_handle {
                                                // records|fields> on this device
   bool b1_attr_set = false;                    // same for the one-shot batch-1 kernel
   size_t so_attr_smem = 0;                     // same for small_out_kernel
+  size_t split_attr_smem[3] = {};              // same for wide_gemm_kernel<128 | 64 | 16, split>
   WideModel wide{};
   // activation ping-pong buffers between the per-layer launches of the fp32 path and of the wide path, one pair per
   // stream set: set 0 serves the device-pointer API, sets 1..kPipeDepth the streams of the host-buffer pipeline (which
   // run concurrently)
   struct Scratch { void* buf[2] = {nullptr, nullptr}; int64_t rows = 0; };
-  Scratch fp32_scratch[1 + kPipeDepth], wide_scratch[1 + kPipeDepth];
+  Scratch fp32_scratch[1 + kPipeDepth], wide_scratch[1 + kPipeDepth], split_scratch[1 + kPipeDepth];
   // batch-1
   B1State* d_state = nullptr;
   int32_t* d_step_button = nullptr;   // go2p_step_batch: dead-man buttons extracted by the assembly kernel
@@ -288,12 +290,12 @@ int upload_model(go2p_handle* h) {
       h->tc_ok = true;
     }
   }
-  if (!h->tc_ok) {
-    auto alloc = [h](size_t bytes) { void* p = nullptr; return owned_alloc(h, p, bytes) ? nullptr : p; };
-    int rc = wide_prepare(m, alloc, &h->wide, g_err);
-    if (rc == 0) h->wide_ok = true;
-    else if (rc > 0) return rc;   // CUDA failure; rc < 0 means "shape not served"
-  }
+  // the per-layer GEMMs: bf16 / fp16 for the shapes the one-launch kernel does not serve, GO2P_PREC_FP32_TC for every
+  // shape they serve
+  auto alloc = [h](size_t bytes) { void* p = nullptr; return owned_alloc(h, p, bytes) ? nullptr : p; };
+  int rc = wide_prepare(m, alloc, &h->wide, !h->tc_ok, g_err);
+  if (rc == 0) { h->wide_ok = !h->tc_ok; h->split_ok = true; }
+  else if (rc > 0) return rc;     // CUDA failure; rc < 0 means "shape not served"
   return GO2P_OK;
 }
 
@@ -1001,6 +1003,18 @@ int go2p_b1_stats_get(go2p_handle* h, go2p_b1_stats* out, int reset) {
 
 // ------------------------------------------------------------------------------------- batched
 namespace {
+// the per-layer GEMM chain (kernels_wide.cuh) with the activation buffers sc of one stream set
+int launch_wide(go2p_handle* h, go2p_handle::Scratch& sc, WdOperands operands, const float* d_obs, const int32_t* d_button0,
+                float* d_act, double* d_qdes, MotorCmdDev* cmd, int64_t B, uint32_t flags, cudaStream_t st) {
+  const size_t pieces = operands == kWdSplit ? 3 : 1;
+  if (ensure_scratch(h, sc, wide_act_rows(B), pieces * h->wide.max_kp * sizeof(uint16_t)))
+    return fail(GO2P_ERR_CUDA, "wide_launch: cudaMalloc of the activation buffers failed");
+  uint16_t* const act[2] = {static_cast<uint16_t*>(sc.buf[0]), static_cast<uint16_t*>(sc.buf[1])};
+  int rc = wide_launch(h->wide, act, d_obs, d_button0, d_act, d_qdes, cmd, B, operands, flags, h->cc, h->sm_count,
+                       h->split_attr_smem, st, &h->last_launches, g_err);
+  return rc ? fail(rc, g_err.c_str()) : GO2P_OK;
+}
+
 // go2p_infer_batch_cmd with the activation scratch of stream set `set`
 int infer_batch_on(go2p_handle* h, int set, const float* d_obs, const int32_t* d_button0, float* d_act, double* d_qdes,
                    go2p_motor_cmd* d_cmd, int64_t B, int precision, uint32_t flags, cudaStream_t st) {
@@ -1022,16 +1036,14 @@ int infer_batch_on(go2p_handle* h, int set, const float* d_obs, const int32_t* d
     case GO2P_PREC_BF16:
     case GO2P_PREC_FP16:
       if (h->tc_ok) return launch_tc(h, d_obs, d_button0, d_act, d_qdes, cmd, B, precision == GO2P_PREC_FP16, flags, st);
-      if (h->wide_ok) {
-        go2p_handle::Scratch& sc = h->wide_scratch[set];
-        if (ensure_scratch(h, sc, wide_act_rows(B), (size_t)h->wide.max_kp * sizeof(uint16_t)))
-          return fail(GO2P_ERR_CUDA, "wide_launch: cudaMalloc of the activation buffers failed");
-        uint16_t* const act[2] = {static_cast<uint16_t*>(sc.buf[0]), static_cast<uint16_t*>(sc.buf[1])};
-        int rc = wide_launch(h->wide, act, d_obs, d_button0, d_act, d_qdes, cmd, B, precision == GO2P_PREC_FP16, flags, h->cc,
-                             h->sm_count, st, &h->last_launches, g_err);
-        return rc ? fail(rc, g_err.c_str()) : GO2P_OK;
-      }
+      if (h->wide_ok)
+        return launch_wide(h, h->wide_scratch[set], precision == GO2P_PREC_FP16 ? kWdFp16 : kWdBf16, d_obs, d_button0, d_act,
+                           d_qdes, cmd, B, flags, st);
       return fail(GO2P_ERR_UNSUPPORTED, "tensor-core kernels do not serve this layer shape; use GO2P_PREC_FP32");
+    case GO2P_PREC_FP32_TC:
+      if (h->split_ok) return launch_wide(h, h->split_scratch[set], kWdSplit, d_obs, d_button0, d_act, d_qdes, cmd, B, flags, st);
+      return fail(GO2P_ERR_UNSUPPORTED, "GO2P_PREC_FP32_TC serves 2-8 layers, hidden widths that are multiples of 64 and at "
+                                        "most 16 outputs; use GO2P_PREC_FP32");
     default: return fail(GO2P_ERR_INVALID, "unknown precision");
   }
 }
@@ -1329,6 +1341,10 @@ int pack_and_publish(go2p_handle* h, const float* const* w, const float* const* 
       for (int f = 0; f < 2; ++f) P.wd[f] = const_cast<uint16_t*>(W.w[f]);
       P.wd_bias = const_cast<float*>(W.bias); P.wd_NT = W.NT; P.wd_Kp = W.Kp;
     }
+    if (h->split_ok) {
+      const WideLayerDev& W = h->wide.L[l];
+      pa.S[l] = PackSplitLayer{const_cast<uint16_t*>(W.w3), const_cast<float*>(W.bias), W.NT3, W.Kp};
+    }
     widest = std::max<long long>(widest, (long long)D.N * (D.K + 1));
   }
   if (mean) {
@@ -1341,7 +1357,9 @@ int pack_and_publish(go2p_handle* h, const float* const* w, const float* const* 
     pa.L[0].b = h->w_fold + (size_t)N * K;
   }
   const int blocks = (int)std::min<long long>((widest + 255) / 256, (long long)h->sm_count * 4);
-  pack_weights_kernel<<<dim3((unsigned)blocks, (unsigned)dm.n_layers), 256, 0, st>>>(pa);
+  const dim3 grid((unsigned)blocks, (unsigned)dm.n_layers);
+  if (h->split_ok) pack_weights_kernel<true><<<grid, 256, 0, st>>>(pa);
+  else pack_weights_kernel<false><<<grid, 256, 0, st>>>(pa);
   CU_TRY(cudaGetLastError());
   CU_TRY(cudaEventRecord(h->w_event, st));
   for (cudaStream_t s : own_streams(h))

@@ -5,7 +5,8 @@
 //                            prefix), into a scratch copy of layer 0
 //   pack_weights_kernel      per layer: the fp32 layouts of DevLayer (w_rm, w_k4, w_kn, bias), the 16-bit UMMA K-major
 //                            images of the narrow tensor-core kernel (capi.cu: pack_umma_kmajor) and the blocked tiles +
-//                            padded bias of the wide GEMMs (kernels_wide.cuh: wd_pack_weights)
+//                            padded bias of the wide GEMMs (kernels_wide.cuh: wd_pack_weights), and with kSplit the
+//                            three-piece bf16 images of GO2P_PREC_FP32_TC (wd_pack_split)
 //
 // The images must be byte-identical to what the host packers produce for the same tensors.  The host code is built
 // without -march, so it has no FMA; the device compiler contracts a*b+c into FMA by default.  Every rounding step is
@@ -40,9 +41,17 @@ struct PackLayer {
   int wd_NT, wd_Kp;
 };
 
+// the split images of GO2P_PREC_FP32_TC (kernels_wide.cuh: wd_pack_split)
+struct PackSplitLayer {
+  uint16_t* w3;
+  float* bias;             // the wide GEMMs' padded bias
+  int NT, Kp;
+};
+
 struct PackArgs {
   PackLayer L[kMaxLayers];
   int n_layers;
+  PackSplitLayer S[kMaxLayers];   // read by pack_weights_kernel<true> only; after n_layers, so L keeps its offsets
 };
 
 // capi.cu: to_bf16 / to_f16 / from_bf16 / from_f16.  std::max(-65504.f, f) is (-65504 < f ? f : -65504) and
@@ -78,7 +87,9 @@ __global__ void fold_normaliser_kernel(const float* __restrict__ w, const float*
   b_out[o] = __double2float_rn(acc);
 }
 
-// blockIdx.y = layer; a grid-stride walk over its N x (K + 1) elements, column K standing for the bias
+// blockIdx.y = layer; a grid-stride walk over its N x (K + 1) elements, column K standing for the bias.  kSplit: also the
+// split images (a.S) of a handle that serves GO2P_PREC_FP32_TC
+template <bool kSplit>
 __global__ void pack_weights_kernel(const __grid_constant__ PackArgs a) {
   const PackLayer& L = a.L[blockIdx.y];
   const long long total = (long long)L.N * (L.K + 1);
@@ -103,6 +114,15 @@ __global__ void pack_weights_kernel(const __grid_constant__ PackArgs a) {
         L.wd[0][idx] = __bfloat16_as_ushort(__float2bfloat16_rn(v));
         L.wd[1][idx] = __half_as_ushort(__float2half_rn(c));
       }
+      if constexpr (kSplit) {
+        const PackSplitLayer& S = a.S[blockIdx.y];
+        const size_t tile_elems = (size_t)S.NT * kWdChunkK;
+        const size_t idx = ((size_t)(n / S.NT) * (S.Kp / kWdChunkK) + k / kWdChunkK) * 3 * tile_elems + wd_tile_offset(n % S.NT, k % kWdChunkK) / 2;
+        uint16_t p[3];
+        wd_split_weight(v, p);
+#pragma unroll
+        for (int q = 0; q < 3; ++q) S.w3[idx + q * tile_elems] = p[q];
+      }
     } else {
       const float v = L.b ? L.b[n] : 0.f;
       L.bias[n] = v;
@@ -119,6 +139,7 @@ __global__ void pack_weights_kernel(const __grid_constant__ PackArgs a) {
         }
       }
       if (L.wd[0]) L.wd_bias[n] = v;
+      if constexpr (kSplit) a.S[blockIdx.y].bias[n] = v;
     }
   }
 }

@@ -36,9 +36,10 @@ constexpr int kWdChunkK = 64;                       // K columns per pipeline st
 constexpr int kWdATileBytes = kWdTileM * kWdChunkK * 2;   // 16 KB
 constexpr int kWdStages = 4;                        // 4 x 48 KB (N tile 256) = 192 KB of operands in flight per SM
 // operand ring depth: as many stages as fit in ~192 KB (the L2 round trip under load is ~4,000 cycles, so the bytes in
-// flight, not the stage count, set the delivered bandwidth), at most 8
-__host__ __device__ constexpr int wd_stages(int nt, bool pair) {
-  const int stage = 128 * 64 * 2 + (pair ? nt / 2 : nt) * 64 * 2;
+// flight, not the stage count, set the delivered bandwidth), at most 8.  split: a stage holds three bf16 pieces of each
+// operand (GO2P_PREC_FP32_TC)
+__host__ __device__ constexpr int wd_stages(int nt, bool pair, bool split = false) {
+  const int stage = (split ? 3 : 1) * (128 * 64 * 2 + (pair ? nt / 2 : nt) * 64 * 2);
   const int n = (192 * 1024) / stage;
   return n > 8 ? 8 : n;
 }
@@ -54,10 +55,46 @@ __host__ __device__ inline uint32_t wd_tile_offset(int r, int c) {
   return (uint32_t)(((r >> 3) * 8 + (c >> 3)) * 128 + (r & 7) * 16 + (c & 7) * 2);
 }
 
+// ---- GO2P_PREC_FP32_TC: every fp32 operand as three bf16 pieces (DESIGN.md §3.3c).  A split tile group is the hi, mid
+// and lo tiles of one (row or N tile, K chunk), 16-bit blocked images as above, stored one after the other.
+//
+// Activations (the A operand): x = h + m + l, h = bf16_rn(x), m = bf16_rn(x - h), l = x - h - m (exact in bf16): 24
+// significand bits, fp32's exponent range.  +-Inf and NaN ride in h alone with m = l = 0 (x - h would be NaN); a finite
+// x beyond bf16's largest finite value is truncated into h instead of rounding to Inf.
+__device__ __forceinline__ void wd_split_act(float x, float& h, float& m, float& l) {
+  const bool fin = fabsf(x) <= 3.40282347e38f;
+  float t = __bfloat162float(__float2bfloat16_rn(x));
+  if (fin && isinf(t)) t = __bfloat162float(__float2bfloat16_rz(x));
+  const float r = fin ? __fsub_rn(x, t) : 0.f;
+  h = t;
+  m = __bfloat162float(__float2bfloat16_rn(r));
+  l = __fsub_rn(r, m);
+}
+
+// Weights (the B operand): W = h + m + l with h = bf16_rz(W), m = bf16_rz(W - h), l = W - h - m, so every piece has W's
+// sign, and for W != 0 a piece that would be 0 holds bf16_rz(W * 2^-32) instead (2^-32 of W: far below the contract).
+// An Inf activation then meets three products of one sign and no zero -- Inf * W stays +-Inf as in the reference instead
+// of turning into Inf - Inf or Inf * 0 = NaN.  Every operation is exact, so the host packer and the device packer
+// (kernels_pack.cuh) agree bit for bit without explicit rounding modes.
+__host__ __device__ inline void wd_split_weight(float w, uint16_t p[3]) {
+  const __nv_bfloat16 h = __float2bfloat16_rz(w);
+  const float r = w - __bfloat162float(h);
+  const __nv_bfloat16 m = __float2bfloat16_rz(r);
+  const __nv_bfloat16 l = __float2bfloat16_rz(r - __bfloat162float(m));
+  const uint16_t tiny = __bfloat16_as_ushort(__float2bfloat16_rz(w * 0x1p-32f));
+  const bool nz = w != 0.f;
+  p[0] = __bfloat16_as_ushort(h);
+  p[1] = (nz && __bfloat162float(m) == 0.f) ? tiny : __bfloat16_as_ushort(m);
+  p[2] = (nz && __bfloat162float(l) == 0.f) ? tiny : __bfloat16_as_ushort(l);
+}
+
 struct WideLayerDev {
-  const uint16_t* w[2];    // [0] bf16, [1] fp16: per (n tile, k chunk) blocked image, NT rows x 64
+  const uint16_t* w[2];    // [0] bf16, [1] fp16: per (n tile, k chunk) blocked image, NT rows x 64 (null for a model
+                           // the one-launch kernel serves: only the split images are built for it)
+  const uint16_t* w3;      // GO2P_PREC_FP32_TC: per (n tile, k chunk) the hi, mid and lo bf16 images, NT3 rows x 64 each
   const float* bias;       // [Npad]
   int K, N, Kp, Np, NT;    // Kp multiple of 64, Np multiple of NT
+  int NT3;                 // N tile of the split images (Np is a multiple of it too)
   int has_elu;
   float alpha;
 };
@@ -93,7 +130,8 @@ struct WideGemmArgs {
 // A warp converts 8 rows x 32 columns: lane = (column group of 8) * 8 + (row & 7), so its 32 16-byte stores are the four
 // K-adjacent cores of one 8-row group -- 512 contiguous bytes (the first version walked along a row: every lane's
 // 16 bytes went to a different 128-byte line, and the conversion took 34 us of a 195-us pass).
-template <bool kFp16>
+// kSplit: the three bf16 pieces of every value into the row tile's split tile group (wd_split_act)
+template <bool kFp16, bool kSplit = false>
 __global__ void obs_to_blocked_kernel(const float* __restrict__ obs, uint16_t* __restrict__ out, long long B, int in_dim, int Kp,
                                       long long m_tiles) {
   const int kg4 = Kp / 32;                                           // groups of four 8-column cores per row
@@ -109,6 +147,27 @@ __global__ void obs_to_blocked_kernel(const float* __restrict__ obs, uint16_t* _
     const int kg = (int)(it % kg4) * 4 + cgl;                        // this lane's 8-column core
     const long long row = rg * 8 + r8;
     const float* src = obs + row * in_dim + kg * 8;
+    if constexpr (kSplit) {
+      uint32_t p[3][4];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const int k = kg * 8 + 2 * j;
+        const float x0 = (row < B && k < in_dim) ? src[2 * j] : 0.f;
+        const float x1 = (row < B && k + 1 < in_dim) ? src[2 * j + 1] : 0.f;
+        float s0[3], s1[3];
+        wd_split_act(x0, s0[0], s0[1], s0[2]);
+        wd_split_act(x1, s1[0], s1[1], s1[2]);
+#pragma unroll
+        for (int q = 0; q < 3; ++q) p[q][j] = ptx::pack_bf16(s0[q], s1[q]);
+      }
+      const long long mt = row / kWdTileM;
+      const int r = (int)(row % kWdTileM);
+      const int kc = (kg * 8) / kWdChunkK, c = (kg * 8) % kWdChunkK;
+      uint8_t* dst = reinterpret_cast<uint8_t*>(out) + ((mt * (Kp / kWdChunkK) + kc) * 3 * (long long)kWdATileBytes) + wd_tile_offset(r, c);
+#pragma unroll
+      for (int q = 0; q < 3; ++q) *reinterpret_cast<uint4*>(dst + q * kWdATileBytes) = make_uint4(p[q][0], p[q][1], p[q][2], p[q][3]);
+      continue;
+    }
     uint32_t p[4];
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
@@ -136,15 +195,24 @@ __global__ void obs_to_blocked_kernel(const float* __restrict__ obs, uint16_t* _
 // MMAs once its own and the peer's stage have landed (the peer relays its full-barrier to the leader), and its
 // tcgen05.commit releases stages and publishes accumulators in both CTAs; both CTAs' epilogue warps report the drained
 // accumulator to the leader.
-template <int NT, bool kFp16, int kCS, bool kPair = false>
+//
+// kSplit (GO2P_PREC_FP32_TC, single CTA, bf16): a and w are split tile groups (wd_split_act / wd_split_weight).  A stage
+// holds the three A pieces and the three B pieces of one K chunk, and per K16 step the MMA warp issues the six products
+// whose size is at least 2^-16 of the leading term from that one stage: hi*hi into the main accumulator, hi*mid,
+// mid*hi, hi*lo, lo*hi, mid*mid into a second one (the dropped mid*lo, lo*mid, lo*lo are <= 2^-23 relative).  The
+// epilogue adds the two accumulators, then the bias in fp32; a hidden layer stores the three pieces of its output.
+template <int NT, bool kFp16, int kCS, bool kPair = false, bool kSplit = false>
 __global__ void __launch_bounds__(kWdThreads, 1) wide_gemm_kernel(const WideGemmArgs a) {
   static_assert(!kPair || kCS == 2, "a CTA pair is a cluster of two");
+  static_assert(!kSplit || (kCS == 1 && !kFp16 && NT <= 128), "the split operands are bf16, one CTA per tile, N tile <= 128");
   extern __shared__ __align__(128) uint8_t smem[];
   constexpr int kBTileBytes = NT * kWdChunkK * 2;
-  constexpr int kStageBytes = kWdATileBytes + (kPair ? kBTileBytes / 2 : kBTileBytes);   // pair: half of the weight tile per CTA
-  constexpr int kStages = wd_stages(NT, kPair);
-  constexpr uint32_t kAccCols = NT < 32 ? 32 : NT;               // TMEM columns per accumulator buffer
-  constexpr uint32_t kTmemCols = 2 * kAccCols;                   // 64 .. 512, a power of two
+  constexpr int kStageBytes = kSplit ? 3 * (kWdATileBytes + kBTileBytes)
+                                     : kWdATileBytes + (kPair ? kBTileBytes / 2 : kBTileBytes);   // pair: half of the weight tile per CTA
+  constexpr int kStages = wd_stages(NT, kPair, kSplit);
+  constexpr uint32_t kAccCols = NT < 32 ? 32 : NT;               // TMEM columns per accumulator
+  constexpr uint32_t kAccs = kSplit ? 2 : 1;                     // accumulators per buffer
+  constexpr uint32_t kTmemCols = 2 * kAccs * kAccCols;           // 64 .. 512, a power of two
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kStages * kStageBytes);
   uint64_t* full = bars;                 // [kStages] chunk landed
@@ -201,6 +269,21 @@ __global__ void __launch_bounds__(kWdThreads, 1) wide_gemm_kernel(const WideGemm
       for (int kc = 0; kc < a.k_chunks; ++kc, ++it) {
         const int s = it % kStages;
         ptx::mbar_wait(&empty[s], ((it / kStages) & 1u) ^ 1u);
+        if constexpr (kSplit) {
+          if (ptx::elect_one_sync()) {
+            uint8_t* st = smem + s * kStageBytes;
+            ptx::mbar_arrive_expect_tx(&full[s], (uint32_t)kStageBytes);
+            const uint8_t* asrc = reinterpret_cast<const uint8_t*>(a.a) + (mt * a.k_chunks + kc) * 3 * (long long)kWdATileBytes;
+            const uint8_t* wsrc = reinterpret_cast<const uint8_t*>(a.w) + ((long long)nt * a.k_chunks + kc) * 3 * (long long)kBTileBytes;
+#pragma unroll
+            for (int q = 0; q < 3; ++q) ptx::bulk_g2s(st + q * kWdATileBytes, asrc + q * kWdATileBytes, kWdATileBytes, &full[s]);
+#pragma unroll
+            for (int q = 0; q < 3; ++q)
+              ptx::bulk_g2s(st + 3 * kWdATileBytes + q * kBTileBytes, wsrc + q * kBTileBytes, kBTileBytes, &full[s]);
+          }
+          __syncwarp();
+          continue;
+        }
         if (ptx::elect_one_sync()) {
           uint8_t* st = smem + s * kStageBytes;
           ptx::mbar_arrive_expect_tx(&full[s], (uint32_t)(kPair ? kWdATileBytes + kBTileBytes / 2 : kStageBytes));
@@ -236,12 +319,38 @@ __global__ void __launch_bounds__(kWdThreads, 1) wide_gemm_kernel(const WideGemm
         const uint32_t buf = tile_i & 1u;
         ptx::mbar_wait(&acc_empty[buf], ((tile_i >> 1) & 1u) ^ 1u);
         ptx::tc_fence_after();
-        const uint32_t d_t = tmem_base + buf * kAccCols;
+        const uint32_t d_t = tmem_base + buf * kAccs * kAccCols;
         for (int kc = 0; kc < a.k_chunks; ++kc, ++it) {
           const int s = it % kStages;
           ptx::mbar_wait(&full[s], (it / kStages) & 1u);
           if (kPair) ptx::mbar_wait(&peer_full[s], (it / kStages) & 1u);
           ptx::tc_fence_after();
+          if constexpr (kSplit) {
+            if (ptx::elect_one_sync()) {
+              const uint32_t sa = ptx::smem_u32(smem + s * kStageBytes);
+              uint64_t ad[3], bd[3];
+#pragma unroll
+              for (int q = 0; q < 3; ++q) {
+                ad[q] = ptx::make_smem_desc_nosw(sa + q * kWdATileBytes, 128u, 1024u);
+                bd[q] = ptx::make_smem_desc_nosw(sa + 3 * kWdATileBytes + q * kBTileBytes, 128u, 1024u);
+              }
+#pragma unroll
+              for (int j = 0; j < kWdChunkK / 16; ++j) {
+                const uint64_t o = (uint64_t)(j * 16);
+                const uint32_t acc = (kc | j) ? 1u : 0u;
+                ptx::mma_f16_ss(d_t, ad[0] + o, bd[0] + o, idesc, acc);                 // hi * hi
+                ptx::mma_f16_ss(d_t + kAccCols, ad[0] + o, bd[1] + o, idesc, acc);      // hi * mid
+                ptx::mma_f16_ss(d_t + kAccCols, ad[1] + o, bd[0] + o, idesc, 1u);       // mid * hi
+                ptx::mma_f16_ss(d_t + kAccCols, ad[0] + o, bd[2] + o, idesc, 1u);       // hi * lo
+                ptx::mma_f16_ss(d_t + kAccCols, ad[2] + o, bd[0] + o, idesc, 1u);       // lo * hi
+                ptx::mma_f16_ss(d_t + kAccCols, ad[1] + o, bd[1] + o, idesc, 1u);       // mid * mid
+              }
+              ptx::mma_commit(&empty[s]);
+              if (kc == a.k_chunks - 1) ptx::mma_commit(&acc_full[buf]);
+            }
+            __syncwarp();
+            continue;
+          }
           if (ptx::elect_one_sync()) {
             const uint32_t sa = ptx::smem_u32(smem + s * kStageBytes);
             const uint64_t adesc = ptx::make_smem_desc_nosw(sa, 128u, 1024u);
@@ -275,10 +384,63 @@ __global__ void __launch_bounds__(kWdThreads, 1) wide_gemm_kernel(const WideGemm
       const uint32_t buf = tile_i & 1u;
       ptx::mbar_wait(&acc_full[buf], (tile_i >> 1) & 1u);
       ptx::tc_fence_after();
-      const uint32_t acc_t = tmem_base + buf * kAccCols + lane_addr;
+      const uint32_t acc_t = tmem_base + buf * kAccs * kAccCols + lane_addr;
       const long long row = mt * kWdTileM + r;
       if (ghost) {
         // nothing to store; the accumulator is simply released
+      } else if (kSplit && a.out_blocked) {
+        if constexpr (kSplit) {   // discarded in the 16-bit instantiations, whose code stays as it was
+          // hidden layer: 16 columns at a time -> both accumulators + bias + ELU -> three bf16 pieces -> two 16-byte
+          // stores into each of the next layer's three tiles
+          const long long next_chunks = (long long)a.n_tiles * (NT / kWdChunkK);
+          constexpr int kShare = (NT / kWdEpiParts) < 16 ? 16 : (NT / kWdEpiParts);
+#pragma unroll 1
+          for (int c0 = half * kShare; c0 < (half + 1) * kShare && c0 < NT; c0 += 16) {
+            uint32_t v[16], u[16];
+            ptx::tmem_ld_x16(acc_t + (uint32_t)c0, v);
+            ptx::tmem_ld_x16(acc_t + kAccCols + (uint32_t)c0, u);
+            ptx::tc_wait_ld();
+            float x[16];
+            {
+              const float4* b4 = reinterpret_cast<const float4*>(a.bias + nt * NT + c0);
+#pragma unroll
+              for (int j4 = 0; j4 < 4; ++j4) {
+                const float4 b = __ldg(b4 + j4);
+                const float bl[4] = {b.x, b.y, b.z, b.w};
+#pragma unroll
+                for (int i = 0; i < 4; ++i)
+                  x[4 * j4 + i] = (__uint_as_float(v[4 * j4 + i]) + __uint_as_float(u[4 * j4 + i])) + bl[i];
+              }
+            }
+            // the activation test is hoisted out of the unrolled loop, as in the 16-bit epilogue below
+            if (a.has_elu) {
+              const float alpha = a.alpha, nalpha = -a.alpha;
+#pragma unroll
+              for (int i = 0; i < 16; ++i) {
+                const float e = fmaf(alpha, ptx::ex2_approx(x[i] * 1.4426950408889634f), nalpha);
+                x[i] = (x[i] < 0.f) ? e : x[i];
+              }
+            }
+            uint32_t p[3][8];
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+              float s0[3], s1[3];
+              wd_split_act(x[2 * j], s0[0], s0[1], s0[2]);
+              wd_split_act(x[2 * j + 1], s1[0], s1[1], s1[2]);
+#pragma unroll
+              for (int q = 0; q < 3; ++q) p[q][j] = ptx::pack_bf16(s0[q], s1[q]);
+            }
+            const int kn = nt * NT + c0;                 // K index of the next layer
+            uint8_t* dst = reinterpret_cast<uint8_t*>(a.out_blocked) + ((mt * next_chunks + kn / kWdChunkK) * 3 * (long long)kWdATileBytes) +
+                           wd_tile_offset(r, kn % kWdChunkK);
+#pragma unroll
+            for (int q = 0; q < 3; ++q)
+#pragma unroll
+              for (int c = 0; c < 2; ++c)                // consecutive 8-column cores are 128 B apart inside the tile
+                *reinterpret_cast<uint4*>(dst + q * kWdATileBytes + c * 128) =
+                    make_uint4(p[q][4 * c], p[q][4 * c + 1], p[q][4 * c + 2], p[q][4 * c + 3]);
+          }
+        }
       } else if (a.out_blocked) {
         // hidden layer: 32 columns at a time -> bias + ELU -> 16 bit -> four 16-byte stores into the next layer's tile
         const int kcn_per_tile = NT / kWdChunkK;       // 64-column chunks of the next layer covered by this N tile
@@ -330,6 +492,13 @@ __global__ void __launch_bounds__(kWdThreads, 1) wide_gemm_kernel(const WideGemm
         // output layer (NT == 16): bias (+ELU) (+clamp/mask) (+q_des) -> fp32 rows
         uint32_t v[16];
         ptx::tmem_ld_x16(acc_t, v);
+        if constexpr (kSplit) {
+          uint32_t u[16];
+          ptx::tmem_ld_x16(acc_t + kAccCols, u);
+          ptx::tc_wait_ld();
+#pragma unroll
+          for (int j = 0; j < 16; ++j) v[j] = __float_as_uint(__uint_as_float(v[j]) + __uint_as_float(u[j]));
+        }
         ptx::tc_wait_ld();
         if (row < a.M && half == 0) {
           const int b0 = ((a.flags & 5u) && a.button0) ? a.button0[row] : 0;
@@ -385,10 +554,25 @@ inline void wd_pack_weights(const MlpLayer& L, int NT, int Np, int Kp, bool fp16
     }
 }
 
+// the split images of W [N][K] (wd_split_weight): tile group (nt, kc) = the hi, mid and lo NT x 64 tiles
+inline void wd_pack_split(const MlpLayer& L, int NT, int Np, int Kp, std::vector<uint16_t>& out) {
+  out.assign((size_t)Np * Kp * 3, 0);
+  const int k_chunks = Kp / kWdChunkK;
+  const size_t tile_elems = (size_t)NT * kWdChunkK;
+  for (int n = 0; n < L.out; ++n)
+    for (int k = 0; k < L.in; ++k) {
+      uint16_t p[3];
+      wd_split_weight(L.weight[(size_t)n * L.in + k], p);
+      const size_t idx = ((size_t)(n / NT) * k_chunks + k / kWdChunkK) * 3 * tile_elems + wd_tile_offset(n % NT, k % kWdChunkK) / 2;
+      for (int q = 0; q < 3; ++q) out[idx + q * tile_elems] = p[q];
+    }
+}
+
 // returns 0 = ok, > 0 = go2p_status (CUDA failure), < 0 = this shape is not served by the wide path.
-// alloc(bytes) returns device memory that the caller owns, or null.
+// alloc(bytes) returns device memory that the caller owns, or null.  images16: also build the bf16 / fp16 images (the
+// split images of GO2P_PREC_FP32_TC are always built).
 template <class Alloc>
-inline int wide_prepare(const MlpModel& m, Alloc&& alloc, WideModel* wm, std::string& err) {
+inline int wide_prepare(const MlpModel& m, Alloc&& alloc, WideModel* wm, bool images16, std::string& err) {
   const int nl = (int)m.layers.size();
   if (nl < 2 || nl > kMaxLayers || m.layers.back().out > 16) return -1;
   for (int l = 0; l + 1 < nl; ++l) if (m.layers[l].out % 64 != 0) return -1;
@@ -407,15 +591,23 @@ inline int wide_prepare(const MlpModel& m, Alloc&& alloc, WideModel* wm, std::st
     D.Kp = wd_round_up(L.in, kWdChunkK);
     D.NT = last ? 16 : (L.out % 256 == 0 ? 256 : (L.out % 128 == 0 ? 128 : 64));
     D.Np = wd_round_up(L.out, D.NT);
+    // split stages hold three pieces of each operand: N tiles of at most 128 rows keep two of them (192 KB) in flight
+    D.NT3 = D.NT > 128 ? 128 : D.NT;
     D.has_elu = L.has_elu ? 1 : 0; D.alpha = L.elu_alpha;
     if (l > 0 && D.Kp != wm->L[l - 1].Np) return -1;   // a hidden width that is not a multiple of 64
     wm->max_kp = std::max(wm->max_kp, D.Kp);
     std::vector<uint16_t> img;
-    for (int f = 0; f < 2; ++f) {
+    for (int f = 0; f < 2 && images16; ++f) {
       wd_pack_weights(L, D.NT, D.Np, D.Kp, f == 1, img);
       void* p;
       if (!upload(img.data(), img.size() * 2, &p)) return 4;
       D.w[f] = static_cast<const uint16_t*>(p);
+    }
+    {
+      wd_pack_split(L, D.NT3, D.Np, D.Kp, img);
+      void* p;
+      if (!upload(img.data(), img.size() * 2, &p)) return 4;
+      D.w3 = static_cast<const uint16_t*>(p);
     }
     std::vector<float> bias(D.Np, 0.f);
     for (int n = 0; n < L.out; ++n) bias[n] = L.bias[n];
@@ -495,10 +687,39 @@ inline long long wide_act_rows(long long B) {
   return (std::min<long long>(B, kWdChunkRows) + kWdTileM - 1) / kWdTileM * kWdTileM;
 }
 
-// act: the two blocked activation buffers (ping-pong), each of wide_act_rows(B) rows x wm.max_kp 16-bit columns
+// The split GEMMs (GO2P_PREC_FP32_TC).  configured: the dynamic shared memory this handle has opted the instantiation
+// in to on its device (the attribute is per device and per function; one handle = one device).
+template <int NT>
+inline cudaError_t wd_launch_split(const WideGemmArgs& a, int sm_count, size_t& configured, cudaStream_t st) {
+  const size_t smem = (size_t)wd_stages(NT, false, true) * 3 * (kWdATileBytes + NT * kWdChunkK * 2) + 256;
+  auto kernel = wide_gemm_kernel<NT, false, 1, false, true>;
+  if (configured != smem) {
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    configured = smem;
+  }
+  cudaLaunchConfig_t cfg = {};
+  cudaLaunchAttribute attr;
+  attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;      // see griddepcontrol.wait in the kernel
+  attr.val.programmaticStreamSerializationAllowed = 1;
+  cfg.blockDim = dim3(kWdThreads);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = st;
+  cfg.attrs = &attr; cfg.numAttrs = 1;
+  const long long jobs = (long long)a.m_tiles * a.n_tiles;
+  cfg.gridDim = dim3((unsigned)std::min<long long>(jobs, (long long)sm_count));
+  return cudaLaunchKernelEx(&cfg, kernel, a);
+}
+
+// operand formats of wide_launch
+enum WdOperands { kWdBf16 = 0, kWdFp16 = 1, kWdSplit = 2 };
+
+// act: the two blocked activation buffers (ping-pong), each of wide_act_rows(B) rows x wm.max_kp 16-bit columns (three
+// times that for kWdSplit).  split_attr: the handle's opt-in record of the split instantiations (N tile 128, 64, 16).
 inline int wide_launch(const WideModel& wm, uint16_t* const act[2], const float* d_obs, const int32_t* d_button0, float* d_act, double* d_qdes,
-                       MotorCmdDev* d_cmd, long long B, bool fp16, uint32_t flags, const CtrlConst& cc, int sm_count, cudaStream_t st,
-                       int* launches, std::string& err) {
+                       MotorCmdDev* d_cmd, long long B, WdOperands operands, uint32_t flags, const CtrlConst& cc, int sm_count,
+                       size_t split_attr[3], cudaStream_t st, int* launches, std::string& err) {
+  const bool fp16 = operands == kWdFp16, split = operands == kWdSplit;
   const long long chunk = std::min<long long>(B, kWdChunkRows);
   for (long long r0 = 0; r0 < B; r0 += chunk) {
     const long long rows = std::min(chunk, B - r0);
@@ -514,8 +735,9 @@ inline int wide_launch(const WideModel& wm, uint16_t* const act[2], const float*
       lc.gridDim = dim3((unsigned)blocks); lc.blockDim = dim3(256); lc.stream = st; lc.attrs = &la; lc.numAttrs = 1;
       const float* src = d_obs + r0 * wm.in_dim;
       const long long m_tiles_ll = m_tiles;
-      cudaError_t ec = fp16 ? cudaLaunchKernelEx(&lc, obs_to_blocked_kernel<true>, src, act[0], rows, wm.in_dim, L0.Kp, m_tiles_ll)
-                            : cudaLaunchKernelEx(&lc, obs_to_blocked_kernel<false>, src, act[0], rows, wm.in_dim, L0.Kp, m_tiles_ll);
+      cudaError_t ec = split ? cudaLaunchKernelEx(&lc, obs_to_blocked_kernel<false, true>, src, act[0], rows, wm.in_dim, L0.Kp, m_tiles_ll)
+                     : fp16  ? cudaLaunchKernelEx(&lc, obs_to_blocked_kernel<true>, src, act[0], rows, wm.in_dim, L0.Kp, m_tiles_ll)
+                             : cudaLaunchKernelEx(&lc, obs_to_blocked_kernel<false>, src, act[0], rows, wm.in_dim, L0.Kp, m_tiles_ll);
       if (ec != cudaSuccess) { err = std::string("wide_launch: ") + cudaGetErrorString(ec); return 4; }
       ++*launches;
     }
@@ -524,19 +746,24 @@ inline int wide_launch(const WideModel& wm, uint16_t* const act[2], const float*
       const WideLayerDev& L = wm.L[l];
       const bool last = l == wm.n_layers - 1;
       WideGemmArgs a{};
-      a.a = act[cur]; a.w = L.w[fp16 ? 1 : 0]; a.bias = L.bias;
+      const int NT = split ? L.NT3 : L.NT;
+      a.a = act[cur]; a.w = split ? L.w3 : L.w[fp16 ? 1 : 0]; a.bias = L.bias;
       a.out_blocked = last ? nullptr : act[cur ^ 1];
       a.out_rows = last ? d_act + r0 * wm.out_dim : nullptr;
       a.button0 = d_button0 ? d_button0 + r0 : nullptr;
       a.qdes = d_qdes ? d_qdes + r0 * kDof : nullptr;
       a.cmd = d_cmd ? d_cmd + r0 : nullptr;
       a.kp = cc.kp; a.kd = cc.kd; a.kp_deadman = cc.kp_deadman;
-      a.M = rows; a.m_tiles = m_tiles; a.n_tiles = L.Np / L.NT; a.k_chunks = L.Kp / kWdChunkK;
+      a.M = rows; a.m_tiles = m_tiles; a.n_tiles = L.Np / NT; a.k_chunks = L.Kp / kWdChunkK;
       a.N = L.N; a.out_dim = wm.out_dim; a.has_elu = L.has_elu; a.alpha = L.alpha;
       a.flags = last ? flags : 0u; a.action_limit = cc.action_limit; a.action_scale = cc.action_scale;
       for (int i = 0; i < kDof; ++i) a.q0[i] = cc.q0[i];
       cudaError_t e;
-      if (L.NT == 256) e = fp16 ? wd_launch_gemm<256, true>(a, sm_count, st) : wd_launch_gemm<256, false>(a, sm_count, st);
+      if (split) {
+        if (NT == 128) e = wd_launch_split<128>(a, sm_count, split_attr[0], st);
+        else if (NT == 64) e = wd_launch_split<64>(a, sm_count, split_attr[1], st);
+        else e = wd_launch_split<16>(a, sm_count, split_attr[2], st);
+      } else if (L.NT == 256) e = fp16 ? wd_launch_gemm<256, true>(a, sm_count, st) : wd_launch_gemm<256, false>(a, sm_count, st);
       else if (L.NT == 128) e = fp16 ? wd_launch_gemm<128, true>(a, sm_count, st) : wd_launch_gemm<128, false>(a, sm_count, st);
       else if (L.NT == 64) e = fp16 ? wd_launch_gemm<64, true>(a, sm_count, st) : wd_launch_gemm<64, false>(a, sm_count, st);
       else e = fp16 ? wd_launch_gemm<16, true>(a, sm_count, st) : wd_launch_gemm<16, false>(a, sm_count, st);

@@ -52,9 +52,17 @@ typedef enum go2p_status {
 typedef enum go2p_precision {
   GO2P_PREC_FP32 = 0,        /* CUDA-core FFMA; agrees with ORT-CPU semantics to 1e-5 */
   GO2P_PREC_BF16 = 1,        /* tcgen05 kind::f16, bf16 operands                        */
-  GO2P_PREC_FP16 = 2         /* tcgen05 kind::f16, fp16 operands (saturating convert)   */
+  GO2P_PREC_FP16 = 2,        /* tcgen05 kind::f16, fp16 operands (saturating convert)   */
   /* 3 was reserved for kind::tf32 and is rejected: fp32 weights of the policy do not fit in shared memory beside the
    * observation ring, and fp16 operands have the same 11-bit significand (see DESIGN.md, precision contract) */
+  GO2P_PREC_FP32_TC = 4      /* fp32 accuracy on the tensor cores: every operand split into three bf16 pieces (24
+                              * significand bits, fp32 range), six tcgen05 kind::f16 products per K step, fp32
+                              * accumulation, bias and ELU.  Same contract as GO2P_PREC_FP32 against an fp64
+                              * reference (|a - ref| <= 1e-5 * max(|ref|, 1), row rel-L2 <= 1e-5), no saturation,
+                              * the reference's NaN pattern for +-Inf / NaN inputs, results independent of batch
+                              * size and entry point; not bit-identical to GO2P_PREC_FP32 (other summation order).
+                              * Serves 2-8 layers, hidden widths that are multiples of 64, at most 16 outputs;
+                              * other shapes: GO2P_ERR_UNSUPPORTED.  GO2P_F_SAT_COUNT counts nothing. */
 } go2p_precision;
 
 /* how the batch-1 control-loop step reaches the GPU */
