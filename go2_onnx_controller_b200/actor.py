@@ -141,30 +141,43 @@ RAW_FIELDS = (("quat", 4), ("gyro", 3), ("q", 12), ("dq", 12), ("axes", 4), ("fo
 _FLAG_DTYPES = ("torch.bool", "torch.uint8")
 
 
-def step_field_tensors(in_dim: int, device: int, fields: dict, vel_cmd, obs, action, qdes=None, cmd=None, reset=None) -> int:
+def step_field_tensors(in_dim: int, device: int, fields: dict, vel_cmd, obs, action, qdes=None, cmd=None, reset=None,
+                       action_seq=None, obs_seq=None, seq: bool = False):
     """Validates the arguments of PolicyBatch.step_fields before any native call.  fields: the eight raw-state tensors by
     name (RAW_FIELDS): float32 [B,w], foot_force int16 [B,4], joy_valid / button0 bool or uint8 [B].  vel_cmd float32
     [B,3], obs float32 [B,in_dim], action float32 [B,12], qdes float64 [B,12] or None, cmd uint8 [B,112] or None (not
     both None), reset bool / uint8 [B] or None.  Every tensor is a contiguous CUDA tensor on device ``device`` (duck-typed:
-    this package does not import torch).  Returns B; raises TypeError / ValueError."""
-    if qdes is None and cmd is None:
+    this package does not import torch).  Returns B; raises TypeError / ValueError.
+    seq=True validates PolicyBatch.step_fields_seq instead: the fields, reset, qdes and cmd carry a leading step dimension
+    T ([T,B,w]), action_seq float32 [T,B,12] is required, obs_seq float32 [T,B,in_dim] or None, qdes and cmd may both be
+    None; vel_cmd, obs and action keep their [B,w] shapes.  Returns (T, B)."""
+    if seq:
+        if action_seq is None:
+            raise ValueError("action_seq is required: it receives every step's published action")
+    elif qdes is None and cmd is None:
         raise ValueError("qdes and cmd are both None: the step needs at least one output")
     quat = fields["quat"]
     if not _is_device_tensor(quat):
         raise TypeError(f"quat must be a CUDA tensor, got {type(quat).__name__}")
-    if len(quat.shape) != 2:
-        raise ValueError(f"quat must have shape (B, 4), got {tuple(quat.shape)}")
-    B = int(quat.shape[0])
-    named = [(name, fields[name], (B, w) if w else (B,), "torch.int16" if name == "foot_force" else
+    if len(quat.shape) != (3 if seq else 2):
+        raise ValueError(f"quat must have shape ({'T, ' if seq else ''}B, 4), got {tuple(quat.shape)}")
+    T = int(quat.shape[0]) if seq else None
+    B = int(quat.shape[-2])
+    lead = (T,) if seq else ()                 # the per-step tensors' leading dimension
+    named = [(name, fields[name], lead + ((B, w) if w else (B,)), "torch.int16" if name == "foot_force" else
               _FLAG_DTYPES if w is None else "torch.float32") for name, w in RAW_FIELDS]
     named += [("vel_cmd", vel_cmd, (B, 3), "torch.float32"), ("obs", obs, (B, in_dim), "torch.float32"),
               ("action", action, (B, 12), "torch.float32")]
+    if seq:
+        named.append(("action_seq", action_seq, (T, B, 12), "torch.float32"))
+        if obs_seq is not None:
+            named.append(("obs_seq", obs_seq, (T, B, in_dim), "torch.float32"))
     if qdes is not None:
-        named.append(("qdes", qdes, (B, 12), "torch.float64"))
+        named.append(("qdes", qdes, lead + (B, 12), "torch.float64"))
     if cmd is not None:
-        named.append(("cmd", cmd, (B, C.sizeof(capi.MotorCmd)), "torch.uint8"))
+        named.append(("cmd", cmd, lead + (B, C.sizeof(capi.MotorCmd)), "torch.uint8"))
     if reset is not None:
-        named.append(("reset", reset, (B,), _FLAG_DTYPES))
+        named.append(("reset", reset, lead + (B,), _FLAG_DTYPES))
     for name, a, shape, dtypes in named:
         if not _is_device_tensor(a):
             raise TypeError(f"{name} must be a CUDA tensor, got {type(a).__name__}")
@@ -178,7 +191,7 @@ def step_field_tensors(in_dim: int, device: int, fields: dict, vel_cmd, obs, act
             raise ValueError(f"{name} must have shape {shape}, got {tuple(a.shape)}")
         if not a.is_contiguous():
             raise ValueError(f"{name} must be contiguous")
-    return B
+    return (T, B) if seq else B
 
 
 def _ptr(a):
@@ -400,6 +413,26 @@ class PolicyBatch:
         capi.check(self._hd.lib.go2p_step_batch_fields(self._hd.h, C.byref(f), _ptr(reset), vel_cmd.data_ptr(),
                                                        obs.data_ptr(), action.data_ptr(), _ptr(qdes), _ptr(cmd), B,
                                                        precision, stream or None))
+
+    def step_fields_seq(self, quat, gyro, q, dq, axes, foot_force, joy_valid, button0, vel_cmd, obs, action, action_seq,
+                        qdes_seq=None, cmd_seq=None, obs_seq=None, reset=None, precision: int = capi.PREC_FP32,
+                        stream: int = 0) -> None:
+        """T consecutive step_fields steps in one call (go2p_step_batch_fields_seq), e.g. to replay recorded sensor
+        streams closed-loop: every field and reset as in step_fields with a leading step dimension, [T,B,w].  vel_cmd,
+        obs and action are the robots' state before step 0 on entry and after step T-1 on return.  action_seq float32
+        [T,B,12] receives every step's published action; qdes_seq float64 [T,B,12], cmd_seq uint8 [T,B,112] and obs_seq
+        float32 [T,B,in_dim] (every step's observation) are optional.  T or B = 0 does nothing."""
+        fields = dict(quat=quat, gyro=gyro, q=q, dq=dq, axes=axes, foot_force=foot_force, joy_valid=joy_valid,
+                      button0=button0)
+        T, B = step_field_tensors(self.in_dim, self._hd.cfg.device, fields, vel_cmd, obs, action, qdes_seq, cmd_seq, reset,
+                                  action_seq=action_seq, obs_seq=obs_seq, seq=True)
+        if T == 0 or B == 0:
+            return
+        f = capi.RawFields(*[fields[name].data_ptr() for name, _ in RAW_FIELDS])
+        capi.check(self._hd.lib.go2p_step_batch_fields_seq(self._hd.h, C.byref(f), T, _ptr(reset), vel_cmd.data_ptr(),
+                                                           obs.data_ptr(), action.data_ptr(), action_seq.data_ptr(),
+                                                           _ptr(qdes_seq), _ptr(cmd_seq), _ptr(obs_seq), B, precision,
+                                                           stream or None))
 
     def step_host(self, raw: np.ndarray, action: np.ndarray, cmd: np.ndarray | None = None,
                   precision: int = capi.PREC_FP32, reset: np.ndarray | None = None) -> None:

@@ -108,6 +108,9 @@ SIGNATURES = {
                                       C.c_int64, C.c_int, C.c_void_p]),
     "go2p_step_batch_fields": (C.c_int, [_H, C.POINTER(RawFields), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
+    "go2p_step_batch_fields_seq": (C.c_int, [_H, C.POINTER(RawFields), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
+                                              C.c_int, C.c_void_p]),
     "go2p_step_fused_cmd": (C.c_int, [_H, C.POINTER(RawState), C.POINTER(StepOut), C.POINTER(MotorCmd)]),
     "go2p_motor_order": (C.c_int, [C.POINTER(C.c_int32)]),
     "go2p_step_batch_host": (C.c_int, [_H, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int]),

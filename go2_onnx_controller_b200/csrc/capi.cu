@@ -14,6 +14,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <stdexcept>
 #include <thread>
 #include <string>
@@ -79,8 +80,8 @@ struct go2p_handle {
   size_t tc_off[kMaxLayers] = {};              // layer l's image starts tc_off[l] elements into d_wpack[0] / [1]
   int tc_kp[kMaxLayers] = {};
   double tc_wscale[kMaxLayers] = {}, tc_bscale[kMaxLayers] = {};   // the scales pack_umma_kmajor applied
-  size_t tc_attr_smem[10] = {};                // dynamic shared memory opted in for tc_mlp_kernel<bf16|fp16, plain|fused|fused+reset,
-                                               // records|fields> on this device
+  size_t tc_attr_smem[14] = {};                // dynamic shared memory opted in for tc_mlp_kernel<bf16|fp16, plain|fused|fused+reset,
+                                               // records|fields|field sequence> on this device
   bool b1_attr_set = false;                    // same for the one-shot batch-1 kernel
   size_t so_attr_smem = 0;                     // same for small_out_kernel
   size_t split_attr_smem[3] = {};              // same for wide_gemm_kernel<128 | 64 | 16, split>
@@ -502,12 +503,12 @@ int launch_fp32(go2p_handle* h, int set, const float* d_obs, const int32_t* d_bu
   return GO2P_OK;
 }
 
-template <bool kFp16, bool kFused, bool kReset = false, bool kFields = false>
+template <bool kFp16, bool kFused, bool kReset = false, bool kFields = false, bool kSeq = false>
 int launch_tc_t(go2p_handle* h, const TcArgs& a, cudaStream_t st) {
   const size_t smem = tc_smem_bytes(a);
-  auto kernel = tc_mlp_kernel<kFp16, kFused, kReset, kFields>;
+  auto kernel = tc_mlp_kernel<kFp16, kFused, kReset, kFields, kSeq>;
   // the opt-in is a per-device function attribute: remembered per handle (one handle = one device)
-  size_t& configured = h->tc_attr_smem[(kFp16 ? 1 : 0) + (kFused ? 2 : 0) + (kReset ? 2 : 0) + (kFields ? 4 : 0)];
+  size_t& configured = h->tc_attr_smem[(kFp16 ? 1 : 0) + (kFused ? 2 : 0) + (kReset ? 2 : 0) + (kFields ? 4 : 0) + (kSeq ? 4 : 0)];
   if (configured != smem) {
     CU_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     configured = smem;
@@ -533,12 +534,22 @@ int launch_tc_t(go2p_handle* h, const TcArgs& a, cudaStream_t st) {
   return GO2P_OK;
 }
 
+// the per-step outputs of tc_mlp_kernel<., true, ., true, true>: T steps, [T,B,.] each (TcArgs)
+struct TcSeqOut {
+  int T;
+  float* act;
+  double* qdes;
+  MotorCmdDev* cmd;
+  float* obs;
+};
+
 // raw or fields != null: the fused controller step (A1-A6 in the conversion job) from records or per-field arrays: d_obs
-// is the robots' history, updated in place; d_reset (may be null) the robots' reset flags
+// is the robots' history, updated in place; d_reset (may be null) the robots' reset flags.  seq != null (with fields):
+// seq->T steps in one launch, the fields and d_reset holding T*B rows; d_qdes and d_cmd are unused then
 int launch_tc(go2p_handle* h, const float* d_obs, const int32_t* d_button0, float* d_act, double* d_qdes,
               MotorCmdDev* d_cmd, int64_t B, bool fp16, uint32_t flags, cudaStream_t st,
               const RawStateDev* raw = nullptr, float* d_vel_cmd = nullptr, const uint8_t* d_reset = nullptr,
-              const RawFieldsDev* fields = nullptr) {
+              const RawFieldsDev* fields = nullptr, const TcSeqOut* seq = nullptr) {
   if ((reinterpret_cast<uintptr_t>(d_obs) & 15) || (reinterpret_cast<uintptr_t>(d_act) & 15) ||
       (d_qdes && (reinterpret_cast<uintptr_t>(d_qdes) & 15)))
     return fail(GO2P_ERR_INVALID, "tensor-core path needs 16-byte aligned obs/act/qdes device pointers");
@@ -570,6 +581,12 @@ int launch_tc(go2p_handle* h, const float* d_obs, const int32_t* d_button0, floa
 #endif
   a.raw = raw; a.obs_rw = const_cast<float*>(d_obs); a.vel_cmd = d_vel_cmd; a.H = h->cc.H; a.foot_threshold = h->cc.foot_threshold;
   a.reset = raw || fields ? d_reset : nullptr;
+  if (fields && seq) {
+    a.fields = *fields;
+    a.T = seq->T; a.act_seq = seq->act; a.qdes_seq = seq->qdes; a.cmd_seq = seq->cmd; a.obs_seq = seq->obs;
+    if (d_reset) return fp16 ? launch_tc_t<true, true, true, true, true>(h, a, st) : launch_tc_t<false, true, true, true, true>(h, a, st);
+    return fp16 ? launch_tc_t<true, true, false, true, true>(h, a, st) : launch_tc_t<false, true, false, true, true>(h, a, st);
+  }
   if (fields) {
     a.fields = *fields;
     if (d_reset) return fp16 ? launch_tc_t<true, true, true, true>(h, a, st) : launch_tc_t<false, true, true, true>(h, a, st);
@@ -1124,15 +1141,9 @@ int go2p_assemble_batch(go2p_handle* h, const go2p_raw_state* d_raw, const float
 namespace {
 bool aligned16(const void* p) { return !(reinterpret_cast<uintptr_t>(p) & 15); }
 
-// publish() for B robots on device buffers; button_scratch [B] receives the dead-man buttons for the epilogue.
-// The raw states are records (d_raw) or per-field arrays (fields); exactly one of the two is non-null.
-// d_reset [B] (may be null): robots to start from the initial state, applied by whichever kernel assembles the
-// observations (the fused kernel's conversion job or assemble_batch_kernel); the path choice does not depend on it.
-// `set`: the stream set whose activation scratch the policy uses.
-int step_batch_on(go2p_handle* h, int set, const go2p_raw_state* d_raw, const RawFieldsDev* fields, const uint8_t* d_reset,
-                  float* d_vel_cmd, float* d_obs, float* d_action, double* d_qdes, go2p_motor_cmd* d_cmd,
-                  int32_t* button_scratch, int64_t B, int precision, cudaStream_t st) {
-  const uint32_t all_flags = GO2P_F_CLAMP_MASK | (d_qdes ? GO2P_F_QDES : 0u) | (d_cmd ? GO2P_F_MOTOR_CMD : 0u);
+// whether the fused tensor-core kernel serves this step (the one-launch path)
+bool fused_step_ok(const go2p_handle* h, const go2p_raw_state* d_raw, const RawFieldsDev* fields, const float* d_obs,
+                   const float* d_action, const double* d_qdes, const go2p_motor_cmd* d_cmd, int precision) {
   TcArgs probe{};
   probe.n_layers = h->dm.n_layers; probe.in_dim = h->dm.in_dim; probe.k0p = h->k0p;
   probe.raw = reinterpret_cast<const RawStateDev*>(d_raw);          // the fused kernel also stages the raw states
@@ -1142,10 +1153,22 @@ int step_batch_on(go2p_handle* h, int set, const go2p_raw_state* d_raw, const Ra
                                         aligned16(fields->dq) && aligned16(fields->axes) && aligned16(fields->foot_force) &&
                                         aligned16(fields->joy_valid) && aligned16(fields->button0)
                                   : aligned16(d_raw);
-  if (h->tc_ok && (precision == GO2P_PREC_FP16 || precision == GO2P_PREC_BF16) && (h->dm.in_dim & 1) == 0 &&
-      tc_smem_bytes(probe) <= (size_t)227 * 1024 && raw_aligned &&
-      !(reinterpret_cast<uintptr_t>(d_obs) & 15) && !(reinterpret_cast<uintptr_t>(d_action) & 15) &&
-      !(d_qdes && (reinterpret_cast<uintptr_t>(d_qdes) & 15)) && !(d_cmd && (reinterpret_cast<uintptr_t>(d_cmd) & 15))) {
+  return h->tc_ok && (precision == GO2P_PREC_FP16 || precision == GO2P_PREC_BF16) && (h->dm.in_dim & 1) == 0 &&
+         tc_smem_bytes(probe) <= (size_t)227 * 1024 && raw_aligned &&
+         !(reinterpret_cast<uintptr_t>(d_obs) & 15) && !(reinterpret_cast<uintptr_t>(d_action) & 15) &&
+         !(d_qdes && (reinterpret_cast<uintptr_t>(d_qdes) & 15)) && !(d_cmd && (reinterpret_cast<uintptr_t>(d_cmd) & 15));
+}
+
+// publish() for B robots on device buffers; button_scratch [B] receives the dead-man buttons for the epilogue.
+// The raw states are records (d_raw) or per-field arrays (fields); exactly one of the two is non-null.
+// d_reset [B] (may be null): robots to start from the initial state, applied by whichever kernel assembles the
+// observations (the fused kernel's conversion job or assemble_batch_kernel); the path choice does not depend on it.
+// `set`: the stream set whose activation scratch the policy uses.
+int step_batch_on(go2p_handle* h, int set, const go2p_raw_state* d_raw, const RawFieldsDev* fields, const uint8_t* d_reset,
+                  float* d_vel_cmd, float* d_obs, float* d_action, double* d_qdes, go2p_motor_cmd* d_cmd,
+                  int32_t* button_scratch, int64_t B, int precision, cudaStream_t st) {
+  const uint32_t all_flags = GO2P_F_CLAMP_MASK | (d_qdes ? GO2P_F_QDES : 0u) | (d_cmd ? GO2P_F_MOTOR_CMD : 0u);
+  if (fused_step_ok(h, d_raw, fields, d_obs, d_action, d_qdes, d_cmd, precision)) {
     // ONE launch: A1-A6 run inside the policy kernel's conversion job, the newest frame never round-trips HBM
     h->last_launches = 0;
     return launch_tc(h, d_obs, nullptr, d_action, d_qdes, reinterpret_cast<MotorCmdDev*>(d_cmd), B, precision == GO2P_PREC_FP16,
@@ -1162,20 +1185,26 @@ int step_batch_on(go2p_handle* h, int set, const go2p_raw_state* d_raw, const Ra
   return rc;
 }
 
-// the device-buffer step after its pointer checks: batch and policy checks, the button scratch, stream set 0
-int step_batch_device(go2p_handle* h, const char* fn, const go2p_raw_state* d_raw, const RawFieldsDev* fields,
-                      const uint8_t* d_reset, float* d_vel_cmd, float* d_obs, float* d_action, double* d_qdes,
-                      go2p_motor_cmd* d_cmd, int64_t B, int precision, void* stream) {
-  if (B <= 0) return B == 0 ? GO2P_OK : fail(GO2P_ERR_INVALID, "negative batch");
+// the device-buffer step's policy check and its button scratch of B rows, under the handle's device
+int step_setup(go2p_handle* h, const char* fn, int64_t B) {
   if (h->dm.in_dim != kFrame * h->cc.H || h->dm.out_dim != kDof)
     return fail(GO2P_ERR_INVALID, std::string(fn) + ": the policy is not a 49*H -> 12 controller policy");
-  DeviceGuard g(h->device);
   if (h->step_button_rows < B) {
     h->d_step_button = nullptr;   // retire (owned_alloc)
     h->step_button_rows = 0;
     if (const int rc = owned_alloc(h, h->d_step_button, (size_t)B * sizeof(int32_t))) return rc;
     h->step_button_rows = B;
   }
+  return GO2P_OK;
+}
+
+// the device-buffer step after its pointer checks: batch and policy checks, the button scratch, stream set 0
+int step_batch_device(go2p_handle* h, const char* fn, const go2p_raw_state* d_raw, const RawFieldsDev* fields,
+                      const uint8_t* d_reset, float* d_vel_cmd, float* d_obs, float* d_action, double* d_qdes,
+                      go2p_motor_cmd* d_cmd, int64_t B, int precision, void* stream) {
+  if (B <= 0) return B == 0 ? GO2P_OK : fail(GO2P_ERR_INVALID, "negative batch");
+  DeviceGuard g(h->device);
+  if (const int rc = step_setup(h, fn, B)) return rc;
   return step_batch_on(h, 0, d_raw, fields, d_reset, d_vel_cmd, d_obs, d_action, d_qdes, d_cmd, h->d_step_button, B,
                        precision, static_cast<cudaStream_t>(stream));
 }
@@ -1189,25 +1218,92 @@ int go2p_step_batch_ex(go2p_handle* h, const go2p_raw_state* d_raw, const uint8_
                            precision, stream);
 }
 
-int go2p_step_batch_fields(go2p_handle* h, const go2p_raw_fields* f, const uint8_t* d_reset, float* d_vel_cmd,
-                           float* d_obs, float* d_action, double* d_qdes, go2p_motor_cmd* d_cmd, int64_t B,
-                           int precision, void* stream) {
-  const char* fn = "go2p_step_batch_fields";
+namespace {
+// the pointer checks of the per-field steps: handle, f and its fields, the state and output pointers in `more` (named
+// in the message), then `no_output` (the single step's d_qdes and d_cmd both null), then the fields' alignment
+int check_fields_step(const char* fn, const go2p_handle* h, const go2p_raw_fields* f,
+                      std::initializer_list<std::pair<const void*, const char*>> more, bool no_output) {
   if (!h) return fail(GO2P_ERR_INVALID, std::string(fn) + ": null handle");
   if (!f) return fail(GO2P_ERR_INVALID, std::string(fn) + ": null go2p_raw_fields");
   const std::pair<const void*, const char*> ptrs[] = {
       {f->quat, "quat"}, {f->gyro, "gyro"}, {f->q, "q"}, {f->dq, "dq"}, {f->axes, "axes"}, {f->foot_force, "foot_force"},
-      {f->joy_valid, "joy_valid"}, {f->button0, "button0"}, {d_vel_cmd, "d_vel_cmd"}, {d_obs, "d_obs"},
-      {d_action, "d_action"}};
+      {f->joy_valid, "joy_valid"}, {f->button0, "button0"}};
   for (const auto& p : ptrs)
     if (!p.first) return fail(GO2P_ERR_INVALID, std::string(fn) + ": null " + p.second);
-  if (!d_qdes && !d_cmd) return fail(GO2P_ERR_INVALID, std::string(fn) + ": d_qdes and d_cmd are both null");
+  for (const auto& p : more)
+    if (!p.first) return fail(GO2P_ERR_INVALID, std::string(fn) + ": null " + p.second);
+  if (no_output) return fail(GO2P_ERR_INVALID, std::string(fn) + ": d_qdes and d_cmd are both null");
   // the two-kernel chain reads the fields at any alignment of their element type
   const auto addr = [](const void* p) { return reinterpret_cast<uintptr_t>(p); };
   if (((addr(f->quat) | addr(f->gyro) | addr(f->q) | addr(f->dq) | addr(f->axes)) & 3) || (addr(f->foot_force) & 1))
     return fail(GO2P_ERR_INVALID, std::string(fn) + ": a field is not aligned to its element size");
+  return GO2P_OK;
+}
+}  // namespace
+
+int go2p_step_batch_fields(go2p_handle* h, const go2p_raw_fields* f, const uint8_t* d_reset, float* d_vel_cmd,
+                           float* d_obs, float* d_action, double* d_qdes, go2p_motor_cmd* d_cmd, int64_t B,
+                           int precision, void* stream) {
+  const char* fn = "go2p_step_batch_fields";
+  if (const int rc = check_fields_step(fn, h, f, {{d_vel_cmd, "d_vel_cmd"}, {d_obs, "d_obs"}, {d_action, "d_action"}},
+                                       !d_qdes && !d_cmd))
+    return rc;
   const RawFieldsDev fd{f->quat, f->gyro, f->q, f->dq, f->axes, f->foot_force, f->joy_valid, f->button0};
   return step_batch_device(h, fn, nullptr, &fd, d_reset, d_vel_cmd, d_obs, d_action, d_qdes, d_cmd, B, precision, stream);
+}
+
+int go2p_step_batch_fields_seq(go2p_handle* h, const go2p_raw_fields* f, int64_t T, const uint8_t* d_reset,
+                               float* d_vel_cmd, float* d_obs, float* d_action, float* d_action_seq,
+                               double* d_qdes_seq, go2p_motor_cmd* d_cmd_seq, float* d_obs_seq,
+                               int64_t B, int precision, void* stream) {
+  const char* fn = "go2p_step_batch_fields_seq";
+  if (const int rc = check_fields_step(fn, h, f, {{d_vel_cmd, "d_vel_cmd"}, {d_obs, "d_obs"}, {d_action, "d_action"},
+                                                  {d_action_seq, "d_action_seq"}}, false))
+    return rc;
+  if (T < 0 || B < 0) return fail(GO2P_ERR_INVALID, std::string(fn) + ": negative T or B");
+  // bounded with the largest history, before anything reads the handle
+  if (T > 0 && B > 0 && B > INT64_MAX / (kFrame * kMaxHistory) / T)
+    return fail(GO2P_ERR_INVALID, std::string(fn) + ": T * B * 49 * H overflows int64");
+  if (T == 0 || B == 0) return GO2P_OK;
+  const int64_t frame = (int64_t)kFrame * h->cc.H;
+  DeviceGuard g(h->device);
+  if (const int rc = step_setup(h, fn, B)) return rc;
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const RawFieldsDev fd{f->quat, f->gyro, f->q, f->dq, f->axes, f->foot_force, f->joy_valid, f->button0};
+
+  // ONE launch where the fused kernel serves step 0 and every step's slices stay 16-byte aligned (B % 16 == 0: the
+  // one-byte fields), for the 12-output policy without a final activation; a CTA's (tile, step) units must count in int
+  const int64_t tiles = (B + kTcTileM - 1) / kTcTileM;
+  const int64_t grid = std::max<int64_t>(1, std::min<int64_t>(tiles, h->sm_count - (h->resident ? 1 : 0)));
+  const int64_t pairs = ((tiles + grid - 1) / grid + 1) / 2;
+  const auto a16 = [](const void* p) { return !(reinterpret_cast<uintptr_t>(p) & 15); };
+  if (fused_step_ok(h, nullptr, &fd, d_obs, d_action, d_qdes_seq, d_cmd_seq, precision) && (B & 15) == 0 &&
+      a16(d_action_seq) && (!d_obs_seq || a16(d_obs_seq)) && !h->dm.L[h->dm.n_layers - 1].has_elu &&
+      T <= INT32_MAX / 2 / pairs) {
+    h->last_launches = 0;
+    const TcSeqOut seq{(int)T, d_action_seq, d_qdes_seq, reinterpret_cast<MotorCmdDev*>(d_cmd_seq), d_obs_seq};
+    const uint32_t flags = GO2P_F_CLAMP_MASK | (d_qdes_seq ? GO2P_F_QDES : 0u) | (d_cmd_seq ? GO2P_F_MOTOR_CMD : 0u);
+    return launch_tc(h, d_obs, nullptr, d_action, nullptr, nullptr, B, precision == GO2P_PREC_FP16, flags, st, nullptr,
+                     d_vel_cmd, d_reset, &fd, &seq);
+  }
+  // otherwise the single step T times on the step-t slices, each taking its own path, and copies of the state into the
+  // per-step outputs; the launch count is the steps' kernels (the copies are not counted)
+  int launches = 0;
+  for (int64_t t = 0; t < T; ++t) {
+    const int64_t r = t * B;
+    const RawFieldsDev ft{fd.quat + r * 4, fd.gyro + r * 3, fd.q + r * kDof, fd.dq + r * kDof, fd.axes + r * 4,
+                          fd.foot_force + r * 4, fd.joy_valid + r, fd.button0 + r};
+    if (const int rc = step_batch_on(h, 0, nullptr, &ft, d_reset ? d_reset + r : nullptr, d_vel_cmd, d_obs, d_action,
+                                     d_qdes_seq ? d_qdes_seq + r * kDof : nullptr, d_cmd_seq ? d_cmd_seq + r : nullptr,
+                                     h->d_step_button, B, precision, st))
+      return rc;
+    launches += h->last_launches;
+    CU_TRY(cudaMemcpyAsync(d_action_seq + r * kDof, d_action, (size_t)B * kDof * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    if (d_obs_seq)
+      CU_TRY(cudaMemcpyAsync(d_obs_seq + r * frame, d_obs, (size_t)(B * frame) * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  }
+  h->last_launches = launches;
+  return GO2P_OK;
 }
 
 int go2p_step_batch_cmd(go2p_handle* h, const go2p_raw_state* d_raw, float* d_vel_cmd, float* d_obs, float* d_action,

@@ -81,7 +81,26 @@ struct TcArgs {
   const uint8_t* reset;
   // fused step from per-field arrays (tc_mlp_kernel<., true, ., true>): read instead of raw, every pointer 16-byte aligned
   RawFieldsDev fields;
+  // fused step over T steps (tc_mlp_kernel<., true, ., true, true>): fields and reset hold T*B rows, step-major; act,
+  // obs_rw and vel_cmd are the state before step 0 on entry and after step T-1 on return.  Per-step outputs [T,B,.]:
+  // act_seq (every published action), qdes_seq / cmd_seq / obs_seq (each may be null; flags 2 / 4 follow the first two)
+  float* act_seq;
+  double* qdes_seq;
+  MotorCmdDev* cmd_seq;
+  float* obs_seq;
+  int T;
 };
+
+// kSeq: CTA-local unit i = 2p + s (slot s) is step p % T of the CTA's local tile 2 (p / T) + s -- a slot keeps its tile
+// for all T steps (the host rounds a CTA's unit count up to whole pairs: an odd last tile is paired with a tile past the
+// batch, which every job treats as a ragged tile without rows).  Otherwise unit i is local tile i, step 0.
+template <bool kSeq>
+__device__ __forceinline__ long long tc_unit_row0(const TcArgs& a, int i) {
+  if constexpr (kSeq) i = 2 * ((i >> 1) / a.T) + (i & 1);
+  return (blockIdx.x + (long long)i * gridDim.x) * kTcTileM;
+}
+template <bool kSeq>
+__device__ __forceinline__ int tc_unit_step(const TcArgs& a, int i) { return kSeq ? (i >> 1) % a.T : 0; }
 
 #ifdef GO2P_TC_TRACE
 // store-only tracer: every tracing warp owns a 1024-entry lane of the buffer and a local counter (no atomics,
@@ -201,18 +220,18 @@ __device__ __forceinline__ void tc_update_terms(const TcArgs& a, int cb, float* 
     *button_out = (int)rr.button0();
   }
 }
-// L2 prefetch of one tile's per-field raw states (rows row0.. of a.fields, up to a.B): thread m of the tile's 128 takes
-// the m-th 128-byte line of every field's range (a field holds at most 48 B per row: 49 lines with misalignment).
-// A rolled loop over the fields, the pointers read from the kernel parameters: it runs where the pool holds the most
-// registers.
-__device__ __forceinline__ void tc_prefetch_fields(const TcArgs& a, long long row0, int m) {
+// L2 prefetch of one tile's per-field raw states (rows row0.. of a.fields, up to a.B; a sequence step's rows start foff
+// rows in): thread m of the tile's 128 takes the m-th 128-byte line of every field's range (a field holds at most 48 B
+// per row: 49 lines with misalignment).  A rolled loop over the fields, the pointers read from the kernel parameters: it
+// runs where the pool holds the most registers.
+__device__ __forceinline__ void tc_prefetch_fields(const TcArgs& a, long long row0, int m, long long foff = 0) {
   const long long rows = min((long long)kTcTileM, a.B - row0);
   static_assert(sizeof(RawFieldsDev) == 8 * sizeof(void*), "eight field pointers");
 #pragma unroll 1
   for (int f = 0; f < 8; ++f) {
     // bytes per row, one byte per field: quat 16, gyro 12, q 48, dq 48, axes 16, foot_force 8, joy_valid 1, button0 1
     const long long row_bytes = (long long)((0x0101081030300C10ull >> (8 * f)) & 0xFFu);
-    const uintptr_t lo = reinterpret_cast<uintptr_t>(reinterpret_cast<const void* const*>(&a.fields)[f]) + (uintptr_t)(row0 * row_bytes);
+    const uintptr_t lo = reinterpret_cast<uintptr_t>(reinterpret_cast<const void* const*>(&a.fields)[f]) + (uintptr_t)((row0 + foff) * row_bytes);
     const uintptr_t line = (lo & ~(uintptr_t)127) + (uintptr_t)m * 128u;
     if (line < lo + (uintptr_t)(rows * row_bytes)) ptx::prefetch_l2(reinterpret_cast<const void*>(line));
   }
@@ -355,10 +374,13 @@ __device__ __noinline__ void tc_out_generic(const TcArgs& a, uint32_t o_t, long 
 // kReset (fused step only): the step reads a.reset.  A separate instantiation, so that the step without a mask runs
 // exactly the code it ran before resets existed (the per-element selects cost 2 % even when every flag is 0).
 // kFields (fused step only): the raw states come from a.fields (one array per field) instead of a.raw (records).
-template <bool kFp16, bool kFused, bool kReset = false, bool kFields = false>
+// kSeq (per-field fused step only): a.T consecutive steps (tc_unit_row0); each slot keeps its tile's observation stage in
+// shared memory from step 0 to step T-1, and the previous action of step t+1 is the one step t left in that stage.
+template <bool kFp16, bool kFused, bool kReset = false, bool kFields = false, bool kSeq = false>
 __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_constant__ TcArgs a) {
   static_assert(kFused || !kReset, "resets belong to the fused controller step");
   static_assert(kFused || !kFields, "per-field raw states belong to the fused controller step");
+  static_assert(kFields || !kSeq, "the step sequence reads per-field raw states");
   extern __shared__ __align__(128) uint8_t smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 
@@ -434,6 +456,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
 
   const long long n_tiles = (a.B + kTcTileM - 1) / kTcTileM;
   const int n_local = (int)((n_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x);   // tiles b, b+G, ...
+  const int n_units = kSeq ? 2 * a.T * ((n_local + 1) / 2) : n_local;              // (tile, step) units, see tc_unit_row0
   const uint32_t tile_bytes = (uint32_t)(kTcTileM * a.in_dim * 4);
   TC_TRACE_INIT();
 
@@ -451,8 +474,9 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
     uint8_t* stage = stage0 + s * stage_bytes;
     uint32_t par = 0u;                       // all four block barriers of a slot advance one phase per layer
     auto load_tile = [&](int i) {            // i = CTA-local tile index (slot s owns i = s, s+2, ...)
-      const long long row0 = (blockIdx.x + (long long)i * gridDim.x) * kTcTileM;
-      if (a.B - row0 >= kTcTileM) {
+      const long long row0 = tc_unit_row0<kSeq>(a, i);
+      // kSeq: steps after the first find the stage as the slot's previous unit (the same tile) left it
+      if (a.B - row0 >= kTcTileM && tc_unit_step<kSeq>(a, i) == 0) {
         TC_TRACE(0x100u | (uint32_t)s);
         ptx::mbar_arrive_expect_tx(&obs_full[s], tile_bytes);
         ptx::bulk_g2s(stage, a.obs + row0 * a.in_dim, tile_bytes, &obs_full[s]);
@@ -464,19 +488,20 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
     // raw_fields_tile) -> the raw stage; issued when conversion i-1 (the other slot's) has signalled, i.e. when every
     // warp is done with the stage
     auto load_raw = [&](int i) {
-      const long long row0 = (blockIdx.x + (long long)i * gridDim.x) * kTcTileM;
+      const long long row0 = tc_unit_row0<kSeq>(a, i);
       if (a.B - row0 >= kTcTileM) {
         if constexpr (kFields) {
           const RawFieldsDev t = raw_fields_tile(s_raw, kTcTileM);
+          const long long fr0 = row0 + (long long)tc_unit_step<kSeq>(a, i) * a.B;   // the step's rows of the fields
           ptx::mbar_arrive_expect_tx(raw_full, (uint32_t)raw_fields_tile_bytes(kTcTileM));
-          ptx::bulk_g2s(const_cast<float*>(t.quat), a.fields.quat + row0 * 4, kTcTileM * 4 * 4, raw_full);
-          ptx::bulk_g2s(const_cast<float*>(t.gyro), a.fields.gyro + row0 * 3, kTcTileM * 3 * 4, raw_full);
-          ptx::bulk_g2s(const_cast<float*>(t.q), a.fields.q + row0 * kDof, kTcTileM * kDof * 4, raw_full);
-          ptx::bulk_g2s(const_cast<float*>(t.dq), a.fields.dq + row0 * kDof, kTcTileM * kDof * 4, raw_full);
-          ptx::bulk_g2s(const_cast<float*>(t.axes), a.fields.axes + row0 * 4, kTcTileM * 4 * 4, raw_full);
-          ptx::bulk_g2s(const_cast<int16_t*>(t.foot_force), a.fields.foot_force + row0 * 4, kTcTileM * 4 * 2, raw_full);
-          ptx::bulk_g2s(const_cast<uint8_t*>(t.joy_valid), a.fields.joy_valid + row0, kTcTileM, raw_full);
-          ptx::bulk_g2s(const_cast<uint8_t*>(t.button0), a.fields.button0 + row0, kTcTileM, raw_full);
+          ptx::bulk_g2s(const_cast<float*>(t.quat), a.fields.quat + fr0 * 4, kTcTileM * 4 * 4, raw_full);
+          ptx::bulk_g2s(const_cast<float*>(t.gyro), a.fields.gyro + fr0 * 3, kTcTileM * 3 * 4, raw_full);
+          ptx::bulk_g2s(const_cast<float*>(t.q), a.fields.q + fr0 * kDof, kTcTileM * kDof * 4, raw_full);
+          ptx::bulk_g2s(const_cast<float*>(t.dq), a.fields.dq + fr0 * kDof, kTcTileM * kDof * 4, raw_full);
+          ptx::bulk_g2s(const_cast<float*>(t.axes), a.fields.axes + fr0 * 4, kTcTileM * 4 * 4, raw_full);
+          ptx::bulk_g2s(const_cast<int16_t*>(t.foot_force), a.fields.foot_force + fr0 * 4, kTcTileM * 4 * 2, raw_full);
+          ptx::bulk_g2s(const_cast<uint8_t*>(t.joy_valid), a.fields.joy_valid + fr0, kTcTileM, raw_full);
+          ptx::bulk_g2s(const_cast<uint8_t*>(t.button0), a.fields.button0 + fr0, kTcTileM, raw_full);
         } else {
           ptx::mbar_arrive_expect_tx(raw_full, (uint32_t)kTcRawStageBytes);
           ptx::bulk_g2s(s_raw, a.raw + row0, (uint32_t)kTcRawStageBytes, raw_full);
@@ -485,13 +510,13 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
         ptx::mbar_arrive(raw_full);          // ragged last tile: the pool reads global memory directly
       }
     };
-    if (s < n_local && ptx::elect_one_sync()) {
+    if (s < n_units && ptx::elect_one_sync()) {
       load_tile(s);
       if (kFused && s == 0) load_raw(0);
     }
     __syncwarp();
     int phi = 0;
-    for (int i = s; i < n_local; i += 2, phi ^= 1) {
+    for (int i = s; i < n_units; i += 2, phi ^= 1) {
       uint32_t w_off = 0;
       for (int l = 0; l < a.n_layers; ++l) {
         const int kp = tc_layer_kp(a, l), nl = tc_layer_n(a, l);
@@ -506,8 +531,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
           ptx::mbar_wait(&blk[0], par);
           ptx::tc_fence_after();
           if (ptx::elect_one_sync()) {
-            if (!kFused && i + 2 < n_local) load_tile(i + 2);
-            if (kFused && i + 1 < n_local) load_raw(i + 1);
+            if (!kFused && i + 2 < n_units) load_tile(i + 2);
+            if (kFused && i + 1 < n_units) load_raw(i + 1);
             TC_TRACE(0x200u | (uint32_t)(l << 4) | (uint32_t)s);
             const int ksteps = kp / 16;      // A chunk j sits at 32*(j/2) + 8*(j%2), ones inside the data
             for (int j = 0; j < ksteps; ++j)
@@ -519,12 +544,21 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
               // writes towards the async proxy before it signalled): send them back to the caller's history buffer
               // with one bulk copy, and refill the stage only when the copy has read it.  This warp has ~3,000
               // cycles until the slot's next MMA group; the pool never waits for the copy.
-              const long long row0 = (blockIdx.x + (long long)i * gridDim.x) * kTcTileM;
+              const long long row0 = tc_unit_row0<kSeq>(a, i);
               if (a.B - row0 >= kTcTileM) {
-                ptx::bulk_s2g(a.obs_rw + row0 * a.in_dim, stage, tile_bytes);
+                if constexpr (kSeq) {
+                  // every step to obs_seq, the last one also to the history; the stage stays for the next step.  The
+                  // output job of this step writes into the stage only after bulk_wait_read below: it waits for the
+                  // output layer's commit, which this thread issues after it
+                  const int t = tc_unit_step<kSeq>(a, i);
+                  if (a.obs_seq) ptx::bulk_s2g(a.obs_seq + ((long long)t * a.B + row0) * a.in_dim, stage, tile_bytes);
+                  if (t == a.T - 1) ptx::bulk_s2g(a.obs_rw + row0 * a.in_dim, stage, tile_bytes);
+                } else {
+                  ptx::bulk_s2g(a.obs_rw + row0 * a.in_dim, stage, tile_bytes);
+                }
                 ptx::bulk_wait_read();
               }
-              if (i + 2 < n_local) load_tile(i + 2);
+              if (i + 2 < n_units) load_tile(i + 2);
             }
           }
           __syncwarp();
@@ -577,11 +611,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
     float pf_vel[3] = {0.f, 0.f, 0.f};
     bool pf_rst = false;                                  // kReset: the row's reset flag (every column block)
     auto prefetch_state = [&](int pair, int s) {          // for conv_job(pair, s)
-      const long long row = (blockIdx.x + (long long)(pair * 2 + s) * gridDim.x) * kTcTileM + m;
+      const long long row = tc_unit_row0<kSeq>(a, pair * 2 + s) + m;
+      const int t = tc_unit_step<kSeq>(a, pair * 2 + s);
       pf_rst = false;
       if (row < a.B) {
-        if constexpr (kReset) pf_rst = a.reset[row] != 0;
-        if (cb == 3) {
+        if constexpr (kReset) pf_rst = a.reset[row + (long long)t * a.B] != 0;
+        if (cb == 3 && t == 0) {                           // kSeq, t > 0: the conversion reads it from the stage
           const float4* p4 = reinterpret_cast<const float4*>(a.act + row * kDof);
 #pragma unroll
           for (int q = 0; q < 3; ++q) pf_act[q] = p4[q];
@@ -595,7 +630,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
     //      chunk c8 (16 K elements = 8 columns) lands at 32*(c8/2) + 8*(c8%2) of buffer phi: block cb = chunks 2cb, 2cb+1
     auto conv_job = [&](int pair, int s) {
       const int phi = pair & 1;
-      const long long row0 = (blockIdx.x + (long long)(pair * 2 + s) * gridDim.x) * kTcTileM;
+      const long long row0 = tc_unit_row0<kSeq>(a, pair * 2 + s);
       const int valid = (int)min((long long)kTcTileM, a.B - row0);
       const uint32_t a0_t = tmem_base + (uint32_t)s * kTcSlotCols + lane_addr + 128u * (uint32_t)phi;
       ptx::mbar_wait(&obs_full[s], (uint32_t)(pair & 1));
@@ -610,12 +645,21 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
         const bool full = valid == kTcTileM;
         ptx::mbar_wait(raw_full, (uint32_t)(s & 1));       // CTA-local tile i = 2*pair + s: phase i & 1
         TC_TRACE(0xA00u | (uint32_t)s);
+        const int t = tc_unit_step<kSeq>(a, pair * 2 + s);
         if (m < valid) {
           int lo, hi;
           tc_term_range(cb, a.H, lo, hi);
+          if constexpr (kSeq) {
+            // the previous step's output job left the published action in the oldest frame of the action term
+            if (cb == 3 && t > 0) {
+              const float* pa = srow + 33 * a.H;
+#pragma unroll
+              for (int q = 0; q < 3; ++q) pf_act[q] = make_float4(pa[4 * q], pa[4 * q + 1], pa[4 * q + 2], pa[4 * q + 3]);
+            }
+          }
           if (!full) for (int k = lo; k < hi; ++k) srow[k] = a.obs_rw[(row0 + m) * a.in_dim + k];   // ragged tile: no bulk load
           if constexpr (kFields) {
-            if (!full) tc_stage_fields_row(a, cb, s_raw, row0 + m, m);
+            if (!full) tc_stage_fields_row(a, cb, s_raw, row0 + (long long)t * a.B + m, m);
             tc_update_terms(a, cb, srow, RawFieldRow<kTcTileM>{s_raw, m}, row0 + m, &s_button[(s * 2 + (pair & 1)) * kTcTileM + m], pf_act,
                             pf_vel, pf_rst);
           } else {
@@ -624,6 +668,10 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
                             pf_rst);
           }
           if (!full) for (int k = lo; k < hi; ++k) a.obs_rw[(row0 + m) * a.in_dim + k] = srow[k];
+          if constexpr (kSeq) {
+            if (!full && a.obs_seq)
+              for (int k = lo; k < hi; ++k) a.obs_seq[((long long)t * a.B + row0 + m) * a.in_dim + k] = srow[k];
+          }
         }
         TC_TRACE(0xB00u | (uint32_t)s);
         ptx::fence_proxy_async_smem();     // the control warp bulk-copies the stage to global memory once all warps signalled
@@ -669,7 +717,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
     // ---- out(s) (bias already inside the accumulator): (+ELU) (+clamp/mask) (+q_des) -> global
     auto out_job = [&](int pair, int s) {
       const int phi = pair & 1;
-      const long long row0 = (blockIdx.x + (long long)(pair * 2 + s) * gridDim.x) * kTcTileM;
+      const long long row0 = tc_unit_row0<kSeq>(a, pair * 2 + s);
+      const int t = tc_unit_step<kSeq>(a, pair * 2 + s);
       const int valid = (int)min((long long)kTcTileM, a.B - row0);
       const uint32_t o_t = tmem_base + (uint32_t)s * kTcSlotCols + lane_addr + 128u * (uint32_t)((phi + 1 + L) & 1);
       ptx::mbar_wait(&acc_full[s], par_acc[s]);
@@ -683,7 +732,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
           ptx::tmem_ld_x4(o_t + (uint32_t)(cb * 4), v);
           ptx::tc_wait_ld();
           if (m < valid) {
-            const long long row = row0 + m;
+            const long long row = row0 + m + (long long)t * a.B;
             float o[4];
 #pragma unroll
             for (int j = 0; j < 4; ++j) o[j] = __uint_as_float(v[j]);
@@ -693,27 +742,42 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
 #pragma unroll
               for (int j = 0; j < 4; ++j) o[j] = clamp_mask(o[j], a.action_limit, b0);
             }
-            reinterpret_cast<float4*>(a.act + row * 12)[cb] = make_float4(o[0], o[1], o[2], o[3]);
+            if constexpr (kSeq) {
+              reinterpret_cast<float4*>(a.act_seq + row * 12)[cb] = make_float4(o[0], o[1], o[2], o[3]);
+              if (t == a.T - 1) {
+                reinterpret_cast<float4*>(a.act + (row0 + m) * 12)[cb] = make_float4(o[0], o[1], o[2], o[3]);
+              } else {
+                // the next step's previous action, into the oldest frame of the row's action term in the stage (that
+                // conversion discards the frame; the bulk stores of this step's stage have been read, see the control
+                // warp).  Not at the last step: the next tile's observations may be landing in the stage by then
+                float* pa = reinterpret_cast<float*>(stage0 + s * stage_bytes) + (size_t)m * a.in_dim + 33 * a.H + cb * 4;
+#pragma unroll
+                for (int j = 0; j < 4; ++j) pa[j] = o[j];
+              }
+            } else {
+              reinterpret_cast<float4*>(a.act + row * 12)[cb] = make_float4(o[0], o[1], o[2], o[3]);
+            }
             if (a.flags & 6u) {
               double qd[4];
 #pragma unroll
               for (int j = 0; j < 4; ++j) qd[j] = joint_target(o[j], a.q0[cb * 4 + j], a.action_scale);
-              if ((a.flags & 2u) && a.qdes) {
-                double2* q2 = reinterpret_cast<double2*>(a.qdes + row * kDof + cb * 4);
+              // kSeq: the step's slices of the per-step outputs (row includes t*B)
+              if ((a.flags & 2u) && (kSeq ? a.qdes_seq : a.qdes)) {
+                double2* q2 = reinterpret_cast<double2*>((kSeq ? a.qdes_seq : a.qdes) + row * kDof + cb * 4);
                 q2[0] = make_double2(qd[0], qd[1]);
                 q2[1] = make_double2(qd[2], qd[3]);
               }
-              if ((a.flags & 4u) && a.cmd) {
+              if ((a.flags & 4u) && (kSeq ? a.cmd_seq : a.cmd)) {
                 // Isaac joint 4*cb + j = joint type cb of leg j -> Unitree motor (j ^ 1)*3 + cb
-                MotorCmdDev* c = a.cmd + row;
+                MotorCmdDev* c = (kSeq ? a.cmd_seq : a.cmd) + row;
 #pragma unroll
                 for (int j = 0; j < 4; ++j) c->q_des[(j ^ 1) * 3 + cb] = qd[j];
-                if (cb == 0) store_gains(a.cmd, row, kFused ? s_button[(s * 2 + (pair & 1)) * kTcTileM + m] : (s ? b0_s1 : b0_s0), a.kp, a.kd, a.kp_deadman);
+                if (cb == 0) store_gains(kSeq ? a.cmd_seq : a.cmd, row, kFused ? s_button[(s * 2 + (pair & 1)) * kTcTileM + m] : (s ? b0_s1 : b0_s0), a.kp, a.kd, a.kp_deadman);
               }
             }
           }
         }
-      } else if (cb == 0) {
+      } else if (cb == 0 && !kSeq) {          // kSeq serves the 12-output, no-activation case only (the host checks)
         tc_out_generic(a, o_t, row0 + m, m < valid);
       }
       ptx::tc_fence_before();
@@ -726,13 +790,13 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
     // a whole job of cover each (they used to be waited for).  Hazards: conv'(s) writes the buffer that held A(L),
     // consumed by the MMA out(s) has just waited for; the layer-0 MMA of the new tile overwrites the buffer out(s)
     // reads, but it is issued only after ALL warps signalled conv'(s), i.e. after their out(s) reads.
-    for (int s = 0; s < min(2, n_local); ++s) {
+    for (int s = 0; s < min(2, n_units); ++s) {
       if constexpr (kFused) prefetch_state(0, s);
       conv_job(0, s);
     }
-    for (int pair = 0; pair * 2 < n_local; ++pair) {
-      const int ns = min(2, n_local - pair * 2);
-      const int ns_next = max(0, min(2, n_local - (pair + 1) * 2));
+    for (int pair = 0; pair * 2 < n_units; ++pair) {
+      const int ns = min(2, n_units - pair * 2);
+      const int ns_next = max(0, min(2, n_units - (pair + 1) * 2));
       const int phi = pair & 1;
 
       // ---- E(l,s): accumulator block -> ELU -> 16-bit A operand of the next layer, in place
@@ -751,10 +815,10 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
           if (l == 0) {
             // the next pair's conversion jobs read these robots' raw states and previous actions: pull them into L2 now,
             // two layers ahead (no registers held, nothing waited for)
-            const long long r0 = (blockIdx.x + (long long)(pair * 2 + 2 + (cb & 1)) * gridDim.x) * kTcTileM + m;
+            const long long r0 = tc_unit_row0<kSeq>(a, pair * 2 + 2 + (cb & 1)) + m;
             if (r0 < a.B) {
               if (cb < 2) {
-                if constexpr (kFields) tc_prefetch_fields(a, r0 - m, m);
+                if constexpr (kFields) tc_prefetch_fields(a, r0 - m, m, (long long)tc_unit_step<kSeq>(a, pair * 2 + 2 + (cb & 1)) * a.B);
                 else { ptx::prefetch_l2(a.raw + r0); ptx::prefetch_l2(reinterpret_cast<const uint8_t*>(a.raw + r0) + sizeof(RawStateDev) - 1); }
               }
               else { ptx::prefetch_l2(a.act + r0 * kDof); ptx::prefetch_l2(a.vel_cmd + r0 * 3); }
@@ -805,7 +869,9 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
         // layer-0 operand: the four warps of a lane quarter (the only ones touching these lanes) meet before any of
         // them converts the next tile, so no conversion store can overtake a sibling's output read.  (Odd counts --
         // the Go2 policy -- use the other buffer and skip this.)
-        if ((L & 1) == 0) {
+        // kSeq: the same meeting orders the action stores of column blocks 0-2 into the stage before column block 3's
+        // read of them in the conversion of the tile's next step.
+        if (kSeq || (L & 1) == 0) {
           __syncwarp();
           asm volatile("bar.sync %0, 128;" ::"r"(1 + quarter) : "memory");
         }

@@ -252,6 +252,24 @@ typedef struct go2p_raw_fields {
 int go2p_step_batch_fields(go2p_handle* h, const go2p_raw_fields* f, const uint8_t* d_reset, float* d_vel_cmd,
                            float* d_obs, float* d_action, double* d_qdes, go2p_motor_cmd* d_cmd, int64_t B,
                            int precision, void* stream);
+/* T consecutive go2p_step_batch_fields steps of B robots in one call, e.g. to replay recorded sensor streams
+ * closed-loop.  Every field of f points at T*B rows, step-major ([T,B,w]: step t's array starts t*B rows in).
+ * d_reset: [T,B] uint8 or NULL.  State in/out exactly as in the single step: d_vel_cmd [B,3], d_obs [B,49*H],
+ * d_action [B,12] hold the state before step 0 on entry and after step T-1 on return.  Per-step outputs:
+ * d_action_seq [T,B,12] float (required) = the published action of every step; d_qdes_seq [T,B,12] double, d_cmd_seq
+ * [T,B] go2p_motor_cmd, d_obs_seq [T,B,49*H] float (the ObservationAction observation of every step): each may be NULL
+ * (unlike the single step, d_qdes and d_cmd may both be NULL).
+ * The call leaves exactly the bytes that T calls of go2p_step_batch_fields leave on the step-t slices, with d_action
+ * copied to d_action_seq[t] and d_obs to d_obs_seq[t] after each.  fp16 / bf16 take ONE launch (go2p_last_launch_count
+ * 1) where the one-launch single step would serve step 0 and every step's slices are 16-byte aligned (B % 16 == 0,
+ * aligned bases); the history then stays in shared memory from step 0 to step T-1.  Every other case steps T times,
+ * each step by the single step's rules (the launch count is the sum of their kernels).  Argument rules as in
+ * go2p_step_batch_fields; T or B = 0 does nothing; a negative T or B, or T*B*49*H beyond int64 for
+ * the largest history (H = 8), is GO2P_ERR_INVALID. */
+int go2p_step_batch_fields_seq(go2p_handle* h, const go2p_raw_fields* f, int64_t T, const uint8_t* d_reset,
+                               float* d_vel_cmd, float* d_obs, float* d_action, float* d_action_seq,
+                               double* d_qdes_seq, go2p_motor_cmd* d_cmd_seq, float* d_obs_seq,
+                               int64_t B, int precision, void* stream);
 /* go2p_step_fused + the same step's send_command arguments in motor order (out may be NULL) */
 int go2p_step_fused_cmd(go2p_handle* h, const go2p_raw_state* raw, go2p_step_out* out, go2p_motor_cmd* cmd);
 /* isaac_of_motor[u] = Isaac joint index of Unitree motor u */

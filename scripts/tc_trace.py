@@ -1,6 +1,9 @@
 """Timeline of one CTA of tc_mlp_kernel (trace build: -DGO2P_TC_TRACE, lib/libgo2policy_trace.so).
 usage: tc_trace.py [rows] [first event] [count] [warps, comma separated]
-GO2P_TRACE_STEP=1 traces the fused controller step; GO2P_TRACE_RESET=p adds a mask resetting a fraction p of the robots."""
+GO2P_TRACE_STEP=1 traces the fused controller step; GO2P_TRACE_RESET=p adds a mask resetting a fraction p of the robots.
+GO2P_TRACE_SEQ=T traces T steps from per-field streams in one launch (go2p_step_batch_fields_seq); GO2P_TRACE_SEQ=F the
+single per-field step (go2p_step_batch_fields).  Every run also prints, per traced pool warp, the cycles per output job
+(one output job per tile-step)."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -35,10 +38,29 @@ if FUSED:
     # GO2P_TRACE_RESET=p: the step with per-robot resets (go2p_step_batch_ex), a fraction p of the robots reset
     RESET = float(os.environ["GO2P_TRACE_RESET"]) if os.environ.get("GO2P_TRACE_RESET") else None
     d_rst = (torch.rand(B, device="cuda", generator=torch.Generator(device="cuda").manual_seed(5)) < RESET) if RESET is not None else None
+SEQ = os.environ.get("GO2P_TRACE_SEQ")
+if SEQ:
+    import ctypes as C
+    from go2_onnx_controller_b200 import actor
+    T = 1 if SEQ == "F" else int(SEQ)
+    g = torch.Generator(device="cuda").manual_seed(5)
+    fl = {n: (torch.rand((T, B) + ((w,) if w else ()), device="cuda", generator=g) * (60 if n == "foot_force" else 1)).to(
+        torch.int16 if n == "foot_force" else torch.uint8 if w is None else torch.float32) for n, w in actor.RAW_FIELDS}
+    f = capi.RawFields(*[fl[n].data_ptr() for n, _ in actor.RAW_FIELDS])
+    d_obs = torch.zeros((B, 98), device="cuda"); d_vel = torch.zeros((B, 3), device="cuda")
+    d_act = torch.zeros((B, 12), device="cuda"); d_q = torch.zeros((B, 12), device="cuda", dtype=torch.float64)
+    d_aseq = torch.zeros((T, B, 12), device="cuda")
 for _ in range(3):
     trace.zero_()
     torch.cuda.synchronize()
-    if FUSED:
+    if SEQ == "F":
+        capi.check(pb._hd.lib.go2p_step_batch_fields(pb._hd.h, C.byref(f), None, d_vel.data_ptr(), d_obs.data_ptr(),
+                                                     d_act.data_ptr(), d_q.data_ptr(), None, B, capi.PREC_FP16, None))
+    elif SEQ:
+        capi.check(pb._hd.lib.go2p_step_batch_fields_seq(pb._hd.h, C.byref(f), T, None, d_vel.data_ptr(), d_obs.data_ptr(),
+                                                         d_act.data_ptr(), d_aseq.data_ptr(), None, None, None, B,
+                                                         capi.PREC_FP16, None))
+    elif FUSED:
         pb.step_device(d_raw.data_ptr(), d_vel.data_ptr(), d_obs.data_ptr(), d_act.data_ptr(), d_q.data_ptr(), B, capi.PREC_FP16,
                        d_reset=None if d_rst is None else d_rst.data_ptr())
     else:
@@ -53,6 +75,9 @@ c0 = min(int(t[w, 1]) for w in range(17) if t[w, 2046] > 0)
 for w in warps:
     n = int(t[w, 2046]); ev = t[w, 0:2 * n:2]; ck = t[w, 1:2 * n:2]
     print(f"--- warp {w}: {n} events, span {int(ck[-1] - ck[0])} cycles")
+    outs = ck[(ev >> 8) == 9]
+    if len(outs) > 2:
+        print(f"    {np.diff(outs).mean() * 1.0:.0f} cycles per output job (median {np.median(np.diff(outs)):.0f}) over {len(outs)} jobs")
     prev = None
     for e, c in list(zip(ev, ck))[(lo if w < 16 else lo * 13 // 19):][:cnt]:
         e = int(e); k = e >> 8; l = (e >> 4) & 15; s = e & 3
