@@ -567,7 +567,8 @@ int launch_tc(go2p_handle* h, const float* d_obs, const int32_t* d_button0, floa
   a.wpack = h->d_wpack[fp16 ? 1 : 0];
   a.n_layers = h->dm.n_layers; a.in_dim = h->dm.in_dim; a.k0p = h->k0p; a.out_dim = h->dm.out_dim;
   for (int l = 0; l < h->dm.n_layers; ++l) {
-    a.has_elu[l] = h->dm.L[l].has_elu;
+    const float alpha = h->dm.L[l].alpha;
+    a.has_elu[l] = !h->dm.L[l].has_elu ? kEluNone : (alpha >= 0.f && alpha <= 1.f) ? kEluMax : kEluSelect;
     a.elu_c[l] = (float)((double)h->dm.L[l].alpha * 1.4426950408889634074);
   }
   a.out_scale = h->dm.L[h->dm.n_layers - 1].has_elu ? 0.69314718055994530942f : 1.0f;

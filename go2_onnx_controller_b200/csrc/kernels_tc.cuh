@@ -23,10 +23,10 @@
 //   * the chain is evaluated in the base-2 exponent domain: layer l produces z' = log2(e)*z, the ELU is
 //     h' = z' > 0 ? z' : c*(2^z' - 1) with c = alpha*log2(e), h' = log2(e)*h feeds the next layer whose weights
 //     carry the inverse factor (folded on the host);
-//   * fp16 path: the ELU runs on packed pairs -- F2FP (pack z'), ex2.approx.f16x2 (2 MUFU + PRMT), one HFMA2
-//     (c*e - c), HSET2 + LOP3 select: 7 instructions per pair; two pairs in eight take a packed-half polynomial
-//     2^x on the FMA pipe instead (elu_neg_poly_f16x2): the MUFU (4 lanes/clk per scheduler, an ex2.f16x2 is two
-//     MUFU.EX2.F16) is what an epilogue job saturates.  bf16 keeps the fp32 exponential;
+//   * fp16 path: the ELU runs on packed pairs -- F2FP (pack z'), ex2.approx.f16x2 of -|z'| (2 MUFU + PRMT), one
+//     HFMA2 (c*e - c), one HMNMX2.NAN select max(z', e) when 0 <= alpha <= 1: 6 instructions per pair; four pairs in
+//     sixteen take a packed-half polynomial 2^x on the FMA pipe instead (elu_neg_poly_f16x2): the MUFU (an ex2.f16x2 is
+//     two MUFU.EX2.F16) is what an epilogue job saturates.  bf16 keeps the fp32 exponential;
 //   * one elected thread issues every tcgen05.mma and signals completion with tcgen05.commit; ONE pool of 16 worker
 //     warps walks the jobs of both slots alternately, so a slot's MMAs run while the pool works on the other slot.
 #pragma once
@@ -54,7 +54,7 @@ struct TcArgs {
   long long B;
   const uint16_t* wpack;     // per layer: N_l x Kp_l 16-bit, UMMA K-major interleaved layout (bias rows included)
   int n_layers, in_dim, k0p, out_dim;
-  int has_elu[kMaxLayers];
+  int has_elu[kMaxLayers];   // kEluNone / kEluSelect / kEluMax (elu_pack32; the output layer tests != 0 only)
   float elu_c[kMaxLayers];   // alpha * log2(e)
   float out_scale;           // ln(2) if the last layer has an ELU (its output is in the scaled domain), else 1
   uint32_t flags;
@@ -243,49 +243,58 @@ __device__ __forceinline__ void tc_term_range(int cb, int H, int& lo, int& hi) {
   hi = cb == 0 ? 9 * H : cb == 1 ? 21 * H : cb == 2 ? 33 * H : 49 * H;
 }
 
-// c*(2^z - 1) for z < 0 on a packed fp16 pair without the MUFU: clamp at -13 (2^-13 is below the resolution of the
-// result), split z = -k + r with the 1536 = 1.5*2^10 rounding trick (k = 0..13 lands in the low mantissa bits of u),
-// degree-3 polynomial for 2*2^r on [-0.5, 0.5] (the factor 2 keeps every pair's exponent field >= k, so the packed
-// integer subtraction of k << 10 never borrows across the halves, whatever garbage a discarded z >= 0 lane holds),
-// then (c/2)*p - c as one HFMA2: 10 instructions after the pack, none on the MUFU.  Max abs error 9.1e-4 over all
-// negative fp16 inputs vs 8.4e-4 for a correctly rounded 2^z followed by the same HFMA2 (exhaustive CPU emulation,
-// scripts/experiments/polyelu.py).
+// c*(2^x - 1) for x = -|z| <= 0 on a packed fp16 pair without the MUFU: clamp at -13 (2^-13 is below the resolution of
+// the result; the -|.| rides on the clamp's HMNMX2 as a source modifier), split x = -k + r with the 1536 = 1.5*2^10
+// rounding trick (k = 0..13 lands in the low mantissa bits of u), degree-3 polynomial for 2*2^r on [-0.5, 0.5] (p's
+// exponent field is >= 15 > k, so the packed integer subtraction of k << 10 keeps the result normal and never borrows
+// across the halves), then (c/2)*p - c as one HFMA2: 10 instructions after the pack, none on the MUFU.  Max abs error
+// 9.1e-4 over all negative fp16 inputs vs 8.4e-4 for a correctly rounded 2^z followed by the same HFMA2; the max.NaN
+// select of elu_pack16 keeps both bounds (exhaustive CPU emulation over every fp16 input, scripts/experiments/polyelu.py).
 __device__ __forceinline__ uint32_t elu_neg_poly_f16x2(uint32_t z, uint32_t ch2, uint32_t nc2) {
-  const uint32_t kM = 0x66006600u;                        // (1536, 1536)
-  const uint32_t zc = ptx::max_f16x2(z, 0xCA80CA80u);     // max(z, -13)
-  const uint32_t u = ptx::sub_f16x2(kM, zc);              // 1536 + k, k = round(-zc)
-  const uint32_t r = ptx::add_f16x2(zc, ptx::sub_f16x2(u, kM));
+  const uint32_t kM = 0x66006600u;                                              // (1536, 1536)
+  const uint32_t xc = ptx::max_f16x2(ptx::negabs_f16x2(z), 0xCA80CA80u);      // max(-|z|, -13)
+  const uint32_t u = ptx::sub_f16x2(kM, xc);                                    // 1536 + k, k = round(-xc)
+  const uint32_t r = ptx::add_f16x2(xc, ptx::sub_f16x2(u, kM));
   uint32_t p = ptx::fma_f16x2(0x2F102F10u, r, 0x37C337C3u);   // 0.11035 r + 0.48511
   p = ptx::fma_f16x2(p, r, 0x3D8C3D8Cu);                      // ... + 1.38672
   p = ptx::fma_f16x2(p, r, 0x40004000u);                      // ... + 2.0
-  p -= (u & 0x000F000Fu) << 10;                               // * 2^-k
+  p = ptx::mad_lo_u32(u & 0x000F000Fu, 0xFFFFFC00u, p);       // * 2^-k: p - (k << 10) per half, as LOP3 + IMAD
   return ptx::fma_f16x2(p, ch2, nc2);
 }
 
-// same on 16 accumulator columns -> 8 packed words.  fp16: every pair stays packed -- F2FP (pack z'), then either
-// ex2.approx.f16x2 (2 MUFU + PRMT) + HFMA2 (c*e - c) or, for the pairs selected by GO2P_TC_POLYMASK, the FMA-pipe
-// polynomial above; HSET2 + LOP3 select.  bf16 keeps the fp32 exponential everywhere (its budget has no slack).
+// TcArgs::has_elu of a hidden layer: how elu_pack32 selects between z' and the exponential branch e' = c*2^-|z'| - c
+enum : int {
+  kEluNone = 0,
+  kEluSelect = 1,   // z' < 0 ? e' : z' (HSET2 + LOP3): any alpha
+  kEluMax = 2,      // max.NaN(z', e') (one HMNMX2): 0 <= alpha <= 1, where c*(2^z' - 1) >= z' for every z' <= 0
+};
+
+// ELU of 16 accumulator columns -> 8 packed words.  fp16: every pair stays packed -- F2FP (pack z'), then either
+// ex2.approx.f16x2 of -|z'| (2 MUFU with the -|.| source modifier + PRMT) + HFMA2 (c*e - c) or, for the pairs in kMask,
+// the FMA-pipe polynomial above; then the select.  kEluMax is exact: for z' > 0, e' < 0 < z'; for z' <= 0, e' is the
+// ELU, which is >= z' when alpha <= 1 (where rounding puts the computed e' below z', z' is the closer of the two to the
+// true value); max.NaN keeps a NaN input NaN.  bf16: the fp32 exponential of -|z| (its budget has no room for the fp16
+// one) and the same select in bf16x2.  c2, ch2, nc2: c, c/2 and -c as packed fp16 pairs.
 #ifndef GO2P_TC_WARM_L2
 #define GO2P_TC_WARM_L2 1
 #endif
 #ifndef GO2P_TC_POLYMASK
-#define GO2P_TC_POLYMASK 0x88u     // bit j: column pair j of every 8 takes the FMA-pipe exponential (2 of 8)
+#define GO2P_TC_POLYMASK 0xC0C0u   // bit j: column pair j of a warp's 16 per job takes the FMA-pipe exponential (4 of 16)
 #endif
 
-template <bool kFp16>
-__device__ __forceinline__ void elu_pack16(const uint32_t (&v)[16], bool has_elu, float c, uint32_t (&p)[8]) {
+template <bool kFp16, int kElu, uint32_t kMask>
+__device__ __forceinline__ void elu_pack16(const uint32_t (&v)[16], float c, uint32_t c2, uint32_t ch2, uint32_t nc2, uint32_t (&p)[8]) {
   const float nc = -c;
   if constexpr (kFp16) {
-    const uint32_t c2 = ptx::pack_f16_sat(c, c), nc2 = ptx::pack_f16_sat(nc, nc), ch2 = ptx::pack_f16_sat(0.5f * c, 0.5f * c);
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
       const uint32_t zp = ptx::pack_f16_sat(__uint_as_float(v[2 * j]), __uint_as_float(v[2 * j + 1]));
-      if (has_elu) {
-        const uint32_t f = ((GO2P_TC_POLYMASK >> j) & 1u) ? elu_neg_poly_f16x2(zp, ch2, nc2)
-                                                         : ptx::fma_f16x2(ptx::ex2_f16x2(zp), c2, nc2);
-        p[j] = ptx::select_neg_f16x2(zp, f);
-      } else {
+      if constexpr (kElu == kEluNone) {
         p[j] = zp;
+      } else {
+        const uint32_t e = ((kMask >> j) & 1u) ? elu_neg_poly_f16x2(zp, ch2, nc2)
+                                               : ptx::fma_f16x2(ptx::ex2_f16x2(ptx::negabs_f16x2(zp)), c2, nc2);
+        p[j] = kElu == kEluMax ? ptx::max_nan_f16x2(zp, e) : ptx::select_neg_f16x2(zp, e);
       }
     }
   } else {
@@ -293,15 +302,32 @@ __device__ __forceinline__ void elu_pack16(const uint32_t (&v)[16], bool has_elu
     for (int j = 0; j < 8; ++j) {
       const float z0 = __uint_as_float(v[2 * j]), z1 = __uint_as_float(v[2 * j + 1]);
       const uint32_t zp = ptx::pack_bf16(z0, z1);
-      if (has_elu) {
-        const float f0 = fmaf(ptx::ex2_approx(z0), c, nc);
-        const float f1 = fmaf(ptx::ex2_approx(z1), c, nc);
-        p[j] = ptx::select_neg_bf16x2(zp, ptx::pack_bf16(f0, f1));
-      } else {
+      if constexpr (kElu == kEluNone) {
         p[j] = zp;
+      } else {
+        const uint32_t e = ptx::pack_bf16(fmaf(ptx::ex2_approx(-fabsf(z0)), c, nc), fmaf(ptx::ex2_approx(-fabsf(z1)), c, nc));
+        p[j] = kElu == kEluMax ? ptx::max_nan_bf16x2(zp, e) : ptx::select_neg_bf16x2(zp, e);
       }
     }
   }
+}
+// a warp's whole job (32 columns = 16 pairs) under ONE branch on the layer's ELU: the compiler interleaves the two
+// halves, so the MUFU queue of one half runs under the dependent tail (PRMT, HFMA2, select) of the other
+template <bool kFp16, int kElu>
+__device__ __forceinline__ void elu_pack32_sel(const uint32_t (&v0)[16], const uint32_t (&v1)[16], float c, uint32_t c2, uint32_t ch2,
+                                               uint32_t nc2, uint32_t (&p)[16]) {
+  uint32_t p0[8], p1[8];
+  elu_pack16<kFp16, kElu, (GO2P_TC_POLYMASK & 0xFFu)>(v0, c, c2, ch2, nc2, p0);
+  elu_pack16<kFp16, kElu, ((GO2P_TC_POLYMASK >> 8) & 0xFFu)>(v1, c, c2, ch2, nc2, p1);
+#pragma unroll
+  for (int j = 0; j < 8; ++j) { p[j] = p0[j]; p[8 + j] = p1[j]; }
+}
+template <bool kFp16>
+__device__ __forceinline__ void elu_pack32(const uint32_t (&v0)[16], const uint32_t (&v1)[16], int elu, float c, uint32_t (&p)[16]) {
+  const uint32_t c2 = ptx::pack_f16_sat(c, c), ch2 = ptx::pack_f16_sat(0.5f * c, 0.5f * c), nc2 = ptx::pack_f16_sat(-c, -c);
+  if (elu == kEluMax) elu_pack32_sel<kFp16, kEluMax>(v0, v1, c, c2, ch2, nc2, p);
+  else if (elu == kEluSelect) elu_pack32_sel<kFp16, kEluSelect>(v0, v1, c, c2, ch2, nc2, p);
+  else elu_pack32_sel<kFp16, kEluNone>(v0, v1, c, c2, ch2, nc2, p);
 }
 
 
@@ -801,7 +827,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
 
       // ---- E(l,s): accumulator block -> ELU -> 16-bit A operand of the next layer, in place
       for (int l = 0; l < L; ++l) {
-        const bool he = a.has_elu[l] != 0;
+        const int elu = a.has_elu[l];
         const float c = a.elu_c[l];
         if (l == L - 1 && masked) {
           // the output jobs of this pair need the rows' dead-man buttons: request them two jobs ahead, so the global
@@ -831,24 +857,18 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
           par_acc[s] ^= 1u;
           ptx::tc_fence_after();
           TC_TRACE(0x600u | (uint32_t)(l << 4) | (uint32_t)s);
-          // rolled loop over 4 groups of 8 columns (small code: it stays in the instruction cache); the load of group
-          // g+1 is in flight while group g is evaluated.  In-place store: the 4 packed words of group g land on
-          // columns that hold accumulator values of groups <= g, all of which are already in registers.
-          // two halves of 16 columns: the second half's load is in flight while the first is evaluated.  In-place
-          // store: the 8 packed words of half h land on columns 8h..8h+7, which hold accumulator values of half 0 only.
-          uint32_t cur[16], nxt[16], pk[8];
+          // the block's 32 accumulator columns in two loads, the 16 packed words in one store, in place: they land on
+          // columns 0..15, whose accumulator values are already in registers
+          uint32_t cur[16], nxt[16];
           ptx::tmem_ld_x16(d_t, cur);
           ptx::tmem_ld_x16(d_t + 16u, nxt);
           ptx::tc_wait_ld();
           TC_TRACE(0xF00u | (1u << 4) | (uint32_t)s);
-          elu_pack16<kFp16>(cur, he, c, pk);
-          TC_TRACE(0xF00u | (2u << 4) | (uint32_t)s);
-          ptx::tmem_st_x8(d_t, pk);
-          bool sat = kFp16 && a.sat_count && any_saturated_f16x2(pk);
-          elu_pack16<kFp16>(nxt, he, c, pk);
+          uint32_t pk[16];
+          elu_pack32<kFp16>(cur, nxt, elu, c, pk);
           TC_TRACE(0xF00u | (3u << 4) | (uint32_t)s);
-          ptx::tmem_st_x8(d_t + 8u, pk);
-          if (kFp16 && a.sat_count) n_sat += (sat || any_saturated_f16x2(pk)) ? 1u : 0u;
+          ptx::tmem_st_x16(d_t, pk);
+          if (kFp16 && a.sat_count) n_sat += any_saturated_f16x2(pk) ? 1u : 0u;
           if (cb == 0) {   // constant-one columns (K = 128,129; zeros up to 143) in the dead half of block 0
             const uint32_t ones[8] = {one2, 0u, 0u, 0u, 0u, 0u, 0u, 0u};
             ptx::tmem_st_x8(d_t + 16u, ones);

@@ -337,6 +337,31 @@ __device__ __forceinline__ uint32_t max_f16x2(uint32_t a, uint32_t b) {
   asm("max.f16x2 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b));
   return r;
 }
+// per half: the larger operand; NaN if either operand is NaN (one HMNMX2.NAN)
+__device__ __forceinline__ uint32_t max_nan_f16x2(uint32_t a, uint32_t b) {
+  uint32_t r;
+  asm("max.NaN.f16x2 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b));
+  return r;
+}
+__device__ __forceinline__ uint32_t max_nan_bf16x2(uint32_t a, uint32_t b) {
+  uint32_t r;
+  asm("max.NaN.bf16x2 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b));
+  return r;
+}
+// a*b + c (mod 2^32) as one IMAD: the compiler splits a multiplication by a power of two into a shift and an add
+__device__ __forceinline__ uint32_t mad_lo_u32(uint32_t a, uint32_t b, uint32_t c) {
+  uint32_t r;
+  asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(r) : "r"(a), "r"(b), "r"(c));
+  return r;
+}
+// per half: -|x|.  Two separate PTX operations so that ptxas folds them into the consumer's source operand as the -|.|
+// modifier (MUFU.EX2.F16 R, -|R0|; HMNMX2 R, -|R0|, ...): no instruction of its own
+__device__ __forceinline__ uint32_t negabs_f16x2(uint32_t x) {
+  uint32_t a, r;
+  asm("abs.f16x2 %0, %1;" : "=r"(a) : "r"(x));
+  asm("neg.f16x2 %0, %1;" : "=r"(r) : "r"(a));
+  return r;
+}
 // 2^x for x <= 0 on the FMA/ALU pipes (no MUFU): round-to-nearest split x = n + r via the 1.5*2^23 trick,
 // degree-3 minimax polynomial for 2^r on [-0.5, 0.5] (max relative error 7.5e-5, below half an fp16 ulp), exponent
 // patched in with an integer add.  Inputs below -24 are clamped (2^-24 is far below the resolution of c*(2^x - 1));
