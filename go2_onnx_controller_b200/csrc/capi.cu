@@ -80,11 +80,7 @@ struct go2p_handle {
   size_t tc_off[kMaxLayers] = {};              // layer l's image starts tc_off[l] elements into d_wpack[0] / [1]
   int tc_kp[kMaxLayers] = {};
   double tc_wscale[kMaxLayers] = {}, tc_bscale[kMaxLayers] = {};   // the scales pack_umma_kmajor applied
-  size_t tc_attr_smem[14] = {};                // dynamic shared memory opted in for tc_mlp_kernel<bf16|fp16, plain|fused|fused+reset,
-                                               // records|fields|field sequence> on this device
-  bool b1_attr_set = false;                    // same for the one-shot batch-1 kernel
-  size_t so_attr_smem = 0;                     // same for small_out_kernel
-  size_t split_attr_smem[3] = {};              // same for wide_gemm_kernel<128 | 64 | 16, split>
+  std::vector<std::pair<const void*, size_t>> smem_opt_in;   // (kernel, dynamic shared memory it is opted in to): opt_in_smem
   WideModel wide{};
   // activation ping-pong buffers between the per-layer launches of the fp32 path and of the wide path, one pair per
   // stream set: set 0 serves the device-pointer API, sets 1..kPipeDepth the streams of the host-buffer pipeline (which
@@ -180,6 +176,18 @@ int dev_upload(go2p_handle* h, const std::vector<T>& v, T** out) {
   CU_TRY(cudaMemcpy(p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
   *out = p;
   return GO2P_OK;
+}
+
+// Opts kernel fn in to `bytes` of dynamic shared memory.  The opt-in is a per-device function attribute, so the handle
+// (bound to one device) remembers it and sets the attribute only when the size it needs changes.
+cudaError_t opt_in_smem(go2p_handle* h, const void* fn, size_t bytes) {
+  auto it = std::find_if(h->smem_opt_in.begin(), h->smem_opt_in.end(), [fn](const auto& r) { return r.first == fn; });
+  if (it != h->smem_opt_in.end() && it->second == bytes) return cudaSuccess;
+  const cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  if (e != cudaSuccess) return e;
+  if (it != h->smem_opt_in.end()) it->second = bytes;
+  else h->smem_opt_in.emplace_back(fn, bytes);
+  return cudaSuccess;
 }
 
 inline int round_up(int v, int m) { return (v + m - 1) / m * m; }
@@ -301,11 +309,7 @@ int upload_model(go2p_handle* h) {
 }
 
 // the Go2 topology keeps its weights in registers (kernels_b1.cuh: B1RegWeights)
-bool b1_regs_ok(const go2p_handle* h) {
-  const DevModel& m = h->dm;
-  return m.n_layers == 4 && m.L[0].N == 128 && m.L[1].N == 128 && m.L[2].N == 128 && m.L[1].K == 128 && m.L[2].K == 128 &&
-         m.L[3].K == 128 && m.L[3].N <= 16 && m.L[0].Kp <= 112 && std::getenv("GO2P_B1_NO_REGS") == nullptr;
-}
+bool b1_regs_ok(const go2p_handle* h) { return B1RegWeights::supported(h->dm); }
 
 size_t b1_smem_bytes(const go2p_handle* h, bool resident, bool* weights_fit) {
   const int XW = b1_xw(std::max(h->dm.max_width, h->n_in_slots));
@@ -401,7 +405,7 @@ int b1_dispatch(go2p_handle* h) {
     if (!h->graph_exec) {
       bool fit;
       const size_t smem = b1_smem_bytes(h, false, &fit);
-      CU_TRY(cudaFuncSetAttribute(b1_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      CU_TRY(opt_in_smem(h, reinterpret_cast<const void*>(b1_kernel<false>), smem));
       B1Args a = make_b1_args(h, false);
       CU_TRY(cudaStreamBeginCapture(h->b1_stream, cudaStreamCaptureModeThreadLocal));
       b1_kernel<false><<<1, kB1Threads, smem, h->b1_stream>>>(a);
@@ -413,10 +417,7 @@ int b1_dispatch(go2p_handle* h) {
   }
   bool fit;
   const size_t smem = b1_smem_bytes(h, false, &fit);
-  if (!h->b1_attr_set) {
-    CU_TRY(cudaFuncSetAttribute(b1_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    h->b1_attr_set = true;
-  }
+  CU_TRY(opt_in_smem(h, reinterpret_cast<const void*>(b1_kernel<false>), smem));
   B1Args a = make_b1_args(h, false);
   b1_kernel<false><<<1, kB1Threads, smem, h->b1_stream>>>(a);
   CU_TRY(cudaGetLastError());
@@ -473,10 +474,7 @@ int launch_fp32(go2p_handle* h, int set, const float* d_obs, const int32_t* d_bu
       // wider ones take the generic GEMM + the elementwise A9/A11 kernel
       const size_t so_smem = ((size_t)kSoRows * (L.K | 1) + (size_t)L.N * L.Kp) * sizeof(float);
       if (last && L.N <= 32 && so_smem <= (size_t)227 * 1024) {
-        if (h->so_attr_smem < so_smem) {
-          CU_TRY(cudaFuncSetAttribute(small_out_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)so_smem));
-          h->so_attr_smem = so_smem;
-        }
+        CU_TRY(opt_in_smem(h, reinterpret_cast<const void*>(small_out_kernel), so_smem));
         small_out_kernel<<<(unsigned)((rows + kSoRows - 1) / kSoRows), kSoRows, so_smem, st>>>(
             in, lda, L.w_rm, L.Kp, L.bias, out, ldc, rows, L.K, L.N, L.has_elu, L.alpha, flags,
             d_button0 ? d_button0 + r0 : nullptr, d_qdes ? d_qdes + r0 * kDof : nullptr, d_cmd ? d_cmd + r0 : nullptr, h->cc);
@@ -507,12 +505,7 @@ template <bool kFp16, bool kFused, bool kReset = false, bool kFields = false, bo
 int launch_tc_t(go2p_handle* h, const TcArgs& a, cudaStream_t st) {
   const size_t smem = tc_smem_bytes(a);
   auto kernel = tc_mlp_kernel<kFp16, kFused, kReset, kFields, kSeq>;
-  // the opt-in is a per-device function attribute: remembered per handle (one handle = one device)
-  size_t& configured = h->tc_attr_smem[(kFp16 ? 1 : 0) + (kFused ? 2 : 0) + (kReset ? 2 : 0) + (kFields ? 4 : 0) + (kSeq ? 4 : 0)];
-  if (configured != smem) {
-    CU_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    configured = smem;
-  }
+  CU_TRY(opt_in_smem(h, reinterpret_cast<const void*>(kernel), smem));
   const long long tiles = (a.B + kTcTileM - 1) / kTcTileM;
   int grid = (int)std::min<long long>(tiles, h->sm_count - (h->resident ? 1 : 0));
   // programmatic stream serialization: the kernel's prologue may overlap the tail of the previous kernel of the stream
@@ -825,8 +818,7 @@ int go2p_persistent_start(go2p_handle* h) {
   bool fit = false;
   const size_t smem = b1_smem_bytes(h, true, &fit);
   const bool regs = b1_regs_ok(h);
-  if (regs) CU_TRY(cudaFuncSetAttribute(b1_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  else CU_TRY(cudaFuncSetAttribute(b1_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  CU_TRY(opt_in_smem(h, regs ? reinterpret_cast<const void*>(b1_kernel<true, true>) : reinterpret_cast<const void*>(b1_kernel<true, false>), smem));
   ++h->epoch;
   B1Args a = make_b1_args(h, fit);
   if (regs) b1_kernel<true, true><<<1, kB1Threads, smem, h->b1_stream>>>(a);
@@ -968,8 +960,7 @@ int go2p_b1_selfdriven(go2p_handle* h, const go2p_raw_state* raws, int n_raws, i
     init.kp = h->cfg.kp; init.kd = h->cfg.kd;
     CU_TRY(cudaMemcpy(d_st, &init, sizeof(init), cudaMemcpyHostToDevice));
     CU_TRY(cudaMemcpy(d_raws, words.data(), words.size() * 4, cudaMemcpyHostToDevice));
-    if (regs) CU_TRY(cudaFuncSetAttribute(b1_selfdriven_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    else CU_TRY(cudaFuncSetAttribute(b1_selfdriven_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CU_TRY(opt_in_smem(h, regs ? reinterpret_cast<const void*>(b1_selfdriven_kernel<true>) : reinterpret_cast<const void*>(b1_selfdriven_kernel<false>), smem));
     B1Args a = make_b1_args(h, true);
     a.gstate = d_st;
     CU_TRY(cudaEventCreate(&e0));
@@ -1028,8 +1019,9 @@ int launch_wide(go2p_handle* h, go2p_handle::Scratch& sc, WdOperands operands, c
   if (ensure_scratch(h, sc, wide_act_rows(B), pieces * h->wide.max_kp * sizeof(uint16_t)))
     return fail(GO2P_ERR_CUDA, "wide_launch: cudaMalloc of the activation buffers failed");
   uint16_t* const act[2] = {static_cast<uint16_t*>(sc.buf[0]), static_cast<uint16_t*>(sc.buf[1])};
-  int rc = wide_launch(h->wide, act, d_obs, d_button0, d_act, d_qdes, cmd, B, operands, flags, h->cc, h->sm_count,
-                       h->split_attr_smem, st, &h->last_launches, g_err);
+  auto opt_in = [h](const void* fn, size_t bytes) { return opt_in_smem(h, fn, bytes); };
+  int rc = wide_launch(h->wide, act, d_obs, d_button0, d_act, d_qdes, cmd, B, operands, flags, h->cc, h->sm_count, opt_in, st,
+                       &h->last_launches, g_err);
   return rc ? fail(rc, g_err.c_str()) : GO2P_OK;
 }
 

@@ -261,7 +261,7 @@ __device__ __forceinline__ void b1_layer_n128(const float4* __restrict__ w4, con
 struct B1RegWeights {
   float4 w0[7], w1[8], w2[8], w3;
 
-  __device__ __forceinline__ static bool supported(const DevModel& m) {
+  __host__ __device__ __forceinline__ static bool supported(const DevModel& m) {
     return m.n_layers == 4 && m.L[0].N == 128 && m.L[1].N == 128 && m.L[2].N == 128 && m.L[1].K == 128 && m.L[2].K == 128 &&
            m.L[3].K == 128 && m.L[3].N <= 16 && m.L[0].Kp <= 112;
   }

@@ -269,19 +269,16 @@ enum : int {
   kEluMax = 2,      // max.NaN(z', e') (one HMNMX2): 0 <= alpha <= 1, where c*(2^z' - 1) >= z' for every z' <= 0
 };
 
+// bit j: column pair j of a warp's 16 per job takes the FMA-pipe exponential (4 of 16; DESIGN.md §3.2 lists every mask
+// measured)
+constexpr uint32_t kTcPolyMask = 0xC0C0u;
+
 // ELU of 16 accumulator columns -> 8 packed words.  fp16: every pair stays packed -- F2FP (pack z'), then either
 // ex2.approx.f16x2 of -|z'| (2 MUFU with the -|.| source modifier + PRMT) + HFMA2 (c*e - c) or, for the pairs in kMask,
 // the FMA-pipe polynomial above; then the select.  kEluMax is exact: for z' > 0, e' < 0 < z'; for z' <= 0, e' is the
 // ELU, which is >= z' when alpha <= 1 (where rounding puts the computed e' below z', z' is the closer of the two to the
 // true value); max.NaN keeps a NaN input NaN.  bf16: the fp32 exponential of -|z| (its budget has no room for the fp16
 // one) and the same select in bf16x2.  c2, ch2, nc2: c, c/2 and -c as packed fp16 pairs.
-#ifndef GO2P_TC_WARM_L2
-#define GO2P_TC_WARM_L2 1
-#endif
-#ifndef GO2P_TC_POLYMASK
-#define GO2P_TC_POLYMASK 0xC0C0u   // bit j: column pair j of a warp's 16 per job takes the FMA-pipe exponential (4 of 16)
-#endif
-
 template <bool kFp16, int kElu, uint32_t kMask>
 __device__ __forceinline__ void elu_pack16(const uint32_t (&v)[16], float c, uint32_t c2, uint32_t ch2, uint32_t nc2, uint32_t (&p)[8]) {
   const float nc = -c;
@@ -317,8 +314,8 @@ template <bool kFp16, int kElu>
 __device__ __forceinline__ void elu_pack32_sel(const uint32_t (&v0)[16], const uint32_t (&v1)[16], float c, uint32_t c2, uint32_t ch2,
                                                uint32_t nc2, uint32_t (&p)[16]) {
   uint32_t p0[8], p1[8];
-  elu_pack16<kFp16, kElu, (GO2P_TC_POLYMASK & 0xFFu)>(v0, c, c2, ch2, nc2, p0);
-  elu_pack16<kFp16, kElu, ((GO2P_TC_POLYMASK >> 8) & 0xFFu)>(v1, c, c2, ch2, nc2, p1);
+  elu_pack16<kFp16, kElu, (kTcPolyMask & 0xFFu)>(v0, c, c2, ch2, nc2, p0);
+  elu_pack16<kFp16, kElu, ((kTcPolyMask >> 8) & 0xFFu)>(v1, c, c2, ch2, nc2, p1);
 #pragma unroll
   for (int j = 0; j < 8; ++j) { p[j] = p0[j]; p[8 + j] = p1[j]; }
 }
@@ -461,7 +458,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
   // host launches the first tensor-core kernel after a weight update (go2p_set_weights) on the update's stream without
   // programmatic serialization (capi.cu: launch_tc_t).  The next launch may start its own prologue as soon as
   // this CTA's SM is free (a short batch per GPU, e.g. 1/8 of a sharded step, is otherwise launch-gap bound).
-#if GO2P_TC_WARM_L2
   // While the previous kernel drains, pull this CTA's first two observation slabs into L2 (prefetch only: L2 is the
   // point of coherence, so a line the previous kernel still rewrites is simply updated there).  Matters for short
   // launches -- 1/8 of a sharded step is 7 tiles per CTA, and the first slab's HBM latency is part of every launch.
@@ -476,7 +472,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_mlp_kernel(const __grid_cons
       for (long long i = tid; i < lim; i += blockDim.x) ptx::prefetch_l2(base + i * 128);
     }
   }
-#endif
   ptx::grid_dependency_wait();
   ptx::grid_launch_dependents();
 

@@ -20,8 +20,6 @@
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
-#include <cstdio>
-#include <cstdlib>
 #include <string>
 #include <vector>
 
@@ -34,19 +32,15 @@ namespace go2p {
 constexpr int kWdTileM = 128;
 constexpr int kWdChunkK = 64;                       // K columns per pipeline stage (4 MMA K steps)
 constexpr int kWdATileBytes = kWdTileM * kWdChunkK * 2;   // 16 KB
-constexpr int kWdStages = 4;                        // 4 x 48 KB (N tile 256) = 192 KB of operands in flight per SM
 // operand ring depth: as many stages as fit in ~192 KB (the L2 round trip under load is ~4,000 cycles, so the bytes in
 // flight, not the stage count, set the delivered bandwidth), at most 8.  split: a stage holds three bf16 pieces of each
 // operand (GO2P_PREC_FP32_TC)
-__host__ __device__ constexpr int wd_stages(int nt, bool pair, bool split = false) {
-  const int stage = (split ? 3 : 1) * (128 * 64 * 2 + (pair ? nt / 2 : nt) * 64 * 2);
+__host__ __device__ constexpr int wd_stages(int nt, bool split) {
+  const int stage = (split ? 3 : 1) * (128 * 64 * 2 + nt * 64 * 2);
   const int n = (192 * 1024) / stage;
   return n > 8 ? 8 : n;
 }
-#ifndef GO2P_WD_EPI_WARPS
-#define GO2P_WD_EPI_WARPS 16
-#endif
-constexpr int kWdEpiWarps = GO2P_WD_EPI_WARPS;      // kWdEpiWarps/4 per TMEM lane quarter, each takes a share of the tile's columns
+constexpr int kWdEpiWarps = 16;                     // kWdEpiWarps/4 per TMEM lane quarter, each takes a share of the tile's columns
 constexpr int kWdEpiParts = kWdEpiWarps / 4;
 constexpr int kWdThreads = (2 + kWdEpiWarps) * 32;  // producer, MMA issuer, epilogue warps
 
@@ -184,32 +178,18 @@ __global__ void obs_to_blocked_kernel(const float* __restrict__ obs, uint16_t* _
   }
 }
 
-// kCS = thread-block cluster size (1 or 2).  With kCS = 2 the two CTAs of a cluster work on neighbouring row tiles of
-// the SAME N tile: each loads its own A tile and HALF of the weight tile, which the TMA engine multicasts into both
-// CTAs' shared memory -- the weight tile crosses the L2 -> SM fabric once per cluster instead of once per CTA (32 KB
-// instead of 48 KB of operand traffic per CTA and K chunk at NT = 256).  A stage is refilled only when the MMAs of
-// BOTH CTAs have read it: tcgen05.commit arrives on the stage's empty barrier of every CTA in the cluster.
-// kCS = 2 with kPair: the two CTAs form a CTA PAIR (tcgen05 cta_group::2).  One M256 x NT MMA spans both SMs: each CTA
-// holds its own 128-row A tile and HALF of the weight tile (NT/2 rows), so an SM takes in 32 KB instead of 48 KB per K
-// chunk at NT = 256 -- the remedy for the L2 -> SM intake limit of the single-CTA tile.  The leader (rank 0) issues the
-// MMAs once its own and the peer's stage have landed (the peer relays its full-barrier to the leader), and its
-// tcgen05.commit releases stages and publishes accumulators in both CTAs; both CTAs' epilogue warps report the drained
-// accumulator to the leader.
-//
-// kSplit (GO2P_PREC_FP32_TC, single CTA, bf16): a and w are split tile groups (wd_split_act / wd_split_weight).  A stage
+// kSplit (GO2P_PREC_FP32_TC, bf16): a and w are split tile groups (wd_split_act / wd_split_weight).  A stage
 // holds the three A pieces and the three B pieces of one K chunk, and per K16 step the MMA warp issues the six products
 // whose size is at least 2^-16 of the leading term from that one stage: hi*hi into the main accumulator, hi*mid,
 // mid*hi, hi*lo, lo*hi, mid*mid into a second one (the dropped mid*lo, lo*mid, lo*lo are <= 2^-23 relative).  The
 // epilogue adds the two accumulators, then the bias in fp32; a hidden layer stores the three pieces of its output.
-template <int NT, bool kFp16, int kCS, bool kPair = false, bool kSplit = false>
+template <int NT, bool kFp16, bool kSplit = false>
 __global__ void __launch_bounds__(kWdThreads, 1) wide_gemm_kernel(const WideGemmArgs a) {
-  static_assert(!kPair || kCS == 2, "a CTA pair is a cluster of two");
-  static_assert(!kSplit || (kCS == 1 && !kFp16 && NT <= 128), "the split operands are bf16, one CTA per tile, N tile <= 128");
+  static_assert(!kSplit || (!kFp16 && NT <= 128), "the split operands are bf16, N tile <= 128");
   extern __shared__ __align__(128) uint8_t smem[];
   constexpr int kBTileBytes = NT * kWdChunkK * 2;
-  constexpr int kStageBytes = kSplit ? 3 * (kWdATileBytes + kBTileBytes)
-                                     : kWdATileBytes + (kPair ? kBTileBytes / 2 : kBTileBytes);   // pair: half of the weight tile per CTA
-  constexpr int kStages = wd_stages(NT, kPair, kSplit);
+  constexpr int kStageBytes = (kSplit ? 3 : 1) * (kWdATileBytes + kBTileBytes);
+  constexpr int kStages = wd_stages(NT, kSplit);
   constexpr uint32_t kAccCols = NT < 32 ? 32 : NT;               // TMEM columns per accumulator
   constexpr uint32_t kAccs = kSplit ? 2 : 1;                     // accumulators per buffer
   constexpr uint32_t kTmemCols = 2 * kAccs * kAccCols;           // 64 .. 512, a power of two
@@ -219,25 +199,19 @@ __global__ void __launch_bounds__(kWdThreads, 1) wide_gemm_kernel(const WideGemm
   uint64_t* empty = bars + kStages;    // [kStages] chunk consumed by the tensor core
   uint64_t* acc_full = bars + 2 * kStages;       // [2]
   uint64_t* acc_empty = bars + 2 * kStages + 2;  // [2]
-  uint64_t* peer_full = bars + 2 * kStages + 4;  // [kStages] leader only: the peer's chunk landed
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bars + 3 * kStages + 4);
+  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bars + 2 * kStages + 4);
 
   if (warp == 1) {
     if (lane == 0) {
-      for (int s = 0; s < kStages; ++s) {
-        ptx::mbar_init(&full[s], 1);
-        ptx::mbar_init(&empty[s], kPair ? 1 : kCS);      // pair: one multicast commit of the leader; multicast: one per CTA
-        ptx::mbar_init(&peer_full[s], 1);
-      }
-      for (int b = 0; b < 2; ++b) { ptx::mbar_init(&acc_full[b], 1); ptx::mbar_init(&acc_empty[b], (kPair ? 2 : 1) * kWdEpiWarps); }
+      for (int s = 0; s < kStages; ++s) { ptx::mbar_init(&full[s], 1); ptx::mbar_init(&empty[s], 1); }
+      for (int b = 0; b < 2; ++b) { ptx::mbar_init(&acc_full[b], 1); ptx::mbar_init(&acc_empty[b], kWdEpiWarps); }
       ptx::fence_mbar_init();
     }
     __syncwarp();
-    if (kPair) ptx::tmem_alloc_pair<kTmemCols>(tmem_ptr); else ptx::tmem_alloc<kTmemCols>(tmem_ptr);
+    ptx::tmem_alloc<kTmemCols>(tmem_ptr);
   }
   ptx::tc_fence_before();
   block_sync();
-  if (kCS > 1) ptx::cluster_sync_all();     // the peer's barriers exist before anything is multicast into them
   ptx::tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
   // Programmatic dependent launch: barriers and TMEM are set up while the previous layer's launch drains; its
@@ -250,21 +224,16 @@ __global__ void __launch_bounds__(kWdThreads, 1) wide_gemm_kernel(const WideGemm
   ptx::grid_dependency_wait();
   ptx::grid_launch_dependents();
 
-  // job = (group of kCS row tiles, N tile), N tile fastest: the A tiles stay in L2 for the next N tile.
-  // Every CTA of a cluster walks the same job list; CTA rank r takes row tile group*kCS + r.  A rank whose row tile
-  // does not exist (odd tile count) still loads and multiplies a clamped tile -- its half of the weights is needed by
-  // the peer -- and only skips the stores.
-  const uint32_t crank = kCS > 1 ? ptx::cluster_ctarank() : 0u;
-  const long long job0 = kCS > 1 ? (long long)ptx::cluster_id_x() : (long long)blockIdx.x;
-  const long long job_stride = kCS > 1 ? (long long)ptx::cluster_nctaid_x() : (long long)gridDim.x;
-  const long long m_groups = (a.m_tiles + kCS - 1) / kCS;
-  const long long n_jobs = m_groups * a.n_tiles;
-  auto job_mt = [&](long long job) { return (job / a.n_tiles) * kCS + crank; };
+  // job = (row tile, N tile), N tile fastest: the A tiles stay in L2 for the next N tile.  job < m_tiles * n_tiles, so
+  // mt < m_tiles: the producer's clamp and the epilogue's row-tile test below are redundant.  They stay because without
+  // them ptxas schedules the epilogues differently (other register counts), and this is the code DESIGN.md §3.3b measured.
+  const long long job0 = blockIdx.x, job_stride = gridDim.x;
+  const long long n_jobs = (long long)a.m_tiles * a.n_tiles;
   if (warp == 0) {
     // ================= producer =================
     uint32_t it = 0;
     for (long long job = job0; job < n_jobs; job += job_stride) {
-      const long long mt = min(job_mt(job), (long long)a.m_tiles - 1);
+      const long long mt = min(job / a.n_tiles, (long long)a.m_tiles - 1);
       const int nt = (int)(job % a.n_tiles);
       for (int kc = 0; kc < a.k_chunks; ++kc, ++it) {
         const int s = it % kStages;
@@ -286,88 +255,64 @@ __global__ void __launch_bounds__(kWdThreads, 1) wide_gemm_kernel(const WideGemm
         }
         if (ptx::elect_one_sync()) {
           uint8_t* st = smem + s * kStageBytes;
-          ptx::mbar_arrive_expect_tx(&full[s], (uint32_t)(kPair ? kWdATileBytes + kBTileBytes / 2 : kStageBytes));
+          ptx::mbar_arrive_expect_tx(&full[s], (uint32_t)kStageBytes);
           ptx::bulk_g2s(st, reinterpret_cast<const uint8_t*>(a.a) + (mt * a.k_chunks + kc) * (long long)kWdATileBytes, kWdATileBytes, &full[s]);
           const uint8_t* wsrc = reinterpret_cast<const uint8_t*>(a.w) + ((long long)nt * a.k_chunks + kc) * (long long)kBTileBytes;
-          if (kPair) {
-            // this CTA's NT/2 rows of the weight tile, at the same shared-memory offset in both CTAs
-            ptx::bulk_g2s(st + kWdATileBytes, wsrc + crank * (kBTileBytes / 2), kBTileBytes / 2, &full[s]);
-          } else if (kCS > 1) {
-            constexpr uint32_t kPart = kBTileBytes / kCS;     // whole 8-row groups: a contiguous slice of the tile
-            ptx::bulk_g2s_multicast(st + kWdATileBytes + crank * kPart, wsrc + crank * kPart, kPart, &full[s], (uint16_t)((1u << kCS) - 1u));
-          } else {
-            ptx::bulk_g2s(st + kWdATileBytes, wsrc, kBTileBytes, &full[s]);
-          }
+          ptx::bulk_g2s(st + kWdATileBytes, wsrc, kBTileBytes, &full[s]);
         }
         __syncwarp();
       }
     }
   } else if (warp == 1) {
-    // ================= MMA issuer (pair mode: leader only; the peer's warp relays its full barriers) =================
-    const uint32_t idesc = ptx::make_idesc(kFp16 ? ptx::FMT_F16 : ptx::FMT_BF16, kPair ? 2 * kWdTileM : kWdTileM, (uint32_t)NT);
+    // ================= MMA issuer =================
+    const uint32_t idesc = ptx::make_idesc(kFp16 ? ptx::FMT_F16 : ptx::FMT_BF16, kWdTileM, (uint32_t)NT);
     uint32_t it = 0, tile_i = 0;
-    if (kPair && crank != 0) {
-      for (long long job = job0; job < n_jobs; job += job_stride)
-        for (int kc = 0; kc < a.k_chunks; ++kc, ++it) {
-          const int s = it % kStages;
-          ptx::mbar_wait(&full[s], (it / kStages) & 1u);
-          if (lane == 0) ptx::mbar_arrive_cluster(&peer_full[s], 0u);
-          __syncwarp();
-        }
-    } else {
-      for (long long job = job0; job < n_jobs; job += job_stride, ++tile_i) {
-        const uint32_t buf = tile_i & 1u;
-        ptx::mbar_wait(&acc_empty[buf], ((tile_i >> 1) & 1u) ^ 1u);
+    for (long long job = job0; job < n_jobs; job += job_stride, ++tile_i) {
+      const uint32_t buf = tile_i & 1u;
+      ptx::mbar_wait(&acc_empty[buf], ((tile_i >> 1) & 1u) ^ 1u);
+      ptx::tc_fence_after();
+      const uint32_t d_t = tmem_base + buf * kAccs * kAccCols;
+      for (int kc = 0; kc < a.k_chunks; ++kc, ++it) {
+        const int s = it % kStages;
+        ptx::mbar_wait(&full[s], (it / kStages) & 1u);
         ptx::tc_fence_after();
-        const uint32_t d_t = tmem_base + buf * kAccs * kAccCols;
-        for (int kc = 0; kc < a.k_chunks; ++kc, ++it) {
-          const int s = it % kStages;
-          ptx::mbar_wait(&full[s], (it / kStages) & 1u);
-          if (kPair) ptx::mbar_wait(&peer_full[s], (it / kStages) & 1u);
-          ptx::tc_fence_after();
-          if constexpr (kSplit) {
-            if (ptx::elect_one_sync()) {
-              const uint32_t sa = ptx::smem_u32(smem + s * kStageBytes);
-              uint64_t ad[3], bd[3];
-#pragma unroll
-              for (int q = 0; q < 3; ++q) {
-                ad[q] = ptx::make_smem_desc_nosw(sa + q * kWdATileBytes, 128u, 1024u);
-                bd[q] = ptx::make_smem_desc_nosw(sa + 3 * kWdATileBytes + q * kBTileBytes, 128u, 1024u);
-              }
-#pragma unroll
-              for (int j = 0; j < kWdChunkK / 16; ++j) {
-                const uint64_t o = (uint64_t)(j * 16);
-                const uint32_t acc = (kc | j) ? 1u : 0u;
-                ptx::mma_f16_ss(d_t, ad[0] + o, bd[0] + o, idesc, acc);                 // hi * hi
-                ptx::mma_f16_ss(d_t + kAccCols, ad[0] + o, bd[1] + o, idesc, acc);      // hi * mid
-                ptx::mma_f16_ss(d_t + kAccCols, ad[1] + o, bd[0] + o, idesc, 1u);       // mid * hi
-                ptx::mma_f16_ss(d_t + kAccCols, ad[0] + o, bd[2] + o, idesc, 1u);       // hi * lo
-                ptx::mma_f16_ss(d_t + kAccCols, ad[2] + o, bd[0] + o, idesc, 1u);       // lo * hi
-                ptx::mma_f16_ss(d_t + kAccCols, ad[1] + o, bd[1] + o, idesc, 1u);       // mid * mid
-              }
-              ptx::mma_commit(&empty[s]);
-              if (kc == a.k_chunks - 1) ptx::mma_commit(&acc_full[buf]);
-            }
-            __syncwarp();
-            continue;
-          }
+        if constexpr (kSplit) {
           if (ptx::elect_one_sync()) {
             const uint32_t sa = ptx::smem_u32(smem + s * kStageBytes);
-            const uint64_t adesc = ptx::make_smem_desc_nosw(sa, 128u, 1024u);
-            const uint64_t bdesc = ptx::make_smem_desc_nosw(sa + kWdATileBytes, 128u, 1024u);
+            uint64_t ad[3], bd[3];
+#pragma unroll
+            for (int q = 0; q < 3; ++q) {
+              ad[q] = ptx::make_smem_desc_nosw(sa + q * kWdATileBytes, 128u, 1024u);
+              bd[q] = ptx::make_smem_desc_nosw(sa + 3 * kWdATileBytes + q * kBTileBytes, 128u, 1024u);
+            }
 #pragma unroll
             for (int j = 0; j < kWdChunkK / 16; ++j) {
-              if (kPair) ptx::mma_f16_ss_pair(d_t, adesc + (uint64_t)(j * 16), bdesc + (uint64_t)(j * 16), idesc, (kc | j) ? 1u : 0u);
-              else ptx::mma_f16_ss(d_t, adesc + (uint64_t)(j * 16), bdesc + (uint64_t)(j * 16), idesc, (kc | j) ? 1u : 0u);
+              const uint64_t o = (uint64_t)(j * 16);
+              const uint32_t acc = (kc | j) ? 1u : 0u;
+              ptx::mma_f16_ss(d_t, ad[0] + o, bd[0] + o, idesc, acc);                 // hi * hi
+              ptx::mma_f16_ss(d_t + kAccCols, ad[0] + o, bd[1] + o, idesc, acc);      // hi * mid
+              ptx::mma_f16_ss(d_t + kAccCols, ad[1] + o, bd[0] + o, idesc, 1u);       // mid * hi
+              ptx::mma_f16_ss(d_t + kAccCols, ad[0] + o, bd[2] + o, idesc, 1u);       // hi * lo
+              ptx::mma_f16_ss(d_t + kAccCols, ad[2] + o, bd[0] + o, idesc, 1u);       // lo * hi
+              ptx::mma_f16_ss(d_t + kAccCols, ad[1] + o, bd[1] + o, idesc, 1u);       // mid * mid
             }
-            // frees the stage (in every CTA of the cluster) when these MMAs have read it
-            if (kPair) ptx::mma_commit_pair(&empty[s], 3);
-            else if (kCS > 1) ptx::mma_commit_multicast(&empty[s], (uint16_t)((1u << kCS) - 1u));
-            else ptx::mma_commit(&empty[s]);
-            if (kc == a.k_chunks - 1) { if (kPair) ptx::mma_commit_pair(&acc_full[buf], 3); else ptx::mma_commit(&acc_full[buf]); }
+            ptx::mma_commit(&empty[s]);
+            if (kc == a.k_chunks - 1) ptx::mma_commit(&acc_full[buf]);
           }
           __syncwarp();
+          continue;
         }
+        if (ptx::elect_one_sync()) {
+          const uint32_t sa = ptx::smem_u32(smem + s * kStageBytes);
+          const uint64_t adesc = ptx::make_smem_desc_nosw(sa, 128u, 1024u);
+          const uint64_t bdesc = ptx::make_smem_desc_nosw(sa + kWdATileBytes, 128u, 1024u);
+#pragma unroll
+          for (int j = 0; j < kWdChunkK / 16; ++j)
+            ptx::mma_f16_ss(d_t, adesc + (uint64_t)(j * 16), bdesc + (uint64_t)(j * 16), idesc, (kc | j) ? 1u : 0u);
+          ptx::mma_commit(&empty[s]);                  // frees the stage when these MMAs have read it
+          if (kc == a.k_chunks - 1) ptx::mma_commit(&acc_full[buf]);
+        }
+        __syncwarp();
       }
     }
   } else {
@@ -378,15 +323,15 @@ __global__ void __launch_bounds__(kWdThreads, 1) wide_gemm_kernel(const WideGemm
     const int r = quarter * 32 + lane;               // row inside the tile
     uint32_t tile_i = 0;
     for (long long job = job0; job < n_jobs; job += job_stride, ++tile_i) {
-      const long long mt = job_mt(job);
-      const bool ghost = mt >= a.m_tiles;              // clamped duplicate of the last row tile: no stores
+      const long long mt = job / a.n_tiles;
+      const bool past_end = mt >= a.m_tiles;           // never true (see the job mapping above)
       const int nt = (int)(job % a.n_tiles);
       const uint32_t buf = tile_i & 1u;
       ptx::mbar_wait(&acc_full[buf], (tile_i >> 1) & 1u);
       ptx::tc_fence_after();
       const uint32_t acc_t = tmem_base + buf * kAccs * kAccCols + lane_addr;
       const long long row = mt * kWdTileM + r;
-      if (ghost) {
+      if (past_end) {
         // nothing to store; the accumulator is simply released
       } else if (kSplit && a.out_blocked) {
         if constexpr (kSplit) {   // discarded in the 16-bit instantiations, whose code stays as it was
@@ -522,16 +467,15 @@ __global__ void __launch_bounds__(kWdThreads, 1) wide_gemm_kernel(const WideGemm
       }
       ptx::tc_fence_before();
       __syncwarp();
-      if (lane == 0) { if (kPair) ptx::mbar_arrive_cluster(&acc_empty[buf], 0u); else ptx::mbar_arrive(&acc_empty[buf]); }
+      if (lane == 0) ptx::mbar_arrive(&acc_empty[buf]);
     }
   }
 
   ptx::tc_fence_before();
   block_sync();
-  if (kCS > 1) ptx::cluster_sync_all();     // no CTA leaves while the peer may still multicast into it or arrive on its barriers
   if (warp == 1) {
     ptx::tc_fence_after();
-    if (kPair) ptx::tmem_dealloc_pair<kTmemCols>(tmem_base); else ptx::tmem_dealloc<kTmemCols>(tmem_base);
+    ptx::tmem_dealloc<kTmemCols>(tmem_base);
   }
 }
 
@@ -618,86 +562,14 @@ inline int wide_prepare(const MlpModel& m, Alloc&& alloc, WideModel* wm, bool im
   return 0;
 }
 
-// Launch mode of the GEMM kernels: 1 = one CTA per tile (default), 2 = cluster of two with TMA multicast of the weight
-// tile, 3 = CTA pair (tcgen05 cta_group::2, M256 tiles).  All three pass the same tests.  Measured on B200
-// (scripts/gpu_wide_variants.sh, 606,208 rows, round-1 pass size): 1: 2.25 ms, 2: 2.41 ms, 3: 3.19 ms.  ncu: mode 3
-// does cut the L2 -> SM bytes by a third (233 -> 155 MB in layer 2) but its MMAs retire at a quarter of the single-CTA
-// rate -- the leader/peer hand-offs (full-barrier relay, multicast commits) sit in the per-chunk critical path, and a
-// 1-D bulk copy cannot complete on the peer CTA's barrier.  Modes 2 and 3 are kept as measured build options.
-#ifndef GO2P_WD_CLUSTER
-#define GO2P_WD_CLUSTER 1
-#endif
-
-template <int NT, bool kFp16>
-inline cudaError_t wd_launch_gemm(const WideGemmArgs& a, int sm_count, cudaStream_t st) {
-  constexpr int kCS = GO2P_WD_CLUSTER == 3 ? 2 : GO2P_WD_CLUSTER;      // 3 = CTA pair (cta_group::2)
-  constexpr bool kPair = GO2P_WD_CLUSTER == 3;
-  const size_t smem = (size_t)wd_stages(NT, kPair) * (kWdATileBytes + (kPair ? NT / 2 : NT) * kWdChunkK * 2) + 256;
-  auto kernel = wide_gemm_kernel<NT, kFp16, kCS, kPair>;
-  static thread_local int configured_dev = -1;           // the attribute is per device and per function
-  static thread_local int max_clusters = 0;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  cudaLaunchConfig_t cfg = {};
-  cudaLaunchAttribute attr[2];
-  cfg.blockDim = dim3(kWdThreads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;      // see griddepcontrol.wait in the kernel
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  if (kCS > 1) {
-    attr[1].id = cudaLaunchAttributeClusterDimension;
-    attr[1].val.clusterDim.x = kCS; attr[1].val.clusterDim.y = 1; attr[1].val.clusterDim.z = 1;
-    cfg.numAttrs = 2;
-  }
-  if (configured_dev != dev) {
-    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    max_clusters = sm_count / kCS;
-    if (kCS > 1) {
-      cfg.gridDim = dim3((unsigned)(sm_count / kCS * kCS));
-      int n = 0;
-      e = cudaOccupancyMaxActiveClusters(&n, kernel, &cfg);   // clusters that can be co-resident (GPC boundaries)
-      if (e != cudaSuccess) return e;
-      if (n > 0 && n < max_clusters) max_clusters = n;
-      if (std::getenv("GO2P_DEBUG")) fprintf(stderr, "wide_gemm<%d>: %d co-resident clusters of %d (of %d SMs)\n", NT, n, kCS, sm_count);
-    }
-    configured_dev = dev;
-  }
-  const long long jobs = ((long long)a.m_tiles + kCS - 1) / kCS * a.n_tiles;
-  const long long groups = std::min<long long>(jobs, (long long)max_clusters);
-  cfg.gridDim = dim3((unsigned)(groups * kCS));
-  return cudaLaunchKernelEx(&cfg, kernel, a);
-}
-
-// rows per pass: a multiple of 148 row tiles, so every layer's job count is a whole number of waves over the 148 SMs.
-// Round 1 used ONE wave of row tiles (18,944 rows: the widest activation, 39 MB, stays in the 126 MB L2); measured in
-// round 2 (scripts/gpu_wide_variants.sh, 606,208 rows, fp16 / bf16): 1 wave 1.86 / 1.85 ms, 2 waves 1.62 / 1.66 ms,
-// 4 waves 1.57 / 1.51 ms, 32 waves (the whole batch) 1.54 / 1.48 ms -- the five launches per pass each end in a tail
-// (layers 3 and 4 are ONE job per CTA at one wave: no overlap of epilogue and MMAs at all), and that costs more than
-// reading the activations back from HBM instead of L2.  Four waves: 75,776 rows, 155 MB per activation buffer.
-#ifndef GO2P_WD_PASS_WAVES
-#define GO2P_WD_PASS_WAVES 4
-#endif
-constexpr long long kWdChunkRows = 148 * kWdTileM * GO2P_WD_PASS_WAVES;
-
-// rows of one pass of wide_launch over B rows, in whole row tiles
-inline long long wide_act_rows(long long B) {
-  return (std::min<long long>(B, kWdChunkRows) + kWdTileM - 1) / kWdTileM * kWdTileM;
-}
-
-// The split GEMMs (GO2P_PREC_FP32_TC).  configured: the dynamic shared memory this handle has opted the instantiation
-// in to on its device (the attribute is per device and per function; one handle = one device).
-template <int NT>
-inline cudaError_t wd_launch_split(const WideGemmArgs& a, int sm_count, size_t& configured, cudaStream_t st) {
-  const size_t smem = (size_t)wd_stages(NT, false, true) * 3 * (kWdATileBytes + NT * kWdChunkK * 2) + 256;
-  auto kernel = wide_gemm_kernel<NT, false, 1, false, true>;
-  if (configured != smem) {
-    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    configured = smem;
-  }
+// One persistent CTA per SM (at most one per job).  opt_in(kernel, bytes) -> cudaError_t opts the kernel in to `bytes`
+// of dynamic shared memory on the current device.
+template <int NT, bool kFp16, bool kSplit, class OptIn>
+inline cudaError_t wd_launch(const WideGemmArgs& a, int sm_count, OptIn& opt_in, cudaStream_t st) {
+  const size_t smem = (size_t)wd_stages(NT, kSplit) * (kSplit ? 3 : 1) * (kWdATileBytes + NT * kWdChunkK * 2) + 256;
+  auto kernel = wide_gemm_kernel<NT, kFp16, kSplit>;
+  const cudaError_t e = opt_in(reinterpret_cast<const void*>(kernel), smem);
+  if (e != cudaSuccess) return e;
   cudaLaunchConfig_t cfg = {};
   cudaLaunchAttribute attr;
   attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;      // see griddepcontrol.wait in the kernel
@@ -711,14 +583,28 @@ inline cudaError_t wd_launch_split(const WideGemmArgs& a, int sm_count, size_t& 
   return cudaLaunchKernelEx(&cfg, kernel, a);
 }
 
+// rows per pass: a multiple of 148 row tiles, so every layer's job count is a whole number of waves over the 148 SMs.
+// Round 1 used ONE wave of row tiles (18,944 rows: the widest activation, 39 MB, stays in the 126 MB L2); measured in
+// round 2 (606,208 rows, fp16 / bf16): 1 wave 1.86 / 1.85 ms, 2 waves 1.62 / 1.66 ms,
+// 4 waves 1.57 / 1.51 ms, 32 waves (the whole batch) 1.54 / 1.48 ms -- the five launches per pass each end in a tail
+// (layers 3 and 4 are ONE job per CTA at one wave: no overlap of epilogue and MMAs at all), and that costs more than
+// reading the activations back from HBM instead of L2.  Four waves: 75,776 rows, 155 MB per activation buffer.
+constexpr long long kWdChunkRows = 148 * kWdTileM * 4;
+
+// rows of one pass of wide_launch over B rows, in whole row tiles
+inline long long wide_act_rows(long long B) {
+  return (std::min<long long>(B, kWdChunkRows) + kWdTileM - 1) / kWdTileM * kWdTileM;
+}
+
 // operand formats of wide_launch
 enum WdOperands { kWdBf16 = 0, kWdFp16 = 1, kWdSplit = 2 };
 
 // act: the two blocked activation buffers (ping-pong), each of wide_act_rows(B) rows x wm.max_kp 16-bit columns (three
-// times that for kWdSplit).  split_attr: the handle's opt-in record of the split instantiations (N tile 128, 64, 16).
+// times that for kWdSplit).  opt_in: see wd_launch.
+template <class OptIn>
 inline int wide_launch(const WideModel& wm, uint16_t* const act[2], const float* d_obs, const int32_t* d_button0, float* d_act, double* d_qdes,
                        MotorCmdDev* d_cmd, long long B, WdOperands operands, uint32_t flags, const CtrlConst& cc, int sm_count,
-                       size_t split_attr[3], cudaStream_t st, int* launches, std::string& err) {
+                       OptIn&& opt_in, cudaStream_t st, int* launches, std::string& err) {
   const bool fp16 = operands == kWdFp16, split = operands == kWdSplit;
   const long long chunk = std::min<long long>(B, kWdChunkRows);
   for (long long r0 = 0; r0 < B; r0 += chunk) {
@@ -760,13 +646,13 @@ inline int wide_launch(const WideModel& wm, uint16_t* const act[2], const float*
       for (int i = 0; i < kDof; ++i) a.q0[i] = cc.q0[i];
       cudaError_t e;
       if (split) {
-        if (NT == 128) e = wd_launch_split<128>(a, sm_count, split_attr[0], st);
-        else if (NT == 64) e = wd_launch_split<64>(a, sm_count, split_attr[1], st);
-        else e = wd_launch_split<16>(a, sm_count, split_attr[2], st);
-      } else if (L.NT == 256) e = fp16 ? wd_launch_gemm<256, true>(a, sm_count, st) : wd_launch_gemm<256, false>(a, sm_count, st);
-      else if (L.NT == 128) e = fp16 ? wd_launch_gemm<128, true>(a, sm_count, st) : wd_launch_gemm<128, false>(a, sm_count, st);
-      else if (L.NT == 64) e = fp16 ? wd_launch_gemm<64, true>(a, sm_count, st) : wd_launch_gemm<64, false>(a, sm_count, st);
-      else e = fp16 ? wd_launch_gemm<16, true>(a, sm_count, st) : wd_launch_gemm<16, false>(a, sm_count, st);
+        if (NT == 128) e = wd_launch<128, false, true>(a, sm_count, opt_in, st);
+        else if (NT == 64) e = wd_launch<64, false, true>(a, sm_count, opt_in, st);
+        else e = wd_launch<16, false, true>(a, sm_count, opt_in, st);
+      } else if (L.NT == 256) e = fp16 ? wd_launch<256, true, false>(a, sm_count, opt_in, st) : wd_launch<256, false, false>(a, sm_count, opt_in, st);
+      else if (L.NT == 128) e = fp16 ? wd_launch<128, true, false>(a, sm_count, opt_in, st) : wd_launch<128, false, false>(a, sm_count, opt_in, st);
+      else if (L.NT == 64) e = fp16 ? wd_launch<64, true, false>(a, sm_count, opt_in, st) : wd_launch<64, false, false>(a, sm_count, opt_in, st);
+      else e = fp16 ? wd_launch<16, true, false>(a, sm_count, opt_in, st) : wd_launch<16, false, false>(a, sm_count, opt_in, st);
       if (e != cudaSuccess) { err = std::string("wide_launch: ") + cudaGetErrorString(e); return 4; }
       ++*launches;
       cur ^= 1;

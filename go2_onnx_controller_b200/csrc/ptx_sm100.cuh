@@ -44,15 +44,6 @@ __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
 __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
-__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-  return ok != 0;
-}
 // non-blocking probe (try_wait may suspend the thread for a system-dependent time before answering "not yet":
 // measured ~1000+ cycles, which serialises a poller that watches several barriers)
 __device__ __forceinline__ bool mbar_test_wait(uint64_t* bar, uint32_t parity) {
@@ -85,23 +76,11 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
 // suspend-time hint of a blocking wait: a waiting warp sleeps in the barrier unit until the phase completes (it is woken
 // by the completing arrival) or this many nanoseconds pass, instead of re-polling every few hundred cycles -- the
 // re-polls of the warps that run ahead took issue slots from the warps they were waiting for
-#ifndef GO2P_MBAR_SUSPEND_NS
-#define GO2P_MBAR_SUSPEND_NS 4000
-#endif
-constexpr uint32_t kMbarSuspendNs = GO2P_MBAR_SUSPEND_NS;
+constexpr uint32_t kMbarSuspendNs = 4000;
 
 // the same operations on 32-bit shared-window addresses (no generic -> shared conversion per call)
 __device__ __forceinline__ void mbar_arrive_u32(uint32_t bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ bool mbar_test_wait_u32(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-  return ok != 0;
 }
 __device__ __forceinline__ void mbar_wait_u32(uint32_t bar, uint32_t parity) {
   asm volatile(
@@ -136,39 +115,6 @@ __device__ __forceinline__ void bulk_s2g(void* gdst, const void* smem_src, uint3
 __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }   // sources may be overwritten
 __device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }          // writes are complete
 
-// same copy delivered to the same CTA-relative offset of every CTA in cta_mask (and complete_tx on each one's barrier)
-__device__ __forceinline__ void bulk_g2s_multicast(void* smem_dst, const void* gsrc, uint32_t bytes, uint64_t* bar, uint16_t cta_mask) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;"
-               ::"r"(smem_u32(smem_dst)), "l"(gsrc), "r"(bytes), "r"(smem_u32(bar)), "h"(cta_mask) : "memory");
-}
-// ------------------------------------------------------------------ thread-block clusters
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ uint32_t cluster_id_x() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%clusterid.x;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ uint32_t cluster_nctaid_x() {   // number of clusters in the grid (x)
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%nclusterid.x;" : "=r"(r));
-  return r;
-}
-// arrive on the mbarrier at the same offset in CTA `rank` of the cluster (release at cluster scope)
-__device__ __forceinline__ void mbar_arrive_cluster(uint64_t* bar, uint32_t rank) {
-  asm volatile(
-      "{\n\t.reg .b32 ra;\n\t"
-      "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-      "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t}"
-      ::"r"(smem_u32(bar)), "r"(rank) : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {       // every thread of every CTA of the cluster
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-
 // ------------------------------------------------------------------ tcgen05: TMEM management
 template <uint32_t kCols>
 __device__ __forceinline__ void tmem_alloc(uint32_t* smem_result) {   // one full warp
@@ -178,16 +124,6 @@ __device__ __forceinline__ void tmem_alloc(uint32_t* smem_result) {   // one ful
 template <uint32_t kCols>
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr) {        // same warp that allocated
   asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "n"(kCols) : "memory");
-}
-// CTA-pair (cta_group::2) variants: one warp of EACH CTA of the pair executes them
-template <uint32_t kCols>
-__device__ __forceinline__ void tmem_alloc_pair(uint32_t* smem_result) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_result)), "n"(kCols) : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-template <uint32_t kCols>
-__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "n"(kCols) : "memory");
 }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
@@ -226,28 +162,9 @@ __device__ __forceinline__ void mma_f16_ss(uint32_t d_tmem, uint64_t a_desc, uin
       "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
       ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
 }
-// CTA pair: D[256 x N] (+)= A[256 x K] * B[N x K]^T, rows 0-127 / 128-255 of A and D live in CTA 0 / CTA 1, each CTA
-// holds N/2 rows of B at the same shared-memory offset; issued by one thread of the leader CTA (rank 0)
-__device__ __forceinline__ void mma_f16_ss_pair(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void mma_commit_pair(uint64_t* bar, uint16_t cta_mask) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(smem_u32(bar)), "h"(cta_mask) : "memory");
-}
 // all previously issued MMAs of this thread -> one arrival on the mbarrier when they complete
 __device__ __forceinline__ void mma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-
-// the same, arriving on the barrier at this CTA-relative offset in every CTA of cta_mask
-__device__ __forceinline__ void mma_commit_multicast(uint64_t* bar, uint16_t cta_mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(smem_u32(bar)), "h"(cta_mask) : "memory");
 }
 
 // ------------------------------------------------------------------ tcgen05: TMEM <-> registers
@@ -268,9 +185,6 @@ __device__ __forceinline__ void tmem_ld_x16(uint32_t taddr, uint32_t (&v)[16]) {
       : GO2P_R4(v, 0), GO2P_R4(v, 4), GO2P_R4(v, 8), GO2P_R4(v, 12)
       : "r"(taddr) : "memory");
 }
-__device__ __forceinline__ void tmem_ld_x8(uint32_t taddr, uint32_t (&v)[8]) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];" : GO2P_R4(v, 0), GO2P_R4(v, 4) : "r"(taddr) : "memory");
-}
 __device__ __forceinline__ void tmem_ld_x4(uint32_t taddr, uint32_t (&v)[4]) {
   asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0,%1,%2,%3}, [%4];" : GO2P_R4(v, 0) : "r"(taddr) : "memory");
 }
@@ -278,9 +192,6 @@ __device__ __forceinline__ void tmem_st_x16(uint32_t taddr, const uint32_t (&v)[
   asm volatile(
       "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};"
       ::"r"(taddr), GO2P_W4(v, 0), GO2P_W4(v, 4), GO2P_W4(v, 8), GO2P_W4(v, 12) : "memory");
-}
-__device__ __forceinline__ void tmem_st_x4(uint32_t taddr, const uint32_t (&v)[4]) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1,%2,%3,%4};" ::"r"(taddr), GO2P_W4(v, 0) : "memory");
 }
 __device__ __forceinline__ void tmem_st_x8(uint32_t taddr, const uint32_t (&v)[8]) {
   asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
@@ -361,20 +272,6 @@ __device__ __forceinline__ uint32_t negabs_f16x2(uint32_t x) {
   asm("abs.f16x2 %0, %1;" : "=r"(a) : "r"(x));
   asm("neg.f16x2 %0, %1;" : "=r"(r) : "r"(a));
   return r;
-}
-// 2^x for x <= 0 on the FMA/ALU pipes (no MUFU): round-to-nearest split x = n + r via the 1.5*2^23 trick,
-// degree-3 minimax polynomial for 2^r on [-0.5, 0.5] (max relative error 7.5e-5, below half an fp16 ulp), exponent
-// patched in with an integer add.  Inputs below -24 are clamped (2^-24 is far below the resolution of c*(2^x - 1));
-// results for x > 0 are garbage by design: the ELU select discards them.  Used for a fraction of the columns so the
-// MUFU pipe (16 lanes/clk/SM, the per-SM floor of this policy) is not the only exponential unit.
-__device__ __forceinline__ float ex2_poly(float x) {
-  x = fmaxf(x, -24.0f);
-  const float t = __fadd_rn(x, 12582912.0f);
-  const float r = __fsub_rn(x, __fsub_rn(t, 12582912.0f));
-  float p = fmaf(0.055171653628349304f, r, 0.2426111251115799f);
-  p = fmaf(p, r, 0.6932609677314758f);
-  p = fmaf(p, r, 0.9999280571937561f);
-  return __uint_as_float(__float_as_uint(p) + (__float_as_uint(t) << 23));
 }
 __device__ __forceinline__ float ex2_approx(float x) {
   float r;
